@@ -2,6 +2,7 @@
 """bench.py -- batched SE(3)-MPC solves/sec on B200 (BASELINE.json metric).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--batch B]
+                    [--dump-outputs DIR]
 
 A "step" is one batched solve of the workload (BASELINE.json configs[1]: 4096 hover-to-goal
 problems, seed 1, p0~U(-10,10)^3, v0=0, goal~U(-15,15)^2 x U(3,8), default airframe, N=8,
@@ -12,6 +13,10 @@ output) through the package's public BatchWorkspace API.  One JSON line on stdou
 `--impl reference` times the CPU restatement of the reference path (oracle/, C, all host
 threads) on the same workload; that and the `cpu_baseline` leg are the only places this file
 touches oracle/.
+
+`--dump-outputs DIR` writes what the last timed step of `value` (or of `--impl reference`)
+returned to its caller as DIR/<field>.npy, so that two builds run with the same arguments can be
+compared output for output (the inputs are seeded).
 """
 from __future__ import annotations
 
@@ -34,6 +39,8 @@ L2_FLUSH_BYTES = 256 << 20
 L2_BYTES = 126 << 20
 E2E_DEPTH = 3
 VALUE_DEPTH = int(os.environ.get("DART_BENCH_DEPTH", "4"))
+DUMP_BYTES = 64 * 10 ** 6
+DUMP_FIELDS = ("x", "cost", "nit", "nfev", "status", "task", "accelerations", "attitudes", "body_rates", "thrusts")
 
 
 def workload_inputs(B, seed):
@@ -48,6 +55,23 @@ def workload_inputs(B, seed):
 def alg_bytes_per_solve(N):
     """SURVEY.md 8(d): inputs 9 fp64 + outputs (19N+1) fp64 + 3 int32 (+1 int32 task code)."""
     return 8 * 9 + 8 * (19 * N + 1) + 4 * 4
+
+
+def dump_outputs(out_dir, sol):
+    """sol: the host result of one batched solve (HostSolution or oracle.BatchResult).  Writes each
+    of DUMP_FIELDS as out_dir/<field>.npy in float64 (the int32 counters convert exactly) and
+    index.npy, the problems the rows belong to: all of them, or a fixed seeded sample when the
+    batch's outputs would exceed DUMP_BYTES."""
+    B = len(sol.cost)
+    per_problem = 8 * (1 + sum(np.asarray(getattr(sol, f))[0].size for f in DUMP_FIELDS))     # 1: index
+    idx = np.arange(B)
+    if B * per_problem > DUMP_BYTES:
+        keep = (DUMP_BYTES - (64 << 10)) // per_problem          # 64 KiB left for the .npy headers
+        idx = np.sort(np.random.default_rng(0).choice(B, keep, replace=False))
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "index.npy"), idx.astype(np.float64))
+    for f in DUMP_FIELDS:
+        np.save(os.path.join(out_dir, f + ".npy"), np.asarray(getattr(sol, f))[idx].astype(np.float64))
 
 
 def host_cores():
@@ -171,8 +195,10 @@ def run_reference(args):
         oracle.solve_batch(params, p0, v0, goal, nthreads=cores)
     t0 = time.perf_counter()
     for _ in range(args.steps):
-        oracle.solve_batch(params, p0, v0, goal, nthreads=cores)
+        sol = oracle.solve_batch(params, p0, v0, goal, nthreads=cores)
     dt = time.perf_counter() - t0
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, sol)
     value = args.steps * B / dt
     line = {
         "impl": "reference", "metric": METRIC, "value": value, "unit": UNIT, "n_gpus": args.gpus,
@@ -364,7 +390,11 @@ def main():
     ap.add_argument("--horizon", type=int, default=8)
     ap.add_argument("--dt", type=float, default=0.1)
     ap.add_argument("--no-extras", action="store_true", help="skip sweep / latency / cpu baseline legs")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the outputs of the last timed step (rank 0) as DIR/<field>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3)
 
     if args.impl == "reference":
@@ -427,7 +457,8 @@ def main():
         ring.append(w)
     def run_stream(depth, hint):
         """K steps, `depth` of them in flight (one stream each, round robin); one event pair around
-        all of them on the launching stream.  Returns (milliseconds, launches)."""
+        all of them on the launching stream.  Returns (milliseconds, launches, the last step's
+        BatchSolution)."""
         streams = [stream] + [torch.cuda.Stream() for _ in range(depth - 1)]
         L.dart_se3mpc_set_inflight_hint(hint)
         try:
@@ -445,14 +476,14 @@ def main():
             for st in streams[1:]:
                 st.wait_event(e0)
             for i in range(args.steps):
-                ring[i % nsets].solve_device(streams[i % depth])
+                last = ring[i % nsets].solve_device(streams[i % depth])
             for st in streams[1:]:
                 ev = torch.cuda.Event()
                 ev.record(st)
                 stream.wait_event(ev)
             e1.record(stream)
             torch.cuda.synchronize()
-            return float(e0.elapsed_time(e1)), L.dart_launch_count() - n0
+            return float(e0.elapsed_time(e1)), L.dart_launch_count() - n0, last
         finally:
             L.dart_se3mpc_set_inflight_hint(0)
 
@@ -467,13 +498,16 @@ def main():
     # runs them in the throughput build.  `single_stream`: the same K steps strictly one after the
     # other on one stream (latency build).
     sampler.active.set()
-    total_ms, launches = run_stream(VALUE_DEPTH, VALUE_DEPTH * B)
+    total_ms, launches, last = run_stream(VALUE_DEPTH, VALUE_DEPTH * B)
     sampler.active.clear()
+    if args.dump_outputs and rank == 0:     # before single_stream overwrites the ring's results
+        dump_outputs(args.dump_outputs, last.numpy())
+    del last
     barrier()
     total_ms_max = max_over_ranks(total_ms)
     value = world * B * args.steps / (total_ms_max * 1e-3)
     sampler.active.set()
-    single_ms, _ = run_stream(1, 0)
+    single_ms, _, _ = run_stream(1, 0)
     sampler.active.clear()
     barrier()
     single_value = world * B * args.steps / (max_over_ranks(single_ms) * 1e-3)
