@@ -32,9 +32,16 @@ class ClosedLoopSim:
     >>> sim.reset(p0, v0, goals)
     >>> sim.run(100)                  # 100 launches, state stays on the device
     >>> sim.positions(), sim.velocities(), sim.nfev_total
+
+    Dynamics-consistent params (gradient_mode 3) are accepted: the plan's positions and velocities
+    are then the rollout of the same plant model, so with ``plant_dt == params.dt`` the state after
+    a step is the plan's P_1 / V_1.  Warm starts use the 9-slot kernel (the lateral thrust moves).
+    gradient_mode 2 and 4 need a map, which the step entry does not take: they are refused.
     """
 
     def __init__(self, params: _cabi.Params, B: int, plant_dt: Optional[float] = None, device=None):
+        if int(params.gradient_mode) in (2, 4):
+            raise ValueError("ClosedLoopSim: gradient_mode 2 / 4 need a map; the closed-loop step has none")
         torch = _torch()
         self.params = params
         self.N = int(params.horizon)
@@ -52,7 +59,7 @@ class ClosedLoopSim:
         # the solutions held in self.x come from cold starts of this solver, so their lateral
         # thrust is exactly zero and stays zero: warm starts may use the 7-slot kernel (warm=2;
         # the kernel verifies).  Anyone writing self.x by hand must clear this flag.
-        self.lateral_thrust_is_zero = True
+        self.lateral_thrust_is_zero = int(params.gradient_mode) != 3
         self._lib = _cabi.lib()
 
     def reset(self, p0, v0, goals):
@@ -64,7 +71,7 @@ class ClosedLoopSim:
         self.x.zero_()
         self.nfev_total.zero_()
         self.steps_done = 0
-        self.lateral_thrust_is_zero = True
+        self.lateral_thrust_is_zero = int(self.params.gradient_mode) != 3
 
     def _launch(self, lo: int, hi: int, stream, track_counters: bool):
         """One replanning step of drones [lo, hi) (one launch): solve, store, advance the plant."""

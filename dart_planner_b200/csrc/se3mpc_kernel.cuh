@@ -169,7 +169,7 @@ se3mpc_solve_kernel(const __grid_constant__ dart_se3mpc_params P, const __grid_c
         bool refused = !alive || idle_lane;
         long long b = b_in;
         SolverT sv(P, sm, ws, wy);
-        if (GM == 2) {
+        if (GM == 2 || GM == 4) {
             sv.obs.g = A.grid;
             sv.obs.w = P.w_obstacle;
             sv.obs.free_level = P.obstacle_free_level;
@@ -579,9 +579,10 @@ se3mpc_extract_kernel(const __grid_constant__ dart_se3mpc_params P, const __grid
     }
 }
 
-/* the six instantiations of one lane configuration: [gradient_mode][tilt] */
+/* the eight instantiations of one lane configuration: [gradient_mode][tilt].  The dynamics-consistent
+ * modes 3 / 4 move the lateral thrust, so they exist only with tilt (fn[3][0] = fn[4][0] = null). */
 struct KernelSet {
-    const void *fn[3][2];
+    const void *fn[5][2];
     const void *extract_fn[2]; /* [tilt] */
     int lanes, tpl, block, minb;
     int gpb;      /* problems per block */
@@ -598,6 +599,10 @@ KernelSet make_kernel_set()
     k.fn[0][0] = (const void *)se3mpc_solve_kernel<LANES, TPL, BLK, MINB, 0, false>;
     k.fn[1][0] = (const void *)se3mpc_solve_kernel<LANES, TPL, BLK, MINB, 1, false>;
     k.fn[2][0] = (const void *)se3mpc_solve_kernel<LANES, TPL, BLK, MINB, 2, false>;
+    k.fn[3][1] = (const void *)se3mpc_solve_kernel<LANES, TPL, BLK, MINB, 3, true>;
+    k.fn[4][1] = (const void *)se3mpc_solve_kernel<LANES, TPL, BLK, MINB, 4, true>;
+    k.fn[3][0] = nullptr;
+    k.fn[4][0] = nullptr;
     k.extract_fn[1] = (const void *)se3mpc_extract_kernel<LANES, TPL, BLK, true>;
     k.extract_fn[0] = (const void *)se3mpc_extract_kernel<LANES, TPL, BLK, false>;
     k.lanes = LANES;

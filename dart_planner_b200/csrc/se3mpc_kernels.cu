@@ -100,9 +100,10 @@ unsigned g_prio_next[64] = {0};
 
 size_t stash_bytes_for(const KernelChoice &k, long long grid)
 {
-    /* upper bound of Solver::ctx_doubles(1) over the gradient modes (se3mpc_core.cuh) */
+    /* upper bound of Solver::ctx_doubles(1) over the gradient modes (se3mpc_core.cuh): the
+     * dynamics-consistent modes keep 6 more scalars */
     const size_t S = 9 * (size_t)k.tpl, gpb = (size_t)k.set.gpb;
-    const size_t ctx = 16 + 2 * ((S + 31) / 32) + 7 + (size_t)k.lanes * (4 * S + 3 * k.tpl);
+    const size_t ctx = 16 + 6 + 2 * ((S + 31) / 32) + 7 + (size_t)k.lanes * (4 * S + 3 * k.tpl);
     return (size_t)grid * (2 * gpb - 1) * ctx * sizeof(double);
 }
 
@@ -159,7 +160,9 @@ int prepare(KernelChoice *k)
         if (e != cudaSuccess) return set_err(e, "cudaDeviceGetAttribute");
     }
     const int smem = smem_bytes(*k);
-    for (const void *fn : {k->set.fn[0][0], k->set.fn[0][1], k->set.fn[1][0], k->set.fn[1][1], k->set.fn[2][0], k->set.fn[2][1]}) {
+    const void *fns[] = {k->set.fn[0][0], k->set.fn[0][1], k->set.fn[1][0], k->set.fn[1][1],
+                         k->set.fn[2][0], k->set.fn[2][1], k->set.fn[3][1], k->set.fn[4][1]};
+    for (const void *fn : fns) {
         e = cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
         if (e != cudaSuccess) return set_err(e, "cudaFuncSetAttribute(smem)");
     }
@@ -167,7 +170,7 @@ int prepare(KernelChoice *k)
      * the driver reserves); the rest stays L1 for the per-lane S/Y pairs in local memory */
     int carve = (int)((long long)k->set.resident * (smem + 1024) * 100 / (228 * 1024)) + 1;
     if (carve > 100) carve = 100;
-    for (const void *fn : {k->set.fn[0][0], k->set.fn[0][1], k->set.fn[1][0], k->set.fn[1][1], k->set.fn[2][0], k->set.fn[2][1]}) {
+    for (const void *fn : fns) {
         e = cudaFuncSetAttribute(fn, cudaFuncAttributePreferredSharedMemoryCarveout, carve);
         if (e != cudaSuccess) return set_err(e, "cudaFuncSetAttribute(carveout)");
     }
@@ -188,7 +191,11 @@ int check_params(const dart_se3mpc_params *p)
     if (p->horizon < 1 || p->horizon > 64) return DART_E_UNSUPPORTED;
     if (p->max_corrections < 1 || p->max_corrections > MMAX) return DART_E_UNSUPPORTED;
     if (p->max_iterations < 0 || p->max_linesearch < 0) return DART_E_BADARG;
-    if (p->gradient_mode < 0 || p->gradient_mode > 2) return DART_E_UNSUPPORTED;
+    if (p->gradient_mode < 0 || p->gradient_mode > 4) return DART_E_UNSUPPORTED;
+    /* dynamics-consistent modes: verified against the oracle up to the 16-lane builds; on 32-lane
+     * groups (horizons 17..64) the scan's rounding makes 5-7 % of the solves take other iteration
+     * counts than the sequential oracle at tolerance 1e-3 (DESIGN.md 5c) */
+    if (p->gradient_mode >= 3 && p->horizon > 16) return DART_E_UNSUPPORTED;
     if (!(p->dt > 0.0) || !(p->mass > 0.0)) return DART_E_BADARG;
     if (!(p->gtol >= 0.0)) return DART_E_BADARG; /* the Cauchy step relies on it (se3mpc_core.cuh) */
     return DART_OK;
@@ -359,7 +366,9 @@ static int launch_solve(const dart_se3mpc_params *params, const SolveArgs &a, vo
             stash_event = sb.done;
         }
     }
-    const int cold = ((a.x_warm == nullptr || a.no_tilt_promise) && !getenv("DART_SE3MPC_NO_COLD")) ? 0 : 1;
+    /* never the 7-slot instantiation in the dynamics-consistent modes: their lateral thrust moves */
+    const int cold = ((a.x_warm == nullptr || a.no_tilt_promise) && params->gradient_mode < 3 &&
+                      !getenv("DART_SE3MPC_NO_COLD")) ? 0 : 1;
     const void *fn = k->set.fn[params->gradient_mode][cold];
     cudaError_t e;
     if (prio_event) {
@@ -398,7 +407,7 @@ int dart_se3mpc_solve_batch_map(const dart_se3mpc_params *params, int64_t B, int
     int rc = check_params(params);
     if (rc) return rc;
     if (B < 0 || ld < B || !p0 || !v0 || !goal) return DART_E_BADARG;
-    const bool need_grid = first_hit != nullptr || params->gradient_mode == 2;
+    const bool need_grid = first_hit != nullptr || params->gradient_mode == 2 || params->gradient_mode == 4;
     if (need_grid && (!grid || !grid->occ || grid->nx <= 0 || grid->ny <= 0 || grid->nz <= 0 ||
                       !(grid->resolution > 0.0)))
         return DART_E_BADARG;
@@ -428,7 +437,10 @@ int dart_se3mpc_closed_loop_step(const dart_se3mpc_params *params, int64_t B, in
     int rc = check_params(params);
     if (rc) return rc;
     if (B < 0 || ld < B || !p || !v || !goal || !x || !(plant_dt > 0.0)) return DART_E_BADARG;
-    if (params->gradient_mode == 2) return DART_E_UNSUPPORTED; /* no map argument here */
+    /* no map argument here: no obstacle penalty */
+    if (params->gradient_mode == 2 || params->gradient_mode == 4) return DART_E_UNSUPPORTED;
+    /* the promise of warm == 2 (zero lateral thrust) does not hold in the dynamics-consistent mode */
+    if (params->gradient_mode == 3 && warm == 2) return DART_E_BADARG;
     if (B == 0) return DART_OK;
     SolveArgs a;
     memset(&a, 0, sizeof(a));
@@ -503,7 +515,7 @@ int dart_se3mpc_solve_batch_rows(const dart_se3mpc_params *params, int64_t B, in
     if (row_stride < need || (row_stride & 15) != 0 || row_stride > SM_DOUBLES ||
         ((uintptr_t)rows & 127) != 0)
         return DART_E_BADARG;
-    const bool need_grid = check_map != 0 || params->gradient_mode == 2;
+    const bool need_grid = check_map != 0 || params->gradient_mode == 2 || params->gradient_mode == 4;
     if (need_grid && (!grid || !grid->occ || grid->nx <= 0 || grid->ny <= 0 || grid->nz <= 0 ||
                       !(grid->resolution > 0.0)))
         return DART_E_BADARG;

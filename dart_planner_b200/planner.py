@@ -586,7 +586,7 @@ def plan_batch(positions, velocities, goals, config: Optional[SE3MPCConfig] = No
                has_goal=None, x_warm=None, warm_mask=None, gradient_mode: int = 0,
                device=None, outputs: str = "all", to_host: bool = False, grid=None,
                safety_margin: float = 1.0, collision_threshold: float = 0.6,
-               obstacle_penalty: bool = False):
+               obstacle_penalty: bool = False, dynamics_consistent: bool = False):
     """Solve B independent SE(3)-MPC problems in one call.
 
     positions, velocities, goals : (B, 3) array-likes (NumPy or torch, host or device)
@@ -599,13 +599,21 @@ def plan_batch(positions, velocities, goals, config: Optional[SE3MPCConfig] = No
     obstacle_penalty : with a grid, also add the occupancy-grid obstacle penalty to the objective
              and gradient inside the solve (gradient_mode 2; extension -- the reference solve has
              no obstacle term; weight = config.obstacle_weight, free level = the grid's prior)
+    dynamics_consistent : optimise the thrusts only; positions and velocities are the rollout of
+             the plant model from (p0, v0) (gradient_mode 3, with ``obstacle_penalty`` mode 4;
+             extension).  The P/V rows of the result are that rollout; ``pos_bound`` and
+             ``max_velocity`` are not enforced in this mode.
     Returns a BatchSolution (device) or HostSolution (``to_host=True``).
     """
     cfg = config or SE3MPCConfig()
+    if dynamics_consistent:
+        if gradient_mode != 0:
+            raise ValueError("dynamics_consistent selects its own gradient mode")
+        gradient_mode = 3
     if obstacle_penalty:
-        if grid is None or gradient_mode != 0:
+        if grid is None or gradient_mode not in (0, 3):
             raise ValueError("obstacle_penalty needs grid= and the reference gradient mode")
-        gradient_mode = 2
+        gradient_mode = 2 if gradient_mode == 0 else 4
     params = make_params(cfg, mass=mass, gravity=gravity, dt=dt, gradient_mode=gradient_mode,
                          obstacle_free_level=grid.prob_prior if grid is not None else 0.5)
     B = int(np.shape(positions)[0])

@@ -53,6 +53,19 @@ typedef struct dart_se3mpc_params {
                                /* 1: exact gradient of :516-550 (extension, self-oracle)   */
                                /* 2: mode 0 + occupancy-grid obstacle penalty in f and g    */
                                /*    (extension, self-oracle; needs a grid, see _solve_batch_map) */
+                               /* 3: dynamics-consistent solve (extension, self-oracle): the   */
+                               /*    3N thrusts are the only variables; P and V are the rollout */
+                               /*    of the plant model (:430-431, :445-459) from (p0, v0):     */
+                               /*    a_k = T_k/m - g e3, P_0 = p0, V_0 = v0,                    */
+                               /*    P_{k+1} = (P_k + V_k dt) + (0.5 a_k) dt^2,                 */
+                               /*    V_{k+1} = V_k + a_k dt.  f is :516-550 at [P | V | T], g   */
+                               /*    its exact gradient in T (adjoint).  The P/V rows of x are  */
+                               /*    OUTPUTS (the rollout of the returned T; the P/V rows of a  */
+                               /*    warm start are ignored); pos_bound and max_velocity are    */
+                               /*    NOT enforced.  Closed-loop step: warm == 2 is refused.     */
+                               /*    Horizons 1..16 (DART_E_UNSUPPORTED above).                 */
+                               /* 4: mode 3 + the obstacle penalty of mode 2 on the rolled-out  */
+                               /*    positions (needs a grid; not in the closed-loop step)      */
     int32_t reserved0;
     double dt;                 /* effective planner dt (timing_alignment.py:76-78)         */
     double mass, gravity;      /* 1.5 kg, 9.81 m/s^2 (:149-150)                            */
@@ -63,7 +76,7 @@ typedef struct dart_se3mpc_params {
     double w_pos, w_vel, w_acc, w_thrust; /* cost weights (:56-59)                          */
     double gtol;               /* convergence_tolerance (:264)                             */
     double ftol;               /* 10*convergence_tolerance (:265)                          */
-    /* gradient_mode 2 only: f += w_obstacle * sum_k max(0, o(P_k) - obstacle_free_level)^2 with
+    /* gradient_mode 2 and 4 only: f += w_obstacle * sum_k max(0, o(P_k) - obstacle_free_level)^2 with
      * o = trilinear occupancy over voxel centres.  w_obstacle = SE3MPCConfig.obstacle_weight
      * (:60, unused by the reference solve), free level = the map's prior (0.5). */
     double w_obstacle, obstacle_free_level;
@@ -192,7 +205,10 @@ int dart_se3mpc_solve_batch_rows(const dart_se3mpc_params *params, int64_t B, in
  * warm == 2: warm start with the caller's promise that every lateral thrust entry (T_x, T_y) of
  * x is exactly zero -- true for solutions this library produced from cold starts, since a zero
  * lateral thrust has a zero gradient and never moves.  The faster 7-slot kernel then serves the
- * warm start; a problem whose x breaks the promise is not solved and gets status 3. */
+ * warm start; a problem whose x breaks the promise is not solved and gets status 3.
+ * gradient_mode 3: warm == 2 returns DART_E_BADARG (the lateral thrust moves); with
+ * plant_dt == params->dt the new state is the solution's P_1 / V_1.  gradient_mode 2 and 4
+ * (obstacle penalty: no map argument here) return DART_E_UNSUPPORTED. */
 int dart_se3mpc_closed_loop_step(const dart_se3mpc_params *params, int64_t B, int64_t ld, double *p,
                                  double *v, const double *goal, const uint8_t *has_goal, double *x,
                                  int32_t warm, double *cost, int32_t *nit, int32_t *nfev,
