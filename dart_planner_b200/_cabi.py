@@ -57,6 +57,7 @@ EXPORTS = [
     "dart_launch_count", "dart_se3mpc_set_inflight_hint",
     "dart_se3mpc_kernel_info", "dart_map_query_batch", "dart_map_traj_safe_batch",
     "dart_map_trace_ray_batch", "dart_map_update_batch", "dart_map_add_spheres", "dart_fp64_probe", "dart_ddiv_selftest",
+    "dart_map_signed_distance", "dart_map_clearance_field", "dart_se3mpc_closed_loop_step_map",
 ]
 
 _lib = None
@@ -89,6 +90,10 @@ def lib():
     L.dart_se3mpc_closed_loop_step.argtypes = ([C.POINTER(Params), i64, i64] + [vp] * 5 + [i32] +
                                                [vp] * 4 + [C.c_double, vp])
     L.dart_se3mpc_closed_loop_step.restype = C.c_int
+    L.dart_se3mpc_closed_loop_step_map.argtypes = ([C.POINTER(Params), i64, i64] + [vp] * 5 + [i32] +
+                                                   [vp] * 4 + [C.c_double, C.POINTER(Grid), C.POINTER(Grid),
+                                                                C.c_double, C.c_double, i32, vp, vp])
+    L.dart_se3mpc_closed_loop_step_map.restype = C.c_int
     L.dart_se3mpc_solve_batch_host.argtypes = [C.POINTER(Params), i64] + [vp] * 14
     L.dart_se3mpc_solve_batch_host.restype = C.c_int
     L.dart_se3mpc_extract_batch.argtypes = [C.POINTER(Params), i64, i64] + [vp] * 5 + [i32, vp]
@@ -117,6 +122,10 @@ def lib():
     L.dart_map_update_batch.restype = C.c_int
     L.dart_map_add_spheres.argtypes = [C.POINTER(Grid), vp, i32, vp, vp, C.c_double, vp]
     L.dart_map_add_spheres.restype = C.c_int
+    L.dart_map_signed_distance.argtypes = [C.POINTER(Grid), C.c_double, vp, vp, vp]
+    L.dart_map_signed_distance.restype = C.c_int
+    L.dart_map_clearance_field.argtypes = [C.POINTER(Grid), C.c_double, C.c_double, C.c_double, vp, vp, vp]
+    L.dart_map_clearance_field.restype = C.c_int
     L.dart_fp64_probe.argtypes = [i32, C.POINTER(i32), vp, vp]
     L.dart_fp64_probe.restype = C.c_int
     L.dart_ddiv_selftest.argtypes = [i64, C.c_uint64, i32, vp, vp]

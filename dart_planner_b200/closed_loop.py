@@ -36,13 +36,27 @@ class ClosedLoopSim:
     Dynamics-consistent params (gradient_mode 3) are accepted: the plan's positions and velocities
     are then the rollout of the same plant model, so with ``plant_dt == params.dt`` the state after
     a step is the plan's P_1 / V_1.  Warm starts use the 9-slot kernel (the lateral thrust moves).
-    gradient_mode 2 and 4 need a map, which the step entry does not take: they are refused.
+
+    Against a map (``dart_se3mpc_closed_loop_step_map``):
+      penalty_grid  : DenseOccupancyGrid the obstacle penalty of gradient_mode 2 / 4 reads (those
+                      modes need it; typically ``grid.clearance_field(d_safe)``; params'
+                      ``obstacle_free_level`` should be its prior, 0.5)
+      collision_map : DenseOccupancyGrid the flown path of every step is checked against: the
+                      straight segment from the state before to the state after the step, sampled
+                      at steps of at most half a voxel (at most 64 samples), each sample with
+                      is_trajectory_safe's stencil (``safety_margin``, ``collision_threshold``).
+                      ``first_collision()`` is the first step index at which a drone's path
+                      collided, -1 = never.
     """
 
-    def __init__(self, params: _cabi.Params, B: int, plant_dt: Optional[float] = None, device=None):
-        if int(params.gradient_mode) in (2, 4):
-            raise ValueError("ClosedLoopSim: gradient_mode 2 / 4 need a map; the closed-loop step has none")
+    def __init__(self, params: _cabi.Params, B: int, plant_dt: Optional[float] = None, device=None, *,
+                 penalty_grid=None, collision_map=None, safety_margin: float = 0.0,
+                 collision_threshold: float = 0.6):
+        if int(params.gradient_mode) in (2, 4) and penalty_grid is None:
+            raise ValueError("ClosedLoopSim: gradient_mode 2 / 4 need penalty_grid=")
         torch = _torch()
+        self.penalty_grid, self.collision_map = penalty_grid, collision_map
+        self.safety_margin, self.collision_threshold = float(safety_margin), float(collision_threshold)
         self.params = params
         self.N = int(params.horizon)
         self.B = int(B)
@@ -55,11 +69,12 @@ class ClosedLoopSim:
         self.cost = torch.zeros(self.ld, **f8)
         self.meta = torch.zeros((3, self.ld), dtype=torch.int32, device=self.device)  # nit, nfev, status
         self.nfev_total = torch.zeros(self.ld, dtype=torch.int64, device=self.device)
+        self._first_collision = torch.full((self.ld,), -1, dtype=torch.int32, device=self.device)
         self.steps_done = 0
         # the solutions held in self.x come from cold starts of this solver, so their lateral
         # thrust is exactly zero and stays zero: warm starts may use the 7-slot kernel (warm=2;
         # the kernel verifies).  Anyone writing self.x by hand must clear this flag.
-        self.lateral_thrust_is_zero = int(params.gradient_mode) != 3
+        self.lateral_thrust_is_zero = int(params.gradient_mode) < 3
         self._lib = _cabi.lib()
 
     def reset(self, p0, v0, goals):
@@ -70,8 +85,9 @@ class ClosedLoopSim:
             self.state[3 * i: 3 * i + 3, : self.B] = t.reshape(self.B, 3).t()
         self.x.zero_()
         self.nfev_total.zero_()
+        self._first_collision.fill_(-1)
         self.steps_done = 0
-        self.lateral_thrust_is_zero = int(self.params.gradient_mode) != 3
+        self.lateral_thrust_is_zero = int(self.params.gradient_mode) < 3
 
     def _launch(self, lo: int, hi: int, stream, track_counters: bool):
         """One replanning step of drones [lo, hi) (one launch): solve, store, advance the plant."""
@@ -79,14 +95,22 @@ class ClosedLoopSim:
         es = 8 * self.ld
         base = self.state.data_ptr() + 8 * lo
         meta = self.meta.data_ptr() + 4 * lo
-        with torch.cuda.device(self.device):
-            rc = self._lib.dart_se3mpc_closed_loop_step(
-                C.byref(self.params), hi - lo, self.ld, base, base + 3 * es, base + 6 * es, None,
+        args = (C.byref(self.params), hi - lo, self.ld, base, base + 3 * es, base + 6 * es, None,
                 self.x.data_ptr() + 8 * lo,
                 0 if self.steps_done == 0 else (2 if self.lateral_thrust_is_zero else 1), self.cost.data_ptr() + 8 * lo,
-                meta, meta + 4 * self.ld, meta + 8 * self.ld,
-                self.plant_dt, stream.cuda_stream)
-        _cabi.check(rc, "dart_se3mpc_closed_loop_step")
+                meta, meta + 4 * self.ld, meta + 8 * self.ld, self.plant_dt)
+        with torch.cuda.device(self.device):
+            if self.penalty_grid is None and self.collision_map is None:
+                rc = self._lib.dart_se3mpc_closed_loop_step(*args, stream.cuda_stream)
+            else:
+                pg = self.penalty_grid._grid() if self.penalty_grid is not None else None
+                cg = self.collision_map._grid() if self.collision_map is not None else None
+                rc = self._lib.dart_se3mpc_closed_loop_step_map(
+                    *args, C.byref(pg) if pg is not None else None, C.byref(cg) if cg is not None else None,
+                    self.safety_margin, self.collision_threshold, self.steps_done,
+                    self._first_collision.data_ptr() + 4 * lo if cg is not None else None, stream.cuda_stream)
+        _cabi.check(rc, "dart_se3mpc_closed_loop_step" if self.penalty_grid is None and self.collision_map is None
+                    else "dart_se3mpc_closed_loop_step_map")
         if track_counters:
             with torch.cuda.stream(stream):
                 self.nfev_total[lo:hi] += self.meta[1, lo:hi]
@@ -149,6 +173,11 @@ class ClosedLoopSim:
             done.record(st)
             stream.wait_event(done)
         return None
+
+    def first_collision(self):
+        """(B,) int32: the step index (``steps_done`` when it ran) of each drone's first collision
+        with ``collision_map``, -1 = never (always -1 without a collision map)."""
+        return self._first_collision[: self.B]
 
     def positions(self):
         return self.state[0:3, : self.B].t()

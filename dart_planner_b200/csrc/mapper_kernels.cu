@@ -261,6 +261,129 @@ map_add_spheres_kernel(const __grid_constant__ dart_grid g, CELL *occ, int nsph,
     }
 }
 
+/* Exact Euclidean distance transform of the occupancy (`occ > threshold`, is_collision's strict
+ * test) for the signed distance and the clearance field: the separable lower envelope of parabolas
+ * of Felzenszwalb & Huttenlocher ("Distance Transforms of Sampled Functions", Theory of Computing
+ * 8, 2012), one pass along x, y, z, every comparison in integers (no intersection is ever formed
+ * as a float).  Between passes a cell is ONE int32: +D at a free cell (squared voxel distance to
+ * the nearest occupied cell found so far) and -D at an occupied cell (to the nearest free cell).
+ * The other distance of a cell is 0 at every stage -- the cell is a site of that transform -- so
+ * the sign says which transform the magnitude belongs to.  EDT_INF: no site on the lines so far.
+ * One thread per line; its envelope (sites and f(q) + q^2) lives in shared memory. */
+constexpr int EDT_INF = 0x3fffffff;
+
+template <bool FROM_GRID, bool LAST, class CELL>
+__global__ void __launch_bounds__(32)
+map_edt_pass_kernel(const __grid_constant__ dart_grid g, double thr, int axis, const int *src, int *dst,
+                    float *phi, CELL *field, double dsafe, double free_level, int diag2)
+{
+    extern __shared__ int edt_env[];
+    const int T = blockDim.x, t = threadIdx.x;
+    const int n = axis == 0 ? g.nx : (axis == 1 ? g.ny : g.nz);
+    const long long stride = axis == 0 ? 1ll : (axis == 1 ? (long long)g.nx : (long long)g.nx * g.ny);
+    const long long nlines = (long long)g.nx * g.ny * g.nz / n;
+    const long long line = (long long)blockIdx.x * T + t;
+    if (line >= nlines) return;
+    /* lines of one block are neighbours in x (y and z passes: coalesced) or in y (x pass) */
+    const long long base = axis == 0 ? line * g.nx
+                         : (axis == 1 ? (line / g.nx) * ((long long)g.nx * g.ny) + line % g.nx : line);
+    auto enc = [&](int q) -> int {
+        const long long i = base + q * stride;
+        if constexpr (FROM_GRID) {
+            const double o = g.cell_bytes == 8 ? __ldg(static_cast<const double *>(g.occ) + i)
+                                               : (double)__ldg(static_cast<const float *>(g.occ) + i);
+            return o > thr ? -EDT_INF : EDT_INF;
+        } else {
+            return __ldg(src + i);
+        }
+    };
+    int *sv = edt_env + t, *sh = edt_env + T + t; /* site k: sv[2kT], sh[2kT] */
+#pragma unroll 1
+    for (int sgn = 1; sgn >= -1; sgn -= 2) {
+        /* lower envelope of f(q) + (p - q)^2 over the sites with f(q) < EDT_INF, f = the sign's
+         * distance (0 at the cells of the other sign) */
+        int k = -1;
+        for (int q = 0; q < n; ++q) {
+            const int e = enc(q);
+            const int f = sgn > 0 ? max(e, 0) : max(-e, 0);
+            if (f >= EDT_INF) continue;
+            const long long h = (long long)f + (long long)q * q;
+            /* pop while the new parabola's intersection with the top one lies at or left of the
+             * top one's intersection with the one below:  (h - ha) / 2(q - a) <= (ha - hb) / 2(a - b) */
+            while (k >= 1) {
+                const long long a = sv[2 * k * T], b = sv[2 * (k - 1) * T];
+                const long long ha = sh[2 * k * T], hb = sh[2 * (k - 1) * T];
+                if ((h - ha) * (a - b) <= (ha - hb) * (q - a)) --k;
+                else break;
+            }
+            ++k;
+            sv[2 * k * T] = q;
+            sh[2 * k * T] = (int)h;
+        }
+        int j = 0;
+        for (int p = 0; p < n; ++p) {
+            /* advance while the next parabola's intersection lies left of p */
+            while (j < k && (long long)(sh[2 * (j + 1) * T] - sh[2 * j * T]) <
+                                2ll * p * (sv[2 * (j + 1) * T] - sv[2 * j * T]))
+                ++j;
+            const int e = enc(p);
+            if ((sgn > 0) != (e > 0)) continue; /* the other transform's cell */
+            int D = EDT_INF;
+            if (k >= 0) {
+                const long long q = sv[2 * j * T];
+                D = (int)((long long)sh[2 * j * T] - 2ll * p * q + (long long)p * p);
+            }
+            const long long i = base + p * stride;
+            if constexpr (LAST) {
+                /* no site anywhere: the box diagonal (any finite distance is shorter) */
+                D = min(D, diag2);
+                dst[i] = sgn > 0 ? D : -D;
+                const double dp = sgn > 0 ? (double)D : 0.0, dm = sgn > 0 ? 0.0 : (double)D;
+                const float ph = (float)(g.resolution * (sqrt(dp) - sqrt(dm)));
+                if (phi) phi[i] = ph;
+                if (field) field[i] = (CELL)(free_level + fmax(0.0, dsafe - (double)ph));
+            } else {
+                dst[i] = sgn > 0 ? D : -D;
+            }
+        }
+    }
+}
+
+template <bool FROM_GRID, bool LAST, class CELL>
+int launch_edt_pass(const dart_grid &g, double thr, int axis, const int *src, int *dst, float *phi,
+                    CELL *field, double dsafe, double free_level, int diag2, cudaStream_t s)
+{
+    const int n = axis == 0 ? g.nx : (axis == 1 ? g.ny : g.nz);
+    const long long nlines = (long long)g.nx * g.ny * g.nz / n;
+    int T = 49152 / (8 * n);
+    T = T < 1 ? 1 : (T > 32 ? 32 : T);
+    const int smem = 8 * n * T;
+    const void *fn = (const void *)map_edt_pass_kernel<FROM_GRID, LAST, CELL>;
+    if (smem > 49152 && cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, smem) != cudaSuccess)
+        return DART_E_CUDA;
+    map_edt_pass_kernel<FROM_GRID, LAST, CELL><<<(unsigned)((nlines + T - 1) / T), T, smem, s>>>(
+        g, thr, axis, src, dst, phi, field, dsafe, free_level, diag2);
+    if (cudaGetLastError() != cudaSuccess) return DART_E_CUDA;
+    dart_count_launch_();
+    return DART_OK;
+}
+
+/* the three passes: grid -> S0 (x), S0 -> S1 (y), S1 -> S0 (z, with phi / the field) */
+template <class CELL>
+int edt(const dart_grid &g, double thr, float *phi, CELL *field, double dsafe, double free_level, int *scratch,
+        cudaStream_t s)
+{
+    const long long ncell = (long long)g.nx * g.ny * g.nz;
+    const long long diag2 = (long long)g.nx * g.nx + (long long)g.ny * g.ny + (long long)g.nz * g.nz;
+    /* every D and f(q) + q^2 stays below EDT_INF, and a line's envelope fits one block's shared memory */
+    if (diag2 >= EDT_INF) return DART_E_UNSUPPORTED;
+    int *s0 = scratch, *s1 = scratch + ncell;
+    int rc = launch_edt_pass<true, false, CELL>(g, thr, 0, nullptr, s0, nullptr, nullptr, 0.0, 0.0, 0, s);
+    if (!rc) rc = launch_edt_pass<false, false, CELL>(g, thr, 1, s0, s1, nullptr, nullptr, 0.0, 0.0, 0, s);
+    if (!rc) rc = launch_edt_pass<false, true, CELL>(g, thr, 2, s1, s0, phi, field, dsafe, free_level, (int)diag2, s);
+    return rc;
+}
+
 int grid_blocks(long long B)
 {
     long long nb = (B + 255) / 256;
@@ -358,6 +481,26 @@ int dart_map_add_spheres(const dart_grid *g, void *occ_writable, int32_t n, cons
     if (cudaGetLastError() != cudaSuccess) return DART_E_CUDA;
     dart_count_launch_();
     return DART_OK;
+}
+
+int dart_map_signed_distance(const dart_grid *g, double threshold, float *phi_out, int32_t *sq_scratch,
+                             void *stream)
+{
+    if (check_grid(g) || !sq_scratch) return DART_E_BADARG;
+    return edt<float>(*g, threshold, phi_out, nullptr, 0.0, 0.0, sq_scratch, (cudaStream_t)stream);
+}
+
+int dart_map_clearance_field(const dart_grid *g, double threshold, double safety_distance, double free_level,
+                             void *field_out, int32_t *sq_scratch, void *stream)
+{
+    if (check_grid(g) || !field_out || !sq_scratch || !(safety_distance >= 0.0) || !isfinite(safety_distance) ||
+        !isfinite(free_level))
+        return DART_E_BADARG;
+    if (g->cell_bytes == 8)
+        return edt<double>(*g, threshold, nullptr, (double *)field_out, safety_distance, free_level, sq_scratch,
+                           (cudaStream_t)stream);
+    return edt<float>(*g, threshold, nullptr, (float *)field_out, safety_distance, free_level, sq_scratch,
+                      (cudaStream_t)stream);
 }
 
 } /* extern "C" */

@@ -22,9 +22,12 @@ struct SolveArgs {
     double *x_out, *cost;
     int *nit, *nfev, *status, *task;
     double *acc, *att, *rates, *thrust;
-    /* fused post-solve safety check (is_trajectory_safe on the solved positions); on when
-     * check_map != 0 */
+    /* the obstacle penalty's grid (gradient_mode 2 / 4) */
     dart_grid grid;
+    /* fused post-solve safety check (is_trajectory_safe on the solved positions) against
+     * check_grid; on when check_map != 0.  The same grid as `grid` except in the closed-loop step
+     * with a map, whose penalty grid and collision map are separate */
+    dart_grid check_grid;
     double margin, threshold;
     int *first_hit;
     int check_map; /* 1: run the check (SoA mode: into first_hit; row mode: into the row) */
@@ -32,6 +35,11 @@ struct SolveArgs {
      * advanced with the first control of the new solution; may alias p0 / v0 */
     double *p_next, *v_next;
     double plant_dt;
+    /* collision record of the plant step (off when first_collision == nullptr): the step's path
+     * p -> p_next, sampled at most half a voxel apart, against check_grid (margin, threshold);
+     * a problem whose path collides and whose first_collision is -1 gets `step` */
+    int *first_collision;
+    int step;
     /* the caller promises that every lateral thrust entry of x_warm is exactly zero (solutions
      * this library produced from cold starts): the 7-slot instantiation then serves warm starts
      * too.  The kernel checks the promise per problem and refuses (status 3) where it is broken. */
@@ -330,7 +338,7 @@ se3mpc_solve_kernel(const __grid_constant__ dart_se3mpc_params P, const __grid_c
                 int hit = 0x7fffffff;
 #pragma unroll
                 for (int tt = TPL - 1; tt >= 0; --tt)
-                    if (sv.act[tt] && position_collides(A.grid, sv.x[tt * 9], sv.x[tt * 9 + 1], sv.x[tt * 9 + 2],
+                    if (sv.act[tt] && position_collides(A.check_grid, sv.x[tt * 9], sv.x[tt * 9 + 1], sv.x[tt * 9 + 2],
                                                         A.margin, A.threshold))
                         hit = sv.grp.lane() * TPL + tt;
                 hit = sv.grp.mini(hit);
@@ -388,6 +396,7 @@ se3mpc_solve_kernel(const __grid_constant__ dart_se3mpc_params P, const __grid_c
                  A.status ? A.status + b : nullptr, A.task ? A.task + b : nullptr,
                  A.first_hit ? A.first_hit + b : nullptr, A.ld, A.check_map != 0 && A.first_hit != nullptr);
         }
+        double path[6] = {0.0, 0.0, 0.0, 0.0, 0.0, 0.0}; /* the plant step's p and p' - p */
         if (A.p_next && sv.grp.leader()) {
             /* reference planner model (se3_mpc_planner.py:430-431, :445-459) driven by T_0:
              * a = T_0/m - g e3;  p <- p + v dt + (0.5 a) dt^2;  v <- v + a dt.  Every operation
@@ -399,9 +408,30 @@ se3mpc_solve_kernel(const __grid_constant__ dart_se3mpc_params P, const __grid_c
                  * instead of being kept in 12 registers through the whole solve */
                 const double pc = A.p0[c * A.ld + b], vc = A.v0[c * A.ld + b];
                 const double a = DP_ADD(ddiv(sv.x[6 + c], P.mass), c == 2 ? -P.gravity : -0.0);
-                A.p_next[c * A.ld + b] = DP_ADD(DP_ADD(pc, DP_MUL(vc, dt)), DP_MUL(DP_MUL(0.5, a), dt2));
+                const double pn = DP_ADD(DP_ADD(pc, DP_MUL(vc, dt)), DP_MUL(DP_MUL(0.5, a), dt2));
+                A.p_next[c * A.ld + b] = pn;
                 A.v_next[c * A.ld + b] = DP_ADD(vc, DP_MUL(a, dt));
+                path[c] = pc;
+                path[3 + c] = DP_ADD(pn, -pc);
             }
+        }
+        if (A.p_next && A.first_collision) {
+            /* collision record: q_j = p + (p' - p)(j / S), j = 1..S, S = ceil(|p' - p|_inf / (res/2))
+             * (at least 1, at most 64), every operation individually rounded; lanes strided over j */
+#pragma unroll
+            for (int c = 0; c < 6; ++c) path[c] = sv.grp.bcast(path[c], 0);
+            const double h = 0.5 * A.check_grid.resolution;
+            const double m = fmax(fmax(fabs(path[3]), fabs(path[4])), fabs(path[5]));
+            const int S = (m <= 64.0 * h) ? max(1, (int)ceil(m / h)) : 64; /* NaN: 64 */
+            bool hit = false;
+            for (int j = 1 + sv.grp.lane(); j <= S && !hit; j += LANES) {
+                const double t = (double)j / (double)S;
+                hit = position_collides(A.check_grid, DP_ADD(path[0], DP_MUL(path[3], t)),
+                                        DP_ADD(path[1], DP_MUL(path[4], t)), DP_ADD(path[2], DP_MUL(path[5], t)),
+                                        A.margin, A.threshold);
+            }
+            hit = sv.grp.any(hit);
+            if (hit && sv.grp.leader() && A.first_collision[b] == -1) A.first_collision[b] = A.step;
         }
         DP_TICK(41);
         (void)N;

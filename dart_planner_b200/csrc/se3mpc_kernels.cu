@@ -419,7 +419,7 @@ int dart_se3mpc_solve_batch_map(const dart_se3mpc_params *params, int64_t B, int
     a.x_warm = x_warm; a.warm_mask = warm_mask;
     a.x_out = x_out; a.cost = cost; a.nit = nit; a.nfev = nfev; a.status = status; a.task = task;
     a.acc = acc; a.att = att; a.rates = rates; a.thrust = thrust;
-    if (need_grid) a.grid = *grid;
+    if (need_grid) a.grid = a.check_grid = *grid;
     if (first_hit) {
         a.margin = margin;
         a.threshold = threshold;
@@ -450,6 +450,48 @@ int dart_se3mpc_closed_loop_step(const dart_se3mpc_params *params, int64_t B, in
     a.no_tilt_promise = (warm == 2) ? 1 : 0;
     a.x_out = x; a.cost = cost; a.nit = nit; a.nfev = nfev; a.status = status;
     a.p_next = p; a.v_next = v; a.plant_dt = plant_dt;
+    return launch_solve(params, a, cuda_stream);
+}
+
+static bool grid_ok(const dart_grid *g)
+{
+    return g && g->occ && g->nx > 0 && g->ny > 0 && g->nz > 0 && g->resolution > 0.0 &&
+           (g->cell_bytes == 0 || g->cell_bytes == 4 || g->cell_bytes == 8);
+}
+
+int dart_se3mpc_closed_loop_step_map(const dart_se3mpc_params *params, int64_t B, int64_t ld, double *p,
+                                     double *v, const double *goal, const uint8_t *has_goal, double *x,
+                                     int32_t warm, double *cost, int32_t *nit, int32_t *nfev,
+                                     int32_t *status, double plant_dt, const dart_grid *penalty_grid,
+                                     const dart_grid *check_grid, double margin, double threshold,
+                                     int32_t step, int32_t *first_collision, void *cuda_stream)
+{
+    int rc = check_params(params);
+    if (rc) return rc;
+    if (B < 0 || ld < B || !p || !v || !goal || !x || !(plant_dt > 0.0)) return DART_E_BADARG;
+    const bool penalty = params->gradient_mode == 2 || params->gradient_mode == 4;
+    if (penalty && !grid_ok(penalty_grid)) return DART_E_BADARG;
+    if ((check_grid != nullptr) != (first_collision != nullptr)) return DART_E_BADARG;
+    if (check_grid && !grid_ok(check_grid)) return DART_E_BADARG;
+    /* the promise of warm == 2 (zero lateral thrust) does not hold in the dynamics-consistent modes */
+    if (params->gradient_mode >= 3 && warm == 2) return DART_E_BADARG;
+    if (B == 0) return DART_OK;
+    SolveArgs a;
+    memset(&a, 0, sizeof(a));
+    a.B = B; a.ld = ld;
+    a.p0 = p; a.v0 = v; a.goal = goal; a.has_goal = has_goal;
+    a.x_warm = warm ? x : nullptr;
+    a.no_tilt_promise = (warm == 2) ? 1 : 0;
+    a.x_out = x; a.cost = cost; a.nit = nit; a.nfev = nfev; a.status = status;
+    a.p_next = p; a.v_next = v; a.plant_dt = plant_dt;
+    if (penalty) a.grid = *penalty_grid;
+    if (check_grid) {
+        a.check_grid = *check_grid;
+        a.margin = margin;
+        a.threshold = threshold;
+        a.first_collision = first_collision;
+        a.step = step;
+    }
     return launch_solve(params, a, cuda_stream);
 }
 
@@ -526,7 +568,7 @@ int dart_se3mpc_solve_batch_rows(const dart_se3mpc_params *params, int64_t B, in
     a.p0 = p0; a.v0 = v0; a.goal = goal; a.has_goal = has_goal;
     a.x_warm = x_warm; a.warm_mask = warm_mask;
     a.rows = rows; a.row_stride = row_stride; a.rows_kind = row_kind;
-    if (need_grid) a.grid = *grid;
+    if (need_grid) a.grid = a.check_grid = *grid;
     if (check_map) {
         a.margin = margin;
         a.threshold = threshold;

@@ -243,6 +243,54 @@ class DenseOccupancyGrid:
         step = max(1, pts.shape[0] // max_spheres)
         return [(p.copy(), float(radius)) for p in pts[::step]]
 
+    def _sq_scratch(self):
+        torch = _torch()
+        n = 2 * self.nx * self.ny * self.nz
+        if getattr(self, "_sq", None) is None or self._sq.numel() != n:
+            self._sq = torch.empty(n, dtype=torch.int32, device=self.device)
+        return self._sq
+
+    def signed_distance(self, threshold: float = 0.6, stream=None):
+        """Signed distance to the occupied cells (occupancy > threshold), in metres: (nz, ny, nx)
+        float32 device tensor, positive in free space, negative inside obstacles, from the exact
+        Euclidean distance transform between cell centres (three launches).  With no occupied cell
+        every entry is the box diagonal, with no free cell its negative (header:
+        dart_map_signed_distance).  Recompute after the map changes."""
+        torch = _torch()
+        phi = torch.empty((self.nz, self.ny, self.nx), dtype=torch.float32, device=self.device)
+        g = self._grid()
+        rc = _cabi.lib().dart_map_signed_distance(C.byref(g), float(threshold), phi.data_ptr(),
+                                                  self._sq_scratch().data_ptr(), self._stream(stream))
+        _cabi.check(rc, "dart_map_signed_distance")
+        return phi
+
+    def squared_distance_voxels(self):
+        """(nz, ny, nx) int32 view of the exact squared voxel distances the last `signed_distance` /
+        `clearance_field` call computed: D+ at free cells, -D- at occupied cells."""
+        if getattr(self, "_sq", None) is None:
+            raise ValueError("no distance transform has been computed on this grid")
+        return self._sq[: self.nx * self.ny * self.nz].view(self.nz, self.ny, self.nx)
+
+    def clearance_field(self, safety_distance: float, threshold: float = 0.6, stream=None) -> "DenseOccupancyGrid":
+        """A grid of the same geometry and cell type whose cells are
+        ``0.5 + max(0, safety_distance - phi)`` (phi = ``signed_distance(threshold)``) and whose prior
+        is 0.5.  As the penalty grid of ``plan_batch(..., obstacle_penalty=True)`` or of
+        ``ClosedLoopSim(penalty_grid=...)`` it costs nothing farther than ``safety_distance`` from
+        every obstacle and, unlike the occupancy itself, keeps a gradient inside obstacles."""
+        torch = _torch()
+        out = DenseOccupancyGrid.__new__(DenseOccupancyGrid)
+        out.__dict__.update({k: v for k, v in self.__dict__.items() if k not in ("occ", "_counts", "_sq", "_updated")})
+        out._counts, out._sq = None, None
+        out.prob_prior = 0.5
+        out.total_observations = 0
+        out.occ = torch.empty_like(self.occ)
+        g = self._grid()
+        rc = _cabi.lib().dart_map_clearance_field(C.byref(g), float(threshold), float(safety_distance),
+                                                  out.prob_prior, out.occ.data_ptr(),
+                                                  self._sq_scratch().data_ptr(), self._stream(stream))
+        _cabi.check(rc, "dart_map_clearance_field")
+        return out
+
     def get_mapping_stats(self) -> Dict[str, Any]:
         """:353-363 (total_voxels = cells that left the prior)"""
         nvox = int((self.occ != self.prob_prior).sum().item())

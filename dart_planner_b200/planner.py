@@ -264,7 +264,7 @@ class HostSolution:
 def solve_batch_tensors(params: _cabi.Params, inp, B: int, *, has_goal=None, x_warm=None,
                         warm_mask=None, out=None, meta=None, stream=None,
                         outputs: str = "all", grid=None, safety_margin: float = 1.0,
-                        collision_threshold: float = 0.6, hit=None) -> BatchSolution:
+                        collision_threshold: float = 0.6, hit=None, penalty_grid=None) -> BatchSolution:
     """Lowest Python level: device tensors in, device tensors out, one kernel launch.
 
     inp      : (9, ld) float64 CUDA tensor, rows [p0 xyz | v0 xyz | goal xyz]
@@ -274,6 +274,10 @@ def solve_batch_tensors(params: _cabi.Params, inp, B: int, *, has_goal=None, x_w
     grid     : DenseOccupancyGrid or None; when given, the kernel also runs the reference's
                post-hoc `is_trajectory_safe(positions, safety_margin, collision_threshold)` on
                every solved trajectory (fused, same launch) -> BatchSolution.first_hit
+    penalty_grid : DenseOccupancyGrid or None; the grid the obstacle penalty (gradient_mode 2 / 4)
+               reads instead of ``grid``.  ``grid`` is then only the safety check's, which runs as
+               a second launch (dart_map_traj_safe_batch, the same test as the fused check) on
+               the solved positions
     """
     torch = _torch()
     L = _cabi.lib()
@@ -304,6 +308,9 @@ def solve_batch_tensors(params: _cabi.Params, inp, B: int, *, has_goal=None, x_w
         if hit is None:
             hit = torch.empty(ld, dtype=torch.int32, device=inp.device)
         assert hit.is_cuda and hit.dtype == torch.int32 and hit.shape == (ld,) and hit.is_contiguous()
+    fused = g is not None and penalty_grid is None
+    if penalty_grid is not None:
+        g = penalty_grid._grid()
     with torch.cuda.device(inp.device):
         rc = L.dart_se3mpc_solve_batch_map(
             C.byref(params), B, ld, inp.data_ptr(), inp.data_ptr() + 3 * es, inp.data_ptr() + 6 * es,
@@ -315,10 +322,12 @@ def solve_batch_tensors(params: _cabi.Params, inp, B: int, *, has_goal=None, x_w
             base + (15 * N + 1) * es if derived else None,
             base + (18 * N + 1) * es if derived else None,
             C.byref(g) if g is not None else None, float(safety_margin), float(collision_threshold),
-            hit.data_ptr() if g is not None else None,
+            hit.data_ptr() if fused else None,
             stream.cuda_stream)
     _cabi.check(rc, "dart_se3mpc_solve_batch_map")
-    return BatchSolution(N=N, B=B, out=out, meta=meta, hit=hit if g is not None else None)
+    if grid is not None and not fused:
+        grid.trajectories_safe_soa(out[: 3 * N], B, N, safety_margin, collision_threshold, out=hit, stream=stream)
+    return BatchSolution(N=N, B=B, out=out, meta=meta, hit=hit if grid is not None else None)
 
 
 class BatchWorkspace:
@@ -344,6 +353,7 @@ class BatchWorkspace:
         self.x_warm = None
         self.warm_mask = None
         self.grid, self.safety_margin, self.collision_threshold, self.hit = None, 1.0, 0.6, None
+        self.penalty_grid = None
         self.h_inp = self.h_out = self.h_meta = self.h_rows = None
         # DART_ROWS_FULL / DART_ROWS_CONTROLS / DART_ROWS_SOLUTION
         if outputs not in ("all", "controls", "solution"):
@@ -403,10 +413,13 @@ class BatchWorkspace:
         self.has_goal = torch.ones(self.ld, dtype=torch.uint8, device=self.device)
         self.has_goal[: self.B] = h
 
-    def set_map(self, grid, safety_margin: float = 1.0, collision_threshold: float = 0.6):
-        """Attach a DenseOccupancyGrid: every solve also runs the fused trajectory safety check."""
+    def set_map(self, grid, safety_margin: float = 1.0, collision_threshold: float = 0.6, penalty_grid=None):
+        """Attach a DenseOccupancyGrid: every solve also runs the fused trajectory safety check.
+        ``penalty_grid``: a separate grid for the obstacle penalty (see solve_batch_tensors; SoA
+        solves only)."""
         torch = _torch()
         self.grid, self.safety_margin, self.collision_threshold = grid, safety_margin, collision_threshold
+        self.penalty_grid = penalty_grid
         self.hit = None if grid is None else torch.full((self.ld,), -1, dtype=torch.int32, device=self.device)
 
     def solve_device(self, stream=None) -> BatchSolution:
@@ -414,7 +427,8 @@ class BatchWorkspace:
                                    x_warm=self.x_warm, warm_mask=self.warm_mask, out=self.out,
                                    meta=self.meta, stream=stream, outputs=self.outputs,
                                    grid=self.grid, safety_margin=self.safety_margin,
-                                   collision_threshold=self.collision_threshold, hit=self.hit)
+                                   collision_threshold=self.collision_threshold, hit=self.hit,
+                                   penalty_grid=self.penalty_grid)
 
     def stage_host_inputs(self, p0, v0, goal):
         """Write (B,3) host arrays into the pinned SoA staging block (host-side transpose)."""
@@ -457,6 +471,8 @@ class BatchWorkspace:
         the host on first access), half the bytes; ``outputs="controls"`` gets controls rows:
         thrust vectors, cost and counters only (`HostSolution.from_control_rows`), a fifth."""
         torch = _torch()
+        if self.penalty_grid is not None:
+            raise ValueError("row output has no separate penalty grid")
         if not self.rows_supported:
             raise RuntimeError("row output needs pinned buffers and a horizon of at most 25 steps")
         if self.h_rows is None:
@@ -485,6 +501,8 @@ class BatchWorkspace:
         (the shared block of `ShardedSolver(transport="host_block")`) -- and nothing is returned.
         Asynchronous."""
         torch = _torch()
+        if self.penalty_grid is not None:
+            raise ValueError("row output has no separate penalty grid")
         if self.row_stride <= 0:
             raise RuntimeError("row output needs a horizon of at most 25 steps (64 for controls rows)")
         if rows_ptr is None and getattr(self, "d_rows", None) is None:
@@ -586,7 +604,7 @@ def plan_batch(positions, velocities, goals, config: Optional[SE3MPCConfig] = No
                has_goal=None, x_warm=None, warm_mask=None, gradient_mode: int = 0,
                device=None, outputs: str = "all", to_host: bool = False, grid=None,
                safety_margin: float = 1.0, collision_threshold: float = 0.6,
-               obstacle_penalty: bool = False, dynamics_consistent: bool = False):
+               obstacle_penalty: bool = False, dynamics_consistent: bool = False, penalty_grid=None):
     """Solve B independent SE(3)-MPC problems in one call.
 
     positions, velocities, goals : (B, 3) array-likes (NumPy or torch, host or device)
@@ -603,6 +621,9 @@ def plan_batch(positions, velocities, goals, config: Optional[SE3MPCConfig] = No
              the plant model from (p0, v0) (gradient_mode 3, with ``obstacle_penalty`` mode 4;
              extension).  The P/V rows of the result are that rollout; ``pos_bound`` and
              ``max_velocity`` are not enforced in this mode.
+    penalty_grid : DenseOccupancyGrid the obstacle penalty reads instead of ``grid`` (typically
+             ``grid.clearance_field(d_safe)``; free level = its prior).  ``grid``, if given, is then
+             only the safety check's, run as a second launch on the solved positions.
     Returns a BatchSolution (device) or HostSolution (``to_host=True``).
     """
     cfg = config or SE3MPCConfig()
@@ -610,19 +631,22 @@ def plan_batch(positions, velocities, goals, config: Optional[SE3MPCConfig] = No
         if gradient_mode != 0:
             raise ValueError("dynamics_consistent selects its own gradient mode")
         gradient_mode = 3
+    pen = penalty_grid if penalty_grid is not None else grid
     if obstacle_penalty:
-        if grid is None or gradient_mode not in (0, 3):
-            raise ValueError("obstacle_penalty needs grid= and the reference gradient mode")
+        if pen is None or gradient_mode not in (0, 3):
+            raise ValueError("obstacle_penalty needs grid= or penalty_grid= and the reference gradient mode")
         gradient_mode = 2 if gradient_mode == 0 else 4
+    if penalty_grid is not None and not obstacle_penalty:
+        raise ValueError("penalty_grid= is the obstacle penalty's grid: pass obstacle_penalty=True")
     params = make_params(cfg, mass=mass, gravity=gravity, dt=dt, gradient_mode=gradient_mode,
-                         obstacle_free_level=grid.prob_prior if grid is not None else 0.5)
+                         obstacle_free_level=pen.prob_prior if pen is not None else 0.5)
     B = int(np.shape(positions)[0])
     ws = BatchWorkspace(params, B, device=device, pinned=False, outputs=outputs)
     ws.set_inputs_device(positions, velocities, goals)
     ws.set_has_goal(has_goal)
     ws.set_warm(x_warm, warm_mask)
-    if grid is not None:
-        ws.set_map(grid, safety_margin, collision_threshold)
+    if grid is not None or penalty_grid is not None:
+        ws.set_map(grid, safety_margin, collision_threshold, penalty_grid=penalty_grid)
     sol = ws.solve_device()
     return sol.numpy() if to_host else sol
 

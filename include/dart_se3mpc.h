@@ -65,7 +65,7 @@ typedef struct dart_se3mpc_params {
                                /*    NOT enforced.  Closed-loop step: warm == 2 is refused.     */
                                /*    Horizons 1..16 (DART_E_UNSUPPORTED above).                 */
                                /* 4: mode 3 + the obstacle penalty of mode 2 on the rolled-out  */
-                               /*    positions (needs a grid; not in the closed-loop step)      */
+                               /*    positions (needs a grid; closed loop: _step_map)           */
     int32_t reserved0;
     double dt;                 /* effective planner dt (timing_alignment.py:76-78)         */
     double mass, gravity;      /* 1.5 kg, 9.81 m/s^2 (:149-150)                            */
@@ -208,11 +208,34 @@ int dart_se3mpc_solve_batch_rows(const dart_se3mpc_params *params, int64_t B, in
  * warm start; a problem whose x breaks the promise is not solved and gets status 3.
  * gradient_mode 3: warm == 2 returns DART_E_BADARG (the lateral thrust moves); with
  * plant_dt == params->dt the new state is the solution's P_1 / V_1.  gradient_mode 2 and 4
- * (obstacle penalty: no map argument here) return DART_E_UNSUPPORTED. */
+ * (obstacle penalty: no map argument here; see dart_se3mpc_closed_loop_step_map) return
+ * DART_E_UNSUPPORTED. */
 int dart_se3mpc_closed_loop_step(const dart_se3mpc_params *params, int64_t B, int64_t ld, double *p,
                                  double *v, const double *goal, const uint8_t *has_goal, double *x,
                                  int32_t warm, double *cost, int32_t *nit, int32_t *nfev,
                                  int32_t *status, double plant_dt, void *cuda_stream);
+
+/* The same step against a map (extension), still one launch:
+ *   penalty_grid : the grid of the obstacle penalty, required for gradient_mode 2 and 4 (else
+ *                  DART_E_BADARG) and ignored otherwise -- typically a clearance field
+ *                  (dart_map_clearance_field) with params->obstacle_free_level = its prior;
+ *   check_grid, first_collision : optional together (one without the other: DART_E_BADARG).
+ *                  After the plant step, the path of this step from p to p' is sampled at
+ *                  q_j = p + (p' - p) * (j / S), j = 1..S, S = max(1, ceil(|p' - p|_inf / (0.5 res)))
+ *                  capped at 64 (res = check_grid->resolution; every operation individually
+ *                  rounded), and each q_j is tested with is_trajectory_safe's stencil (margin,
+ *                  threshold, as in dart_map_traj_safe_batch).  A problem whose path collides and
+ *                  whose first_collision [ld] int32 entry is -1 gets `step` there (the caller
+ *                  initialises the entries to -1 and passes its step counter).
+ * warm == 2 is refused (DART_E_BADARG) in gradient_mode 3 and 4.  Everything else as
+ * dart_se3mpc_closed_loop_step; with neither grid the results are the same bits. */
+int dart_se3mpc_closed_loop_step_map(const dart_se3mpc_params *params, int64_t B, int64_t ld,
+                                     double *p, double *v, const double *goal,
+                                     const uint8_t *has_goal, double *x, int32_t warm, double *cost,
+                                     int32_t *nit, int32_t *nfev, int32_t *status, double plant_dt,
+                                     const dart_grid *penalty_grid, const dart_grid *check_grid,
+                                     double margin, double threshold, int32_t step,
+                                     int32_t *first_collision, void *cuda_stream);
 
 /* Same call with every buffer in HOST memory (pageable or pinned).  Up to 512 problems go
  * through a mapped pinned block the kernel reads and writes directly (no copies); larger batches
@@ -287,6 +310,31 @@ int dart_map_update_batch(const dart_grid *g, void *occ_writable, uint64_t *coun
 int dart_map_add_spheres(const dart_grid *g, void *occ_writable, int32_t n,
                          const double *centers, const double *radii, double value,
                          void *cuda_stream);
+
+/* ---- signed distance and clearance field of a grid (extension; the reference has none) ----
+ * Occupied means occ > threshold (is_collision's strict test).  For every cell, D+ is the squared
+ * distance in voxels from its centre to the nearest occupied cell centre and D- the same to the
+ * nearest free cell centre, both exact integers (separable lower envelope of parabolas,
+ * Felzenszwalb-Huttenlocher, integer comparisons only; three launches, x, y, z).  Only cells of
+ * the box are sites: with no occupied cell D+ is the squared box diagonal nx^2+ny^2+nz^2, with no
+ * free cell D- is.
+ *   phi = res * (sqrt(D+) - sqrt(D-))   [m, float32, rounded once from double]
+ * sq_scratch: 2*nx*ny*nz int32 of device memory.  On return its first nx*ny*nz entries hold the
+ * signed squared distance: D+ at a free cell, -D- at an occupied cell (the other one is 0).
+ * phi_out: nx*ny*nz float32 in the grid's cell order, or NULL (then only sq_scratch is written).
+ * DART_E_UNSUPPORTED when nx^2+ny^2+nz^2 >= 2^30 - 1. */
+int dart_map_signed_distance(const dart_grid *g, double threshold, float *phi_out,
+                             int32_t *sq_scratch, void *cuda_stream);
+/* Clearance field for the obstacle penalty of gradient_mode 2 / 4: the same transform, then
+ *   c = free_level + max(0, safety_distance - phi)    (double, from the float32 phi)
+ * stored in the grid's own cell type (cell_bytes) to field_out (nx*ny*nz cells, same order).  Used
+ * as a penalty grid with prior = obstacle_free_level = free_level, a cell farther than
+ * safety_distance from every occupied cell (and every key outside the box) costs nothing and
+ * gives no gradient; inside an obstacle the field keeps rising with the depth.  sq_scratch as
+ * above (and holding the same result on return). */
+int dart_map_clearance_field(const dart_grid *g, double threshold, double safety_distance,
+                             double free_level, void *field_out, int32_t *sq_scratch,
+                             void *cuda_stream);
 
 #ifdef __cplusplus
 }
