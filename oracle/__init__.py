@@ -61,6 +61,7 @@ class Grid(C.Structure):
         ("nx", C.c_int32), ("ny", C.c_int32), ("nz", C.c_int32),
         ("ox", C.c_int32), ("oy", C.c_int32), ("oz", C.c_int32),
         ("resolution", C.c_double), ("prior", C.c_double), ("occ", C.POINTER(C.c_float)),
+        ("occ64", C.POINTER(C.c_double)),
     ]
 
 
@@ -282,13 +283,36 @@ class DenseGrid:
                       float(resolution), float(prior),
                       self.occ.ctypes.data_as(C.POINTER(C.c_float)))
 
+    @classmethod
+    def from_cells(cls, occ, origin_voxel, resolution, prior):
+        """A grid over the given (nz, ny, nx) cells, float32 or float64 (the penalty reads float64
+        cells as stored; the mapper queries read only float32 grids)."""
+        occ = np.ascontiguousarray(occ)
+        assert occ.ndim == 3 and occ.dtype in (np.float32, np.float64)
+        nz, ny, nx = occ.shape
+        self = cls.__new__(cls)
+        self.occ = occ
+        f32 = occ if occ.dtype == np.float32 else None
+        self.g = Grid(nx, ny, nz, origin_voxel[0], origin_voxel[1], origin_voxel[2], float(resolution),
+                      float(prior), None if f32 is None else f32.ctypes.data_as(C.POINTER(C.c_float)),
+                      None if f32 is not None else occ.ctypes.data_as(C.POINTER(C.c_double)))
+        return self
+
+    def _mapper_grid(self):
+        """The grid the mapper queries read: they take float32 cells only."""
+        if not self.g.occ:
+            raise TypeError("the mapper queries read float32 cells; this grid holds float64 cells")
+        return self.g
+
     def add_sphere(self, center, radius, value=0.9):
+        self._mapper_grid()
         c = np.ascontiguousarray(center, dtype=np.float64)
         return lib().orc_add_sphere(C.byref(self.g), _dp(c), float(radius), float(value))
 
     def query(self, pos):
         pos = np.ascontiguousarray(pos, dtype=np.float64).reshape(-1, 3)
-        return np.array([lib().orc_query(C.byref(self.g), _dp(q)) for q in pos])
+        g = self._mapper_grid()
+        return np.array([lib().orc_query(C.byref(g), _dp(q)) for q in pos])
 
     def penalty(self, pos, weight, free_level=0.5):
         """(f, grad[3]) of the obstacle penalty at one position (orc_grid_penalty)."""
@@ -302,7 +326,7 @@ class DenseGrid:
 
     def traj_safe(self, positions, margin, threshold):
         q = np.ascontiguousarray(positions, dtype=np.float64).reshape(-1, 3)
-        return lib().orc_traj_safe(C.byref(self.g), _dp(q), q.shape[0], float(margin),
+        return lib().orc_traj_safe(C.byref(self._mapper_grid()), _dp(q), q.shape[0], float(margin),
                                    float(threshold))
 
 
@@ -316,7 +340,7 @@ def update_map(grid: "DenseGrid", occ64, pos, direction, hit, obs_max_range, map
     h = np.ascontiguousarray(hit, np.float64).reshape(n)
     mr = np.ascontiguousarray(obs_max_range, np.float64).reshape(n)
     assert occ64.dtype == np.float64 and occ64.flags.c_contiguous and occ64.shape == grid.occ.shape
-    return L.orc_update_map(C.byref(grid.g), _dp(occ64), _ip(counts) if counts is not None else None,
+    return L.orc_update_map(C.byref(grid._mapper_grid()), _dp(occ64), _ip(counts) if counts is not None else None,
                             C.c_int64(n), _dp(pos), _dp(d), _dp(h), _dp(mr), C.c_double(float(mapper_max_range)))
 
 

@@ -214,7 +214,8 @@ static double grid_cell(const orc_grid *g, int kx, int ky, int kz)
 {
     const int ix = kx - g->ox, iy = ky - g->oy, iz = kz - g->oz;
     if (ix < 0 || iy < 0 || iz < 0 || ix >= g->nx || iy >= g->ny || iz >= g->nz) return g->prior;
-    return (double)g->occ[((int64_t)iz * g->ny + iy) * g->nx + ix];
+    const int64_t i = ((int64_t)iz * g->ny + iy) * g->nx + ix;
+    return g->occ64 ? g->occ64[i] : (double)g->occ[i];
 }
 
 /* Occupancy-grid obstacle penalty (EXTENSION -- the reference solve has no obstacle term, SURVEY
