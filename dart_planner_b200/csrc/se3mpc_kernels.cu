@@ -190,7 +190,8 @@ int check_params(const dart_se3mpc_params *p)
     if (!p || p->struct_size != (int)sizeof(dart_se3mpc_params)) return DART_E_BADARG;
     if (p->horizon < 1 || p->horizon > 64) return DART_E_UNSUPPORTED;
     if (p->max_corrections < 1 || p->max_corrections > MMAX) return DART_E_UNSUPPORTED;
-    if (p->max_iterations < 0 || p->max_linesearch < 0) return DART_E_BADARG;
+    /* maxls >= 1, as SciPy requires; with 0 every solve would end ABNORMAL after one evaluation */
+    if (p->max_iterations < 0 || p->max_linesearch < 1) return DART_E_BADARG;
     if (p->gradient_mode < 0 || p->gradient_mode > 4) return DART_E_UNSUPPORTED;
     /* dynamics-consistent modes: verified against the oracle up to the 16-lane builds; on 32-lane
      * groups (horizons 17..64) the scan's rounding makes 5-7 % of the solves take other iteration

@@ -47,7 +47,7 @@ typedef struct dart_se3mpc_params {
     int32_t horizon;           /* prediction_horizon N, 1..64                              */
     int32_t max_iterations;    /* maxiter                                                  */
     int32_t max_corrections;   /* SciPy maxcor, 1..10 (SciPy default 10)                   */
-    int32_t max_linesearch;    /* SciPy maxls (default 20)                                 */
+    int32_t max_linesearch;    /* SciPy maxls, >= 1 (default 20; 0 is DART_E_BADARG)       */
     int32_t max_fun;           /* SciPy maxfun (default 15000)                             */
     int32_t gradient_mode;     /* 0: reference gradient (:552-580, inconsistent by design) */
                                /* 1: exact gradient of :516-550 (extension, self-oracle)   */

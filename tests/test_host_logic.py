@@ -92,6 +92,14 @@ def test_bad_arguments_are_rejected_without_a_gpu():
     p.max_corrections = 11
     assert L.dart_se3mpc_solve_batch(C.byref(p), 1, 1, *([None] * 17)) == _cabi.DART_E_UNSUPPORTED
     p.max_corrections = 10
+    # maxls must be positive, as in SciPy.  An empty batch with valid inputs returns after the
+    # argument checks, so DART_OK there tells the accepted values from the refused ones
+    buf = np.zeros(3)
+    empty = lambda: L.dart_se3mpc_solve_batch(C.byref(p), 0, 0, *([buf.ctypes.data] * 3), *([None] * 14))  # noqa: E731
+    for maxls, want in ((0, _cabi.DART_E_BADARG), (-1, _cabi.DART_E_BADARG), (1, _cabi.DART_OK), (20, _cabi.DART_OK)):
+        p.max_linesearch = maxls
+        assert empty() == want, maxls
+    p.max_linesearch = 20
     assert L.dart_se3mpc_solve_batch(C.byref(p), 1, 1, *([None] * 17)) == _cabi.DART_E_BADARG  # null inputs
     p.struct_size = 8
     assert L.dart_se3mpc_solve_batch(C.byref(p), 1, 1, *([None] * 17)) == _cabi.DART_E_BADARG
