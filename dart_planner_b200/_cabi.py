@@ -50,6 +50,14 @@ class Grid(C.Structure):
     ]
 
 
+class Spheres(C.Structure):
+    """Mirror of ``dart_spheres``: the sphere list of gradient_mode 5 / 6."""
+
+    _fields_ = [
+        ("n", C.c_int32), ("reserved", C.c_int32), ("cxyzr", C.c_void_p), ("margin", C.c_double),
+    ]
+
+
 EXPORTS = [
     "dart_abi_version", "dart_last_cuda_error", "dart_se3mpc_default_params",
     "dart_se3mpc_solve_batch", "dart_se3mpc_solve_batch_map", "dart_se3mpc_closed_loop_step",
@@ -58,6 +66,7 @@ EXPORTS = [
     "dart_se3mpc_kernel_info", "dart_map_query_batch", "dart_map_traj_safe_batch",
     "dart_map_trace_ray_batch", "dart_map_update_batch", "dart_map_add_spheres", "dart_fp64_probe", "dart_ddiv_selftest",
     "dart_map_signed_distance", "dart_map_clearance_field", "dart_se3mpc_closed_loop_step_map",
+    "dart_se3mpc_solve_batch_spheres", "dart_se3mpc_solve_batch_host_spheres", "dart_se3mpc_closed_loop_step_spheres",
 ]
 
 _lib = None
@@ -96,6 +105,16 @@ def lib():
     L.dart_se3mpc_closed_loop_step_map.restype = C.c_int
     L.dart_se3mpc_solve_batch_host.argtypes = [C.POINTER(Params), i64] + [vp] * 14
     L.dart_se3mpc_solve_batch_host.restype = C.c_int
+    L.dart_se3mpc_solve_batch_spheres.argtypes = ([C.POINTER(Params), i64, i64] + [vp] * 16 +
+                                                  [C.POINTER(Spheres), C.POINTER(Grid), C.c_double, C.c_double,
+                                                   vp, vp])
+    L.dart_se3mpc_solve_batch_spheres.restype = C.c_int
+    L.dart_se3mpc_solve_batch_host_spheres.argtypes = [C.POINTER(Params), i64] + [vp] * 14 + [C.POINTER(Spheres)]
+    L.dart_se3mpc_solve_batch_host_spheres.restype = C.c_int
+    L.dart_se3mpc_closed_loop_step_spheres.argtypes = ([C.POINTER(Params), i64, i64] + [vp] * 5 + [i32] +
+                                                       [vp] * 4 + [C.c_double, C.POINTER(Spheres), C.POINTER(Grid),
+                                                                    C.c_double, C.c_double, i32, vp, vp])
+    L.dart_se3mpc_closed_loop_step_spheres.restype = C.c_int
     L.dart_se3mpc_extract_batch.argtypes = [C.POINTER(Params), i64, i64] + [vp] * 5 + [i32, vp]
     L.dart_se3mpc_extract_batch.restype = C.c_int
     L.dart_se3mpc_release_thread_workspace.argtypes = []

@@ -47,13 +47,22 @@ class ClosedLoopSim:
                       is_trajectory_safe's stencil (``safety_margin``, ``collision_threshold``).
                       ``first_collision()`` is the first step index at which a drone's path
                       collided, -1 = never.
+      spheres       : (centers (S, 3), radii (S,)): the sphere obstacle penalty of gradient_mode 5
+                      (mode 0 + spheres) or 6 (mode 3 + spheres), which need it, every radius
+                      inflated by ``sphere_margin`` (``dart_se3mpc_closed_loop_step_spheres``; a
+                      ``collision_map`` still judges collisions, typically the same spheres
+                      rasterised by ``add_obstacles``).  Mode 5 keeps the lateral thrust at exactly
+                      zero, so its warm starts use the 7-slot kernel as in mode 0.
     """
 
     def __init__(self, params: _cabi.Params, B: int, plant_dt: Optional[float] = None, device=None, *,
                  penalty_grid=None, collision_map=None, safety_margin: float = 0.0,
-                 collision_threshold: float = 0.6):
-        if int(params.gradient_mode) in (2, 4) and penalty_grid is None:
+                 collision_threshold: float = 0.6, spheres=None, sphere_margin: float = 0.0):
+        gm = int(params.gradient_mode)
+        if gm in (2, 4) and penalty_grid is None:
             raise ValueError("ClosedLoopSim: gradient_mode 2 / 4 need penalty_grid=")
+        if (gm in (5, 6)) != (spheres is not None):
+            raise ValueError("ClosedLoopSim: spheres= goes with gradient_mode 5 / 6, and they need it")
         torch = _torch()
         self.penalty_grid, self.collision_map = penalty_grid, collision_map
         self.safety_margin, self.collision_threshold = float(safety_margin), float(collision_threshold)
@@ -63,6 +72,13 @@ class ClosedLoopSim:
         self.ld = max(32, (self.B + 31) // 32 * 32)
         self.plant_dt = float(params.dt if plant_dt is None else plant_dt)
         self.device = torch.device("cuda", torch.cuda.current_device()) if device is None else torch.device(device)
+        self.spheres = self._spheres_dev = None
+        if spheres is not None:
+            from .planner import sphere_rows
+            rows = sphere_rows(spheres)
+            self._spheres_dev = torch.as_tensor(rows).to(self.device) if len(rows) else None
+            self.spheres = _cabi.Spheres(len(rows), 0, None if self._spheres_dev is None
+                                         else self._spheres_dev.data_ptr(), float(sphere_margin))
         f8 = dict(dtype=torch.float64, device=self.device)
         self.state = torch.zeros((9, self.ld), **f8)            # rows p xyz | v xyz | goal xyz
         self.x = torch.zeros((9 * self.N, self.ld), **f8)       # current solution, reference order
@@ -74,8 +90,13 @@ class ClosedLoopSim:
         # the solutions held in self.x come from cold starts of this solver, so their lateral
         # thrust is exactly zero and stays zero: warm starts may use the 7-slot kernel (warm=2;
         # the kernel verifies).  Anyone writing self.x by hand must clear this flag.
-        self.lateral_thrust_is_zero = int(params.gradient_mode) < 3
+        self.lateral_thrust_is_zero = self._untilted_mode()
         self._lib = _cabi.lib()
+
+    def _untilted_mode(self) -> bool:
+        """Modes whose cold-started lateral thrust stays exactly zero (all but the dynamics-consistent
+        modes 3, 4 and 6)."""
+        return int(self.params.gradient_mode) in (0, 1, 2, 5)
 
     def reset(self, p0, v0, goals):
         torch = _torch()
@@ -87,7 +108,7 @@ class ClosedLoopSim:
         self.nfev_total.zero_()
         self._first_collision.fill_(-1)
         self.steps_done = 0
-        self.lateral_thrust_is_zero = int(self.params.gradient_mode) < 3
+        self.lateral_thrust_is_zero = self._untilted_mode()
 
     def _launch(self, lo: int, hi: int, stream, track_counters: bool):
         """One replanning step of drones [lo, hi) (one launch): solve, store, advance the plant."""
@@ -100,17 +121,22 @@ class ClosedLoopSim:
                 0 if self.steps_done == 0 else (2 if self.lateral_thrust_is_zero else 1), self.cost.data_ptr() + 8 * lo,
                 meta, meta + 4 * self.ld, meta + 8 * self.ld, self.plant_dt)
         with torch.cuda.device(self.device):
-            if self.penalty_grid is None and self.collision_map is None:
+            cg = self.collision_map._grid() if self.collision_map is not None else None
+            record = (C.byref(cg) if cg is not None else None, self.safety_margin, self.collision_threshold,
+                      self.steps_done, self._first_collision.data_ptr() + 4 * lo if cg is not None else None,
+                      stream.cuda_stream)
+            if self.spheres is not None:
+                name = "dart_se3mpc_closed_loop_step_spheres"
+                rc = self._lib.dart_se3mpc_closed_loop_step_spheres(*args, C.byref(self.spheres), *record)
+            elif self.penalty_grid is None and self.collision_map is None:
+                name = "dart_se3mpc_closed_loop_step"
                 rc = self._lib.dart_se3mpc_closed_loop_step(*args, stream.cuda_stream)
             else:
+                name = "dart_se3mpc_closed_loop_step_map"
                 pg = self.penalty_grid._grid() if self.penalty_grid is not None else None
-                cg = self.collision_map._grid() if self.collision_map is not None else None
                 rc = self._lib.dart_se3mpc_closed_loop_step_map(
-                    *args, C.byref(pg) if pg is not None else None, C.byref(cg) if cg is not None else None,
-                    self.safety_margin, self.collision_threshold, self.steps_done,
-                    self._first_collision.data_ptr() + 4 * lo if cg is not None else None, stream.cuda_stream)
-        _cabi.check(rc, "dart_se3mpc_closed_loop_step" if self.penalty_grid is None and self.collision_map is None
-                    else "dart_se3mpc_closed_loop_step_map")
+                    *args, C.byref(pg) if pg is not None else None, *record)
+        _cabi.check(rc, name)
         if track_counters:
             with torch.cuda.stream(stream):
                 self.nfev_total[lo:hi] += self.meta[1, lo:hi]

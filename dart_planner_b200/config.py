@@ -117,7 +117,7 @@ def make_params(cfg: SE3MPCConfig, *, mass: float = 1.5, gravity: float = 9.81,
     p.w_thrust = float(cfg.thrust_weight)
     p.gtol = float(cfg.convergence_tolerance)
     p.ftol = float(cfg.convergence_tolerance * 10)
-    p.w_obstacle = float(cfg.obstacle_weight)          # only read in gradient_modes 2 and 4
+    p.w_obstacle = float(cfg.obstacle_weight)          # only read in gradient_modes 2, 4, 5 and 6
     p.obstacle_free_level = float(obstacle_free_level)
     return p
 

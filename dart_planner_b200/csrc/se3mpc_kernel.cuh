@@ -80,6 +80,12 @@ struct SolveArgs {
     int *prio_list;
     unsigned *prio_count;
     double prio_r2;
+    /* the sphere list of the obstacle penalty (gradient_mode 5 / 6): [n_spheres][4] doubles (cx, cy,
+     * cz, r) of device memory, every radius inflated by sphere_margin.  Last, so that the fields
+     * above keep their offsets; 0 spheres in every launch of the other modes */
+    const double *spheres;
+    int n_spheres;
+    double sphere_margin;
 };
 constexpr int PRIO_CAP = 16384;
 
@@ -177,7 +183,12 @@ se3mpc_solve_kernel(const __grid_constant__ dart_se3mpc_params P, const __grid_c
         bool refused = !alive || idle_lane;
         long long b = b_in;
         SolverT sv(P, sm, ws, wy);
-        if (GM == 2 || GM == 4) {
+        if constexpr (SolverT::SPHERES) {
+            sv.obs.s = A.spheres;
+            sv.obs.n = A.n_spheres;
+            sv.obs.w = P.w_obstacle;
+            sv.obs.margin = A.sphere_margin;
+        } else if constexpr (SolverT::POS_PEN || SolverT::ROLLOUT_PEN) {
             sv.obs.g = A.grid;
             sv.obs.w = P.w_obstacle;
             sv.obs.free_level = P.obstacle_free_level;
@@ -609,10 +620,11 @@ se3mpc_extract_kernel(const __grid_constant__ dart_se3mpc_params P, const __grid
     }
 }
 
-/* the eight instantiations of one lane configuration: [gradient_mode][tilt].  The dynamics-consistent
- * modes 3 / 4 move the lateral thrust, so they exist only with tilt (fn[3][0] = fn[4][0] = null). */
+/* the eleven instantiations of one lane configuration: [gradient_mode][tilt].  The dynamics-consistent
+ * modes 3 / 4 / 6 move the lateral thrust, so they exist only with tilt (fn[3][0] = fn[4][0] =
+ * fn[6][0] = null). */
 struct KernelSet {
-    const void *fn[5][2];
+    const void *fn[7][2];
     const void *extract_fn[2]; /* [tilt] */
     int lanes, tpl, block, minb;
     int gpb;      /* problems per block */
@@ -631,8 +643,12 @@ KernelSet make_kernel_set()
     k.fn[2][0] = (const void *)se3mpc_solve_kernel<LANES, TPL, BLK, MINB, 2, false>;
     k.fn[3][1] = (const void *)se3mpc_solve_kernel<LANES, TPL, BLK, MINB, 3, true>;
     k.fn[4][1] = (const void *)se3mpc_solve_kernel<LANES, TPL, BLK, MINB, 4, true>;
+    k.fn[5][1] = (const void *)se3mpc_solve_kernel<LANES, TPL, BLK, MINB, 5, true>;
+    k.fn[5][0] = (const void *)se3mpc_solve_kernel<LANES, TPL, BLK, MINB, 5, false>;
+    k.fn[6][1] = (const void *)se3mpc_solve_kernel<LANES, TPL, BLK, MINB, 6, true>;
     k.fn[3][0] = nullptr;
     k.fn[4][0] = nullptr;
+    k.fn[6][0] = nullptr;
     k.extract_fn[1] = (const void *)se3mpc_extract_kernel<LANES, TPL, BLK, true>;
     k.extract_fn[0] = (const void *)se3mpc_extract_kernel<LANES, TPL, BLK, false>;
     k.lanes = LANES;

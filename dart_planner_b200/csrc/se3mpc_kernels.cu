@@ -161,7 +161,8 @@ int prepare(KernelChoice *k)
     }
     const int smem = smem_bytes(*k);
     const void *fns[] = {k->set.fn[0][0], k->set.fn[0][1], k->set.fn[1][0], k->set.fn[1][1],
-                         k->set.fn[2][0], k->set.fn[2][1], k->set.fn[3][1], k->set.fn[4][1]};
+                         k->set.fn[2][0], k->set.fn[2][1], k->set.fn[3][1], k->set.fn[4][1],
+                         k->set.fn[5][0], k->set.fn[5][1], k->set.fn[6][1]};
     for (const void *fn : fns) {
         e = cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
         if (e != cudaSuccess) return set_err(e, "cudaFuncSetAttribute(smem)");
@@ -185,21 +186,43 @@ int prepare(KernelChoice *k)
     return DART_OK;
 }
 
-int check_params(const dart_se3mpc_params *p)
+/* the dynamics-consistent modes: thrusts are the only variables, P / V their rollout */
+bool rollout_mode(int gm) { return gm == 3 || gm == 4 || gm == 6; }
+
+/* spheres: the caller is one of the _spheres entries, which serve modes 5 and 6 only; every other
+ * entry serves modes 0..4 */
+int check_params(const dart_se3mpc_params *p, bool spheres = false)
 {
     if (!p || p->struct_size != (int)sizeof(dart_se3mpc_params)) return DART_E_BADARG;
     if (p->horizon < 1 || p->horizon > 64) return DART_E_UNSUPPORTED;
     if (p->max_corrections < 1 || p->max_corrections > MMAX) return DART_E_UNSUPPORTED;
     /* maxls >= 1, as SciPy requires; with 0 every solve would end ABNORMAL after one evaluation */
     if (p->max_iterations < 0 || p->max_linesearch < 1) return DART_E_BADARG;
-    if (p->gradient_mode < 0 || p->gradient_mode > 4) return DART_E_UNSUPPORTED;
+    if (spheres) {
+        if (p->gradient_mode != 5 && p->gradient_mode != 6) return DART_E_BADARG;
+    } else if (p->gradient_mode < 0 || p->gradient_mode > 4)
+        return DART_E_UNSUPPORTED;
     /* dynamics-consistent modes: verified against the oracle up to the 16-lane builds; on 32-lane
      * groups (horizons 17..64) the scan's rounding makes 5-7 % of the solves take other iteration
      * counts than the sequential oracle at tolerance 1e-3 (DESIGN.md 5c) */
-    if (p->gradient_mode >= 3 && p->horizon > 16) return DART_E_UNSUPPORTED;
+    if (rollout_mode(p->gradient_mode) && p->horizon > 16) return DART_E_UNSUPPORTED;
     if (!(p->dt > 0.0) || !(p->mass > 0.0)) return DART_E_BADARG;
     if (!(p->gtol >= 0.0)) return DART_E_BADARG; /* the Cauchy step relies on it (se3mpc_core.cuh) */
     return DART_OK;
+}
+
+int check_spheres(const dart_spheres *s)
+{
+    if (!s || s->n < 0 || (s->n > 0 && !s->cxyzr)) return DART_E_BADARG;
+    return DART_OK;
+}
+
+void set_spheres(SolveArgs &a, const dart_spheres *s)
+{
+    if (!s) return;
+    a.spheres = s->cxyzr;
+    a.n_spheres = s->n;
+    a.sphere_margin = s->margin;
 }
 
 long long grid_for(const KernelChoice &k, long long B)
@@ -368,9 +391,14 @@ static int launch_solve(const dart_se3mpc_params *params, const SolveArgs &a, vo
         }
     }
     /* never the 7-slot instantiation in the dynamics-consistent modes: their lateral thrust moves */
-    const int cold = ((a.x_warm == nullptr || a.no_tilt_promise) && params->gradient_mode < 3 &&
+    const int cold = ((a.x_warm == nullptr || a.no_tilt_promise) && !rollout_mode(params->gradient_mode) &&
                       !getenv("DART_SE3MPC_NO_COLD")) ? 0 : 1;
-    const void *fn = k->set.fn[params->gradient_mode][cold];
+    /* an empty sphere list runs the plain mode's own kernel (mode 5 -> 0, 6 -> 3): the same results
+     * bit for bit, which a separate kernel cannot promise -- ptxas contracts the plain products and
+     * sums of the shared solver code kernel by kernel (DESIGN.md 5e) */
+    int gm = params->gradient_mode;
+    if ((gm == 5 || gm == 6) && a.n_spheres == 0) gm = (gm == 5) ? 0 : 3;
+    const void *fn = k->set.fn[gm][cold];
     cudaError_t e;
     if (prio_event) {
         /* programmatic dependent launch: the solve may begin while the scan in front of it runs */
@@ -396,17 +424,19 @@ static int launch_solve(const dart_se3mpc_params *params, const SolveArgs &a, vo
     return DART_OK;
 }
 
-int dart_se3mpc_solve_batch_map(const dart_se3mpc_params *params, int64_t B, int64_t ld,
-                                const double *p0, const double *v0, const double *goal,
-                                const uint8_t *has_goal, const double *x_warm,
-                                const uint8_t *warm_mask, double *x_out, double *cost, int32_t *nit,
-                                int32_t *nfev, int32_t *status, int32_t *task, double *acc,
-                                double *att, double *rates, double *thrust, const dart_grid *grid,
-                                double margin, double threshold, int32_t *first_hit,
-                                void *cuda_stream)
+/* the device solve of dart_se3mpc_solve_batch_map (spheres == NULL) and
+ * dart_se3mpc_solve_batch_spheres */
+static int solve_batch_impl(const dart_se3mpc_params *params, int64_t B, int64_t ld, const double *p0,
+                            const double *v0, const double *goal, const uint8_t *has_goal,
+                            const double *x_warm, const uint8_t *warm_mask, double *x_out, double *cost,
+                            int32_t *nit, int32_t *nfev, int32_t *status, int32_t *task, double *acc,
+                            double *att, double *rates, double *thrust, const dart_grid *grid, double margin,
+                            double threshold, int32_t *first_hit, const dart_spheres *spheres,
+                            void *cuda_stream)
 {
-    int rc = check_params(params);
+    int rc = check_params(params, spheres != nullptr);
     if (rc) return rc;
+    if (spheres && (rc = check_spheres(spheres))) return rc;
     if (B < 0 || ld < B || !p0 || !v0 || !goal) return DART_E_BADARG;
     const bool need_grid = first_hit != nullptr || params->gradient_mode == 2 || params->gradient_mode == 4;
     if (need_grid && (!grid || !grid->occ || grid->nx <= 0 || grid->ny <= 0 || grid->nz <= 0 ||
@@ -427,7 +457,37 @@ int dart_se3mpc_solve_batch_map(const dart_se3mpc_params *params, int64_t B, int
         a.first_hit = first_hit;
         a.check_map = 1;
     }
+    set_spheres(a, spheres);
     return launch_solve(params, a, cuda_stream);
+}
+
+int dart_se3mpc_solve_batch_map(const dart_se3mpc_params *params, int64_t B, int64_t ld,
+                                const double *p0, const double *v0, const double *goal,
+                                const uint8_t *has_goal, const double *x_warm,
+                                const uint8_t *warm_mask, double *x_out, double *cost, int32_t *nit,
+                                int32_t *nfev, int32_t *status, int32_t *task, double *acc,
+                                double *att, double *rates, double *thrust, const dart_grid *grid,
+                                double margin, double threshold, int32_t *first_hit,
+                                void *cuda_stream)
+{
+    return solve_batch_impl(params, B, ld, p0, v0, goal, has_goal, x_warm, warm_mask, x_out, cost, nit, nfev,
+                            status, task, acc, att, rates, thrust, grid, margin, threshold, first_hit, nullptr,
+                            cuda_stream);
+}
+
+int dart_se3mpc_solve_batch_spheres(const dart_se3mpc_params *params, int64_t B, int64_t ld,
+                                    const double *p0, const double *v0, const double *goal,
+                                    const uint8_t *has_goal, const double *x_warm,
+                                    const uint8_t *warm_mask, double *x_out, double *cost, int32_t *nit,
+                                    int32_t *nfev, int32_t *status, int32_t *task, double *acc,
+                                    double *att, double *rates, double *thrust, const dart_spheres *spheres,
+                                    const dart_grid *grid, double margin, double threshold,
+                                    int32_t *first_hit, void *cuda_stream)
+{
+    if (!spheres) return DART_E_BADARG;
+    return solve_batch_impl(params, B, ld, p0, v0, goal, has_goal, x_warm, warm_mask, x_out, cost, nit, nfev,
+                            status, task, acc, att, rates, thrust, grid, margin, threshold, first_hit, spheres,
+                            cuda_stream);
 }
 
 int dart_se3mpc_closed_loop_step(const dart_se3mpc_params *params, int64_t B, int64_t ld, double *p,
@@ -460,22 +520,25 @@ static bool grid_ok(const dart_grid *g)
            (g->cell_bytes == 0 || g->cell_bytes == 4 || g->cell_bytes == 8);
 }
 
-int dart_se3mpc_closed_loop_step_map(const dart_se3mpc_params *params, int64_t B, int64_t ld, double *p,
-                                     double *v, const double *goal, const uint8_t *has_goal, double *x,
-                                     int32_t warm, double *cost, int32_t *nit, int32_t *nfev,
-                                     int32_t *status, double plant_dt, const dart_grid *penalty_grid,
-                                     const dart_grid *check_grid, double margin, double threshold,
-                                     int32_t step, int32_t *first_collision, void *cuda_stream)
+/* the step of dart_se3mpc_closed_loop_step_map (spheres == NULL) and
+ * dart_se3mpc_closed_loop_step_spheres */
+static int closed_loop_step_impl(const dart_se3mpc_params *params, int64_t B, int64_t ld, double *p, double *v,
+                                 const double *goal, const uint8_t *has_goal, double *x, int32_t warm,
+                                 double *cost, int32_t *nit, int32_t *nfev, int32_t *status, double plant_dt,
+                                 const dart_grid *penalty_grid, const dart_spheres *spheres,
+                                 const dart_grid *check_grid, double margin, double threshold, int32_t step,
+                                 int32_t *first_collision, void *cuda_stream)
 {
-    int rc = check_params(params);
+    int rc = check_params(params, spheres != nullptr);
     if (rc) return rc;
+    if (spheres && (rc = check_spheres(spheres))) return rc;
     if (B < 0 || ld < B || !p || !v || !goal || !x || !(plant_dt > 0.0)) return DART_E_BADARG;
     const bool penalty = params->gradient_mode == 2 || params->gradient_mode == 4;
     if (penalty && !grid_ok(penalty_grid)) return DART_E_BADARG;
     if ((check_grid != nullptr) != (first_collision != nullptr)) return DART_E_BADARG;
     if (check_grid && !grid_ok(check_grid)) return DART_E_BADARG;
     /* the promise of warm == 2 (zero lateral thrust) does not hold in the dynamics-consistent modes */
-    if (params->gradient_mode >= 3 && warm == 2) return DART_E_BADARG;
+    if (rollout_mode(params->gradient_mode) && warm == 2) return DART_E_BADARG;
     if (B == 0) return DART_OK;
     SolveArgs a;
     memset(&a, 0, sizeof(a));
@@ -493,7 +556,33 @@ int dart_se3mpc_closed_loop_step_map(const dart_se3mpc_params *params, int64_t B
         a.first_collision = first_collision;
         a.step = step;
     }
+    set_spheres(a, spheres);
     return launch_solve(params, a, cuda_stream);
+}
+
+int dart_se3mpc_closed_loop_step_map(const dart_se3mpc_params *params, int64_t B, int64_t ld, double *p,
+                                     double *v, const double *goal, const uint8_t *has_goal, double *x,
+                                     int32_t warm, double *cost, int32_t *nit, int32_t *nfev,
+                                     int32_t *status, double plant_dt, const dart_grid *penalty_grid,
+                                     const dart_grid *check_grid, double margin, double threshold,
+                                     int32_t step, int32_t *first_collision, void *cuda_stream)
+{
+    return closed_loop_step_impl(params, B, ld, p, v, goal, has_goal, x, warm, cost, nit, nfev, status, plant_dt,
+                                 penalty_grid, nullptr, check_grid, margin, threshold, step, first_collision,
+                                 cuda_stream);
+}
+
+int dart_se3mpc_closed_loop_step_spheres(const dart_se3mpc_params *params, int64_t B, int64_t ld, double *p,
+                                         double *v, const double *goal, const uint8_t *has_goal, double *x,
+                                         int32_t warm, double *cost, int32_t *nit, int32_t *nfev,
+                                         int32_t *status, double plant_dt, const dart_spheres *spheres,
+                                         const dart_grid *check_grid, double margin, double threshold,
+                                         int32_t step, int32_t *first_collision, void *cuda_stream)
+{
+    if (!spheres) return DART_E_BADARG;
+    return closed_loop_step_impl(params, B, ld, p, v, goal, has_goal, x, warm, cost, nit, nfev, status, plant_dt,
+                                 nullptr, spheres, check_grid, margin, threshold, step, first_collision,
+                                 cuda_stream);
 }
 
 int dart_se3mpc_solve_batch(const dart_se3mpc_params *params, int64_t B, int64_t ld,
@@ -587,6 +676,7 @@ struct HostWs {
     size_t pin_cap = 0;
     cudaStream_t stream = nullptr;
     cudaStream_t stream2 = nullptr; /* second lane of the chunk pipeline (large batches) */
+    cudaEvent_t spheres_up = nullptr; /* the sphere list's upload, awaited by the second lane */
     int device = -1;                /* the device everything above belongs to */
 };
 thread_local HostWs g_ws;
@@ -631,20 +721,24 @@ void dart_se3mpc_release_thread_workspace(void)
         if (g_ws.dev) cudaFree(g_ws.dev);
         if (g_ws.stream) cudaStreamDestroy(g_ws.stream);
         if (g_ws.stream2) cudaStreamDestroy(g_ws.stream2);
+        if (g_ws.spheres_up) cudaEventDestroy(g_ws.spheres_up);
         cudaSetDevice(cur);
     }
     if (g_ws.pin) cudaFreeHost(g_ws.pin);
     g_ws = HostWs();
 }
 
-int dart_se3mpc_solve_batch_host(const dart_se3mpc_params *params, int64_t B,
-                                 const double *p0, const double *v0, const double *goal,
-                                 const uint8_t *has_goal, const double *x_warm, double *x_out,
-                                 double *cost, int32_t *nit, int32_t *nfev, int32_t *status,
-                                 double *acc, double *att, double *rates, double *thrust)
+/* the host entry of dart_se3mpc_solve_batch_host (spheres == NULL) and
+ * dart_se3mpc_solve_batch_host_spheres (the list in host memory: staged behind the workspace) */
+static int solve_batch_host_impl(const dart_se3mpc_params *params, int64_t B, const double *p0, const double *v0,
+                                 const double *goal, const uint8_t *has_goal, const double *x_warm,
+                                 double *x_out, double *cost, int32_t *nit, int32_t *nfev, int32_t *status,
+                                 double *acc, double *att, double *rates, double *thrust,
+                                 const dart_spheres *spheres)
 {
-    int rc = check_params(params);
+    int rc = check_params(params, spheres != nullptr);
     if (rc) return rc;
+    if (spheres && (rc = check_spheres(spheres))) return rc;
     if (B < 0 || !p0 || !v0 || !goal) return DART_E_BADARG;
     if (B == 0) return DART_OK;
     const size_t N = (size_t)params->horizon;
@@ -655,6 +749,10 @@ int dart_se3mpc_solve_batch_host(const dart_se3mpc_params *params, int64_t B,
     const bool staged = B <= 512;
     const size_t Bp = staged ? (size_t)((B + 3) / 4 * 4) : (size_t)((B + 31) / 32 * 32);
     const WsLayout L((int)N, Bp);
+    /* the sphere list, if any, follows the workspace: [n][4] doubles at a 16-byte offset */
+    const size_t sph_off = (L.bytes + 15) / 16 * 16;
+    const size_t sph_bytes = spheres ? (size_t)spheres->n * 4 * sizeof(double) : 0;
+    const size_t ws_bytes = sph_off + sph_bytes;
     cudaError_t e;
     {
         int dev = 0;
@@ -669,11 +767,13 @@ int dart_se3mpc_solve_batch_host(const dart_se3mpc_params *params, int64_t B,
                 if (g_ws.dev) cudaFree(g_ws.dev);
                 if (g_ws.stream) cudaStreamDestroy(g_ws.stream);
                 if (g_ws.stream2) cudaStreamDestroy(g_ws.stream2);
+                if (g_ws.spheres_up) cudaEventDestroy(g_ws.spheres_up);
                 cudaSetDevice(dev);
             }
             g_ws.dev = nullptr;
             g_ws.cap = 0;
             g_ws.stream = g_ws.stream2 = nullptr;
+            g_ws.spheres_up = nullptr;
             g_ws.device = dev;
         }
     }
@@ -681,21 +781,21 @@ int dart_se3mpc_solve_batch_host(const dart_se3mpc_params *params, int64_t B,
         e = cudaStreamCreateWithFlags(&g_ws.stream, cudaStreamNonBlocking);
         if (e != cudaSuccess) return set_err(e, "cudaStreamCreate");
     }
-    if (!staged && g_ws.cap < L.bytes) {
+    if (!staged && g_ws.cap < ws_bytes) {
         if (g_ws.dev) cudaFree(g_ws.dev);
         g_ws.dev = nullptr;
         g_ws.cap = 0;
-        e = cudaMalloc(&g_ws.dev, L.bytes);
+        e = cudaMalloc(&g_ws.dev, ws_bytes);
         if (e != cudaSuccess) return set_err(e, "cudaMalloc(workspace)");
-        g_ws.cap = L.bytes;
+        g_ws.cap = ws_bytes;
     }
-    if (staged && g_ws.pin_cap < L.bytes) {
+    if (staged && g_ws.pin_cap < ws_bytes) {
         if (g_ws.pin) cudaFreeHost(g_ws.pin);
         g_ws.pin = nullptr;
         g_ws.pin_cap = 0;
-        e = cudaHostAlloc(&g_ws.pin, L.bytes, cudaHostAllocMapped | cudaHostAllocPortable);
+        e = cudaHostAlloc(&g_ws.pin, ws_bytes, cudaHostAllocMapped | cudaHostAllocPortable);
         if (e != cudaSuccess) return set_err(e, "cudaHostAlloc(staging)");
-        g_ws.pin_cap = L.bytes;
+        g_ws.pin_cap = ws_bytes;
     }
     cudaStream_t s = g_ws.stream;
     char *base = (char *)g_ws.dev;
@@ -713,6 +813,19 @@ int dart_se3mpc_solve_batch_host(const dart_se3mpc_params *params, int64_t B,
     int32_t *d_nit = (int32_t *)(base + L.int_off), *d_nfev = d_nit + Bp, *d_status = d_nfev + Bp,
             *d_task = d_status + Bp;
     uint8_t *d_hg = (uint8_t *)(base + L.hg_off);
+    /* the device copy of the list the solves read (uploaded once per call) */
+    dart_spheres dsph;
+    if (spheres) {
+        dsph = *spheres;
+        dsph.cxyzr = sph_bytes ? (const double *)(base + sph_off) : nullptr;
+        if (sph_bytes && staged)
+            memcpy((char *)g_ws.pin + sph_off, spheres->cxyzr, sph_bytes);
+        else if (sph_bytes) {
+            e = cudaMemcpyAsync(base + sph_off, spheres->cxyzr, sph_bytes, cudaMemcpyHostToDevice, s);
+            if (e != cudaSuccess) return set_err(e, "cudaMemcpyAsync H2D (spheres)");
+        }
+    }
+    const dart_spheres *dsp = spheres ? &dsph : nullptr;
     if (!staged && B >= 65536) {
         /* Large batch: chunks of 32768 problems alternate between two streams, each doing its own
          * pitched H2D rows -> solve -> pitched D2H rows, so the read-back of chunk i (the
@@ -721,6 +834,15 @@ int dart_se3mpc_solve_batch_host(const dart_se3mpc_params *params, int64_t B,
         if (!g_ws.stream2) {
             e = cudaStreamCreateWithFlags(&g_ws.stream2, cudaStreamNonBlocking);
             if (e != cudaSuccess) return set_err(e, "cudaStreamCreate");
+        }
+        if (sph_bytes) { /* the list was uploaded on the first lane: the second waits for it */
+            if (!g_ws.spheres_up) {
+                e = cudaEventCreateWithFlags(&g_ws.spheres_up, cudaEventDisableTiming);
+                if (e != cudaSuccess) return set_err(e, "cudaEventCreate(spheres)");
+            }
+            e = cudaEventRecord(g_ws.spheres_up, g_ws.stream);
+            if (e == cudaSuccess) e = cudaStreamWaitEvent(g_ws.stream2, g_ws.spheres_up, 0);
+            if (e != cudaSuccess) return set_err(e, "cudaStreamWaitEvent(spheres)");
         }
         const int64_t chunk = 32768;
         int ci = 0;
@@ -756,13 +878,13 @@ int dart_se3mpc_solve_batch_host(const dart_se3mpc_params *params, int64_t B,
             ROWS_H2D(d_goal, goal, 3, 8);
             if (has_goal) ROWS_H2D(d_hg, has_goal, 1, 1);
             if (x_warm) ROWS_H2D(d_xw, x_warm, 9 * N, 8);
-            rc = dart_se3mpc_solve_batch(params, cb, (int64_t)Bp, d_p0 + c0, d_v0 + c0, d_goal + c0,
-                                         has_goal ? d_hg + c0 : nullptr, x_warm ? d_xw + c0 : nullptr, nullptr,
-                                         x_out ? d_x + c0 : nullptr, cost ? d_cost + c0 : nullptr,
-                                         nit ? d_nit + c0 : nullptr, nfev ? d_nfev + c0 : nullptr,
-                                         status ? d_status + c0 : nullptr, nullptr, acc ? d_acc + c0 : nullptr,
-                                         att ? d_att + c0 : nullptr, rates ? d_rates + c0 : nullptr,
-                                         thrust ? d_thr + c0 : nullptr, (void *)cs);
+            rc = solve_batch_impl(params, cb, (int64_t)Bp, d_p0 + c0, d_v0 + c0, d_goal + c0,
+                                  has_goal ? d_hg + c0 : nullptr, x_warm ? d_xw + c0 : nullptr, nullptr,
+                                  x_out ? d_x + c0 : nullptr, cost ? d_cost + c0 : nullptr,
+                                  nit ? d_nit + c0 : nullptr, nfev ? d_nfev + c0 : nullptr,
+                                  status ? d_status + c0 : nullptr, nullptr, acc ? d_acc + c0 : nullptr,
+                                  att ? d_att + c0 : nullptr, rates ? d_rates + c0 : nullptr,
+                                  thrust ? d_thr + c0 : nullptr, nullptr, 0.0, 0.0, nullptr, dsp, (void *)cs);
             if (rc) return drain(), rc;
             ROWS_D2H(x_out, d_x, 9 * N, 8);
             ROWS_D2H(cost, d_cost, 1, 8);
@@ -803,13 +925,13 @@ int dart_se3mpc_solve_batch_host(const dart_se3mpc_params *params, int64_t B,
 #undef H2D
     }
     const bool all = false; /* only the rows the caller asked for are computed and written */
-    rc = dart_se3mpc_solve_batch(params, B, (int64_t)Bp, d_p0, d_v0, d_goal, has_goal ? d_hg : nullptr,
-                                 x_warm ? d_xw : nullptr, nullptr, (all || x_out) ? d_x : nullptr,
-                                 (all || cost) ? d_cost : nullptr, (all || nit) ? d_nit : nullptr,
-                                 (all || nfev) ? d_nfev : nullptr, (all || status) ? d_status : nullptr,
-                                 nullptr, (all || acc) ? d_acc : nullptr, (all || att) ? d_att : nullptr,
-                                 (all || rates) ? d_rates : nullptr, (all || thrust) ? d_thr : nullptr,
-                                 (void *)s);
+    rc = solve_batch_impl(params, B, (int64_t)Bp, d_p0, d_v0, d_goal, has_goal ? d_hg : nullptr,
+                          x_warm ? d_xw : nullptr, nullptr, (all || x_out) ? d_x : nullptr,
+                          (all || cost) ? d_cost : nullptr, (all || nit) ? d_nit : nullptr,
+                          (all || nfev) ? d_nfev : nullptr, (all || status) ? d_status : nullptr,
+                          nullptr, (all || acc) ? d_acc : nullptr, (all || att) ? d_att : nullptr,
+                          (all || rates) ? d_rates : nullptr, (all || thrust) ? d_thr : nullptr,
+                          nullptr, 0.0, 0.0, nullptr, dsp, (void *)s);
     if (rc) return rc;
     if (staged) {
         char *h = (char *)g_ws.pin;
@@ -851,6 +973,28 @@ int dart_se3mpc_solve_batch_host(const dart_se3mpc_params *params, int64_t B,
     e = cudaStreamSynchronize(s);
     if (e != cudaSuccess) return set_err(e, "cudaStreamSynchronize");
     return DART_OK;
+}
+
+int dart_se3mpc_solve_batch_host(const dart_se3mpc_params *params, int64_t B,
+                                 const double *p0, const double *v0, const double *goal,
+                                 const uint8_t *has_goal, const double *x_warm, double *x_out,
+                                 double *cost, int32_t *nit, int32_t *nfev, int32_t *status,
+                                 double *acc, double *att, double *rates, double *thrust)
+{
+    return solve_batch_host_impl(params, B, p0, v0, goal, has_goal, x_warm, x_out, cost, nit, nfev, status, acc,
+                                 att, rates, thrust, nullptr);
+}
+
+int dart_se3mpc_solve_batch_host_spheres(const dart_se3mpc_params *params, int64_t B,
+                                         const double *p0, const double *v0, const double *goal,
+                                         const uint8_t *has_goal, const double *x_warm, double *x_out,
+                                         double *cost, int32_t *nit, int32_t *nfev, int32_t *status,
+                                         double *acc, double *att, double *rates, double *thrust,
+                                         const dart_spheres *spheres)
+{
+    if (!spheres) return DART_E_BADARG;
+    return solve_batch_host_impl(params, B, p0, v0, goal, has_goal, x_warm, x_out, cost, nit, nfev, status, acc,
+                                 att, rates, thrust, spheres);
 }
 
 } /* extern "C" */

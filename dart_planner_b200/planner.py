@@ -261,10 +261,23 @@ class HostSolution:
         return self.status == 0
 
 
+def sphere_rows(spheres) -> np.ndarray:
+    """(centers (S, 3), radii (S,)) from NumPy or torch -> the (S, 4) float64 list [cx cy cz r] of
+    ``dart_spheres``."""
+    centers, radii = spheres
+    to_np = lambda a: a.detach().cpu().numpy() if hasattr(a, "detach") else np.asarray(a)  # noqa: E731
+    c = np.asarray(to_np(centers), np.float64).reshape(-1, 3)
+    r = np.asarray(to_np(radii), np.float64).reshape(-1)
+    if len(r) != len(c):
+        raise ValueError("spheres: centers (S, 3) and radii (S,) must have the same length")
+    return np.ascontiguousarray(np.concatenate([c, r[:, None]], axis=1))
+
+
 def solve_batch_tensors(params: _cabi.Params, inp, B: int, *, has_goal=None, x_warm=None,
                         warm_mask=None, out=None, meta=None, stream=None,
                         outputs: str = "all", grid=None, safety_margin: float = 1.0,
-                        collision_threshold: float = 0.6, hit=None, penalty_grid=None) -> BatchSolution:
+                        collision_threshold: float = 0.6, hit=None, penalty_grid=None,
+                        spheres: Optional[_cabi.Spheres] = None) -> BatchSolution:
     """Lowest Python level: device tensors in, device tensors out, one kernel launch.
 
     inp      : (9, ld) float64 CUDA tensor, rows [p0 xyz | v0 xyz | goal xyz]
@@ -278,6 +291,8 @@ def solve_batch_tensors(params: _cabi.Params, inp, B: int, *, has_goal=None, x_w
                reads instead of ``grid``.  ``grid`` is then only the safety check's, which runs as
                a second launch (dart_map_traj_safe_batch, the same test as the fused check) on
                the solved positions
+    spheres  : _cabi.Spheres over a device list, or None; the sphere penalty of gradient_mode 5 / 6
+               (``grid`` then serves only the fused safety check)
     """
     torch = _torch()
     L = _cabi.lib()
@@ -311,20 +326,22 @@ def solve_batch_tensors(params: _cabi.Params, inp, B: int, *, has_goal=None, x_w
     fused = g is not None and penalty_grid is None
     if penalty_grid is not None:
         g = penalty_grid._grid()
-    with torch.cuda.device(inp.device):
-        rc = L.dart_se3mpc_solve_batch_map(
-            C.byref(params), B, ld, inp.data_ptr(), inp.data_ptr() + 3 * es, inp.data_ptr() + 6 * es,
+    args = (C.byref(params), B, ld, inp.data_ptr(), inp.data_ptr() + 3 * es, inp.data_ptr() + 6 * es,
             _ptr(has_goal), _ptr(x_warm), _ptr(warm_mask),
             base, base + 9 * N * es,
             meta.data_ptr(), meta.data_ptr() + 4 * ld, meta.data_ptr() + 8 * ld, meta.data_ptr() + 12 * ld,
             base + (9 * N + 1) * es if derived else None,
             base + (12 * N + 1) * es if derived else None,
             base + (15 * N + 1) * es if derived else None,
-            base + (18 * N + 1) * es if derived else None,
-            C.byref(g) if g is not None else None, float(safety_margin), float(collision_threshold),
-            hit.data_ptr() if fused else None,
-            stream.cuda_stream)
-    _cabi.check(rc, "dart_se3mpc_solve_batch_map")
+            base + (18 * N + 1) * es if derived else None)
+    check = (C.byref(g) if g is not None else None, float(safety_margin), float(collision_threshold),
+             hit.data_ptr() if fused else None, stream.cuda_stream)
+    with torch.cuda.device(inp.device):
+        if spheres is None:
+            rc = L.dart_se3mpc_solve_batch_map(*args, *check)
+        else:
+            rc = L.dart_se3mpc_solve_batch_spheres(*args, C.byref(spheres), *check)
+    _cabi.check(rc, "dart_se3mpc_solve_batch_map" if spheres is None else "dart_se3mpc_solve_batch_spheres")
     if grid is not None and not fused:
         grid.trajectories_safe_soa(out[: 3 * N], B, N, safety_margin, collision_threshold, out=hit, stream=stream)
     return BatchSolution(N=N, B=B, out=out, meta=meta, hit=hit if grid is not None else None)
@@ -354,6 +371,7 @@ class BatchWorkspace:
         self.warm_mask = None
         self.grid, self.safety_margin, self.collision_threshold, self.hit = None, 1.0, 0.6, None
         self.penalty_grid = None
+        self.spheres = self.spheres_dev = None
         self.h_inp = self.h_out = self.h_meta = self.h_rows = None
         # DART_ROWS_FULL / DART_ROWS_CONTROLS / DART_ROWS_SOLUTION
         if outputs not in ("all", "controls", "solution"):
@@ -422,13 +440,24 @@ class BatchWorkspace:
         self.penalty_grid = penalty_grid
         self.hit = None if grid is None else torch.full((self.ld,), -1, dtype=torch.int32, device=self.device)
 
+    def set_spheres(self, spheres, margin: float = 0.0):
+        """The sphere list of the obstacle penalty (gradient_mode 5 / 6): (centers (S, 3), radii (S,)),
+        every radius inflated by ``margin``; uploaded once, used by every SoA solve.  None removes it."""
+        torch = _torch()
+        if spheres is None:
+            self.spheres = self.spheres_dev = None
+            return
+        rows = sphere_rows(spheres)
+        self.spheres_dev = torch.as_tensor(rows).to(self.device) if len(rows) else None
+        self.spheres = _cabi.Spheres(len(rows), 0, _ptr(self.spheres_dev), float(margin))
+
     def solve_device(self, stream=None) -> BatchSolution:
         return solve_batch_tensors(self.params, self.inp, self.B, has_goal=self.has_goal,
                                    x_warm=self.x_warm, warm_mask=self.warm_mask, out=self.out,
                                    meta=self.meta, stream=stream, outputs=self.outputs,
                                    grid=self.grid, safety_margin=self.safety_margin,
                                    collision_threshold=self.collision_threshold, hit=self.hit,
-                                   penalty_grid=self.penalty_grid)
+                                   penalty_grid=self.penalty_grid, spheres=self.spheres)
 
     def stage_host_inputs(self, p0, v0, goal):
         """Write (B,3) host arrays into the pinned SoA staging block (host-side transpose)."""
@@ -441,7 +470,7 @@ class BatchWorkspace:
         """pinned H2D -> solve -> pinned D2H, all on one stream; returns after synchronising."""
         torch = _torch()
         if (self.B >= 65536 and self.B == self.ld and self.has_goal is None and self.x_warm is None
-                and self.grid is None):
+                and self.grid is None and self.spheres is None):
             return self._solve_staged_pipelined()
         stream = stream or torch.cuda.current_stream(self.device)
         with torch.cuda.stream(stream):
@@ -455,7 +484,8 @@ class BatchWorkspace:
 
     @property
     def rows_supported(self) -> bool:
-        return self.row_stride > 0 and self.h_inp is not None
+        """Row output: no entry of it takes a sphere list."""
+        return self.row_stride > 0 and self.h_inp is not None and self.spheres is None
 
     @property
     def d2h_bytes_rows(self) -> int:
@@ -473,6 +503,8 @@ class BatchWorkspace:
         torch = _torch()
         if self.penalty_grid is not None:
             raise ValueError("row output has no separate penalty grid")
+        if self.spheres is not None:
+            raise ValueError("row output has no sphere penalty")
         if not self.rows_supported:
             raise RuntimeError("row output needs pinned buffers and a horizon of at most 25 steps")
         if self.h_rows is None:
@@ -503,6 +535,8 @@ class BatchWorkspace:
         torch = _torch()
         if self.penalty_grid is not None:
             raise ValueError("row output has no separate penalty grid")
+        if self.spheres is not None:
+            raise ValueError("row output has no sphere penalty")
         if self.row_stride <= 0:
             raise RuntimeError("row output needs a horizon of at most 25 steps (64 for controls rows)")
         if rows_ptr is None and getattr(self, "d_rows", None) is None:
@@ -604,7 +638,8 @@ def plan_batch(positions, velocities, goals, config: Optional[SE3MPCConfig] = No
                has_goal=None, x_warm=None, warm_mask=None, gradient_mode: int = 0,
                device=None, outputs: str = "all", to_host: bool = False, grid=None,
                safety_margin: float = 1.0, collision_threshold: float = 0.6,
-               obstacle_penalty: bool = False, dynamics_consistent: bool = False, penalty_grid=None):
+               obstacle_penalty: bool = False, dynamics_consistent: bool = False, penalty_grid=None,
+               spheres=None, sphere_margin: Optional[float] = None):
     """Solve B independent SE(3)-MPC problems in one call.
 
     positions, velocities, goals : (B, 3) array-likes (NumPy or torch, host or device)
@@ -624,6 +659,12 @@ def plan_batch(positions, velocities, goals, config: Optional[SE3MPCConfig] = No
     penalty_grid : DenseOccupancyGrid the obstacle penalty reads instead of ``grid`` (typically
              ``grid.clearance_field(d_safe)``; free level = its prior).  ``grid``, if given, is then
              only the safety check's, run as a second launch on the solved positions.
+    spheres : (centers (S, 3), radii (S,)), NumPy or torch: the sphere obstacle penalty in the solve
+             (gradient_mode 5, with ``dynamics_consistent`` mode 6; extension -- the quadratic
+             penalty of the reference's constraint |P_k - c|^2 >= (r + safety_margin)^2, weight
+             ``config.obstacle_weight``; definition in include/dart_se3mpc.h, dart_spheres).  One list
+             for the whole batch, uploaded once per call.  ``grid`` then only adds the safety check.
+    sphere_margin : added to every radius; default ``config.safety_margin``.
     Returns a BatchSolution (device) or HostSolution (``to_host=True``).
     """
     cfg = config or SE3MPCConfig()
@@ -631,6 +672,12 @@ def plan_batch(positions, velocities, goals, config: Optional[SE3MPCConfig] = No
         if gradient_mode != 0:
             raise ValueError("dynamics_consistent selects its own gradient mode")
         gradient_mode = 3
+    if spheres is not None:
+        if obstacle_penalty or penalty_grid is not None:
+            raise ValueError("spheres= is an obstacle penalty of its own: it does not combine with obstacle_penalty")
+        if gradient_mode not in (0, 3):
+            raise ValueError("spheres= needs the reference gradient mode (or dynamics_consistent=True)")
+        gradient_mode = 5 if gradient_mode == 0 else 6
     pen = penalty_grid if penalty_grid is not None else grid
     if obstacle_penalty:
         if pen is None or gradient_mode not in (0, 3):
@@ -647,6 +694,8 @@ def plan_batch(positions, velocities, goals, config: Optional[SE3MPCConfig] = No
     ws.set_warm(x_warm, warm_mask)
     if grid is not None or penalty_grid is not None:
         ws.set_map(grid, safety_margin, collision_threshold, penalty_grid=penalty_grid)
+    if spheres is not None:
+        ws.set_spheres(spheres, cfg.safety_margin if sphere_margin is None else sphere_margin)
     sol = ws.solve_device()
     return sol.numpy() if to_host else sol
 
@@ -658,12 +707,16 @@ class SE3MPCPlanner:
     Differences, all opt-in: ``store_last_solution=True`` keeps the previous solution so that
     the warm start of :294-327 actually runs (the reference never assigns ``last_solution``);
     ``control_frequency_hz`` selects the timing-alignment frequency whose inverse overrides
-    ``config.dt`` (reference: always 400 Hz unless reconfigured, :99-122).
+    ``config.dt`` (reference: always 400 Hz unless reconfigured, :99-122);
+    ``avoid_obstacles=True`` makes the obstacle list (``add_obstacle``, ``update_plan``,
+    ``refresh_obstacles_from_mapper``) enter the solve as the sphere penalty of gradient_mode 5 with
+    ``config.safety_margin`` and ``config.obstacle_weight`` -- the reference builds that constraint
+    and never passes it to ``minimize`` (:499-514), so by default the list changes nothing here either.
     """
 
     def __init__(self, config: Optional[SE3MPCConfig] = None, *, mass: float = 1.5,
                  control_frequency_hz: Optional[float] = None, respect_config_dt: bool = False,
-                 store_last_solution: bool = False, device=None):
+                 store_last_solution: bool = False, device=None, avoid_obstacles: bool = False):
         if config is None:
             config = SE3MPCConfig()
         if control_frequency_hz is None:
@@ -690,6 +743,8 @@ class SE3MPCPlanner:
                                "last_plan_time": 0.0}
         self.logger = logger
         self._params = make_params(self.se3_config, mass=self.mass, gravity=self.gravity)
+        self.avoid_obstacles = bool(avoid_obstacles)
+        self._params_spheres = make_params(self.se3_config, mass=self.mass, gravity=self.gravity, gradient_mode=5)
         self._device = device
         _cabi.lib()  # fail now, loudly, if the CUDA library is missing
 
@@ -806,11 +861,17 @@ class SE3MPCPlanner:
         meta = np.zeros(3, np.int32)
         vp = lambda a: a.ctypes.data_as(C.c_void_p)  # noqa: E731
         o = out.ctypes.data
-        rc = L.dart_se3mpc_solve_batch_host(
-            C.byref(self._params), 1, vp(p0), vp(v0), vp(goal), vp(hg), None if xw is None else vp(xw),
-            o, o + 8 * 9 * N, meta.ctypes.data, meta.ctypes.data + 4, meta.ctypes.data + 8,
-            o + 8 * (9 * N + 1), o + 8 * (12 * N + 1), o + 8 * (15 * N + 1), o + 8 * (18 * N + 1))
-        _cabi.check(rc, "dart_se3mpc_solve_batch_host")
+        args = (1, vp(p0), vp(v0), vp(goal), vp(hg), None if xw is None else vp(xw),
+                o, o + 8 * 9 * N, meta.ctypes.data, meta.ctypes.data + 4, meta.ctypes.data + 8,
+                o + 8 * (9 * N + 1), o + 8 * (12 * N + 1), o + 8 * (15 * N + 1), o + 8 * (18 * N + 1))
+        if self.avoid_obstacles and self.obstacles:
+            rows = np.ascontiguousarray([[*c, r] for c, r in self.obstacles], np.float64)
+            sph = _cabi.Spheres(len(rows), 0, rows.ctypes.data, float(self.se3_config.safety_margin))
+            rc = L.dart_se3mpc_solve_batch_host_spheres(C.byref(self._params_spheres), *args, C.byref(sph))
+            _cabi.check(rc, "dart_se3mpc_solve_batch_host_spheres")
+        else:
+            rc = L.dart_se3mpc_solve_batch_host(C.byref(self._params), *args)
+            _cabi.check(rc, "dart_se3mpc_solve_batch_host")
         converged = bool(meta[2] == 0)
         self.convergence_history.append(converged)
         if not converged:

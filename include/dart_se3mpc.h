@@ -66,6 +66,10 @@ typedef struct dart_se3mpc_params {
                                /*    Horizons 1..16 (DART_E_UNSUPPORTED above).                 */
                                /* 4: mode 3 + the obstacle penalty of mode 2 on the rolled-out  */
                                /*    positions (needs a grid; closed loop: _step_map)           */
+                               /* 5: mode 0 + the sphere penalty (dart_spheres) on the position */
+                               /*    variables; horizons 1..64 (the _spheres entries only)      */
+                               /* 6: mode 3 + the sphere penalty on the rolled-out positions;   */
+                               /*    horizons 1..16, warm == 2 refused (the _spheres entries)   */
     int32_t reserved0;
     double dt;                 /* effective planner dt (timing_alignment.py:76-78)         */
     double mass, gravity;      /* 1.5 kg, 9.81 m/s^2 (:149-150)                            */
@@ -81,6 +85,29 @@ typedef struct dart_se3mpc_params {
      * (:60, unused by the reference solve), free level = the map's prior (0.5). */
     double w_obstacle, obstacle_free_level;
 } dart_se3mpc_params;
+
+/* Sphere obstacle list of gradient_mode 5 and 6 (extension; the reference builds the constraint
+ * |P_k - c|^2 >= (r + safety_margin)^2, se3_mpc_planner.py:499-514, and never passes it to
+ * minimize).  One list serves the whole batch.  With w = params->w_obstacle (obstacle_weight), for
+ * every timestep k < N and every sphere j = 0 .. n-1 in list order, each product and sum
+ * individually rounded (no contraction):
+ *   e  = P_k - c_j                          (per component)
+ *   d2 = (e_x*e_x + e_y*e_y) + e_z*e_z
+ *   R  = r_j + margin
+ *   h  = R*R - d2
+ *   if h > 0:  f += w*(h*h);   grad_{P_k} += ((-4*w)*h) * e
+ * the quadratic penalty of the reference's constraint function d2 - R^2: no square root, no
+ * division, a continuous gradient.  Per timestep the penalty sum starts at +0 and its gradient at
+ * -0, so a position no sphere reaches leaves the objective and gradient bits of mode 0 / 3 as they
+ * are.  At P_k = c_j the gradient is zero (a stationary point of the penalty).  Mode 5 adds it where
+ * mode 2 adds the grid penalty (the position variables), mode 6 where mode 4 does (the rolled-out
+ * positions, entering the adjoint through dP). */
+typedef struct dart_spheres {
+    int32_t n;             /* >= 0 */
+    int32_t reserved;
+    const double *cxyzr;   /* [n][4]: centre x, y, z, radius (device memory; host memory in the _host entry) */
+    double margin;         /* added to every radius: SE3MPCConfig.safety_margin */
+} dart_spheres;
 
 /* Self-test of the solver's in-line fp64 division (reciprocal seed + Newton + residual
  * correction, csrc/se3mpc_core.cuh) against IEEE division on n random operand pairs with
@@ -237,6 +264,33 @@ int dart_se3mpc_closed_loop_step_map(const dart_se3mpc_params *params, int64_t B
                                      double margin, double threshold, int32_t step,
                                      int32_t *first_collision, void *cuda_stream);
 
+/* ---- the sphere penalty (gradient_mode 5 / 6, see dart_spheres) ------------------------------
+ * Every other entry returns DART_E_UNSUPPORTED for gradient_mode 5 and 6.  These three refuse with
+ * DART_E_BADARG a gradient_mode other than 5 or 6, a NULL `spheres`, spheres->n < 0, n > 0 with a
+ * NULL cxyzr, and warm == 2 in mode 6; mode 6 above horizon 16 is DART_E_UNSUPPORTED.  n == 0 is
+ * allowed and returns the bits of mode 0 / 3.  No row-output entry takes spheres.
+ *
+ * dart_se3mpc_solve_batch_spheres: dart_se3mpc_solve_batch_map with the sphere penalty in the
+ * solve; `grid` (with margin, threshold, first_hit) serves only the optional fused safety check. */
+int dart_se3mpc_solve_batch_spheres(const dart_se3mpc_params *params, int64_t B, int64_t ld,
+                                    const double *p0, const double *v0, const double *goal,
+                                    const uint8_t *has_goal, const double *x_warm,
+                                    const uint8_t *warm_mask, double *x_out, double *cost, int32_t *nit,
+                                    int32_t *nfev, int32_t *status, int32_t *task, double *acc,
+                                    double *att, double *rates, double *thrust, const dart_spheres *spheres,
+                                    const dart_grid *grid, double margin, double threshold,
+                                    int32_t *first_hit, void *cuda_stream);
+/* dart_se3mpc_closed_loop_step_map with the sphere penalty; check_grid / first_collision as there
+ * (the collision record against a map, typically the same spheres rasterised by add_obstacles).
+ * warm == 2 is allowed in mode 5: its lateral thrust stays exactly zero, as in mode 0. */
+int dart_se3mpc_closed_loop_step_spheres(const dart_se3mpc_params *params, int64_t B, int64_t ld,
+                                         double *p, double *v, const double *goal,
+                                         const uint8_t *has_goal, double *x, int32_t warm, double *cost,
+                                         int32_t *nit, int32_t *nfev, int32_t *status, double plant_dt,
+                                         const dart_spheres *spheres, const dart_grid *check_grid,
+                                         double margin, double threshold, int32_t step,
+                                         int32_t *first_collision, void *cuda_stream);
+
 /* Same call with every buffer in HOST memory (pageable or pinned).  Up to 512 problems go
  * through a mapped pinned block the kernel reads and writes directly (no copies); larger batches
  * stage through an internal per-thread device workspace (chunked on two streams from 65536
@@ -249,6 +303,17 @@ int dart_se3mpc_solve_batch_host(const dart_se3mpc_params *params, int64_t B,
                                  double *cost_host, int32_t *nit_host, int32_t *nfev_host,
                                  int32_t *status_host, double *acc_host, double *att_host,
                                  double *rates_host, double *thrust_host);
+
+/* dart_se3mpc_solve_batch_host with the sphere penalty; spheres->cxyzr is HOST memory, staged with
+ * the other inputs (the mapped block up to 512 problems, the device workspace above). */
+int dart_se3mpc_solve_batch_host_spheres(const dart_se3mpc_params *params, int64_t B,
+                                         const double *p0_host, const double *v0_host,
+                                         const double *goal_host, const uint8_t *has_goal_host,
+                                         const double *x_warm_host, double *x_out_host,
+                                         double *cost_host, int32_t *nit_host, int32_t *nfev_host,
+                                         int32_t *status_host, double *acc_host, double *att_host,
+                                         double *rates_host, double *thrust_host,
+                                         const dart_spheres *spheres);
 
 /* Frees what dart_se3mpc_solve_batch_host caches for the CALLING thread (device workspace, mapped
  * pinned staging block, two streams) after draining them.  A host thread that used the host
