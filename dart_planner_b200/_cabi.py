@@ -58,6 +58,12 @@ class Spheres(C.Structure):
     ]
 
 
+class TrackRef(C.Structure):
+    """Mirror of ``dart_track_ref``: the per-timestep reference of gradient_mode 7 / 8."""
+
+    _fields_ = [("len", C.c_int32), ("start", C.c_int32), ("rows", C.c_void_p)]
+
+
 EXPORTS = [
     "dart_abi_version", "dart_last_cuda_error", "dart_se3mpc_default_params",
     "dart_se3mpc_solve_batch", "dart_se3mpc_solve_batch_map", "dart_se3mpc_closed_loop_step",
@@ -67,6 +73,7 @@ EXPORTS = [
     "dart_map_trace_ray_batch", "dart_map_update_batch", "dart_map_add_spheres", "dart_fp64_probe", "dart_ddiv_selftest",
     "dart_map_signed_distance", "dart_map_clearance_field", "dart_se3mpc_closed_loop_step_map",
     "dart_se3mpc_solve_batch_spheres", "dart_se3mpc_solve_batch_host_spheres", "dart_se3mpc_closed_loop_step_spheres",
+    "dart_se3mpc_solve_batch_track", "dart_se3mpc_closed_loop_step_track",
 ]
 
 _lib = None
@@ -115,6 +122,14 @@ def lib():
                                                        [vp] * 4 + [C.c_double, C.POINTER(Spheres), C.POINTER(Grid),
                                                                     C.c_double, C.c_double, i32, vp, vp])
     L.dart_se3mpc_closed_loop_step_spheres.restype = C.c_int
+    L.dart_se3mpc_solve_batch_track.argtypes = ([C.POINTER(Params), i64, i64] + [vp] * 15 +
+                                                 [C.POINTER(TrackRef), C.POINTER(Spheres), C.POINTER(Grid),
+                                                  C.c_double, C.c_double, vp, vp])
+    L.dart_se3mpc_solve_batch_track.restype = C.c_int
+    L.dart_se3mpc_closed_loop_step_track.argtypes = ([C.POINTER(Params), i64, i64] + [vp] * 4 + [i32] +
+                                                     [vp] * 4 + [C.c_double, C.POINTER(TrackRef), C.POINTER(Spheres),
+                                                                  C.POINTER(Grid), C.c_double, C.c_double, i32, vp, vp])
+    L.dart_se3mpc_closed_loop_step_track.restype = C.c_int
     L.dart_se3mpc_extract_batch.argtypes = [C.POINTER(Params), i64, i64] + [vp] * 5 + [i32, vp]
     L.dart_se3mpc_extract_batch.restype = C.c_int
     L.dart_se3mpc_release_thread_workspace.argtypes = []

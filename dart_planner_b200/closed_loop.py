@@ -53,16 +53,29 @@ class ClosedLoopSim:
                       ``collision_map`` still judges collisions, typically the same spheres
                       rasterised by ``add_obstacles``).  Mode 5 keeps the lateral thrust at exactly
                       zero, so its warm starts use the 7-slot kernel as in mode 0.
+
+    Tracking a path (``dart_se3mpc_closed_loop_step_track``):
+      reference_path : (P (B, T, 3), V (B, T, 3) or None = zero velocities), NumPy or torch: the
+                      per-timestep reference of gradient_mode 7 (mode 3 tracking it) or 8 (mode 6
+                      tracking it, with ``spheres``), which need it.  Uploaded once; step s tracks
+                      samples s, s+1, .., s+N-1, the last sample held past the end of the path, so
+                      the window slides one sample per replan (``plant_dt`` must equal ``params.dt``).
+                      ``mission.reference_path`` samples one from waypoints.  Goals are not read.
     """
 
     def __init__(self, params: _cabi.Params, B: int, plant_dt: Optional[float] = None, device=None, *,
                  penalty_grid=None, collision_map=None, safety_margin: float = 0.0,
-                 collision_threshold: float = 0.6, spheres=None, sphere_margin: float = 0.0):
+                 collision_threshold: float = 0.6, spheres=None, sphere_margin: float = 0.0,
+                 reference_path=None):
         gm = int(params.gradient_mode)
         if gm in (2, 4) and penalty_grid is None:
             raise ValueError("ClosedLoopSim: gradient_mode 2 / 4 need penalty_grid=")
-        if (gm in (5, 6)) != (spheres is not None):
-            raise ValueError("ClosedLoopSim: spheres= goes with gradient_mode 5 / 6, and they need it")
+        if (gm in (5, 6, 8)) != (spheres is not None):
+            raise ValueError("ClosedLoopSim: spheres= goes with gradient_mode 5 / 6 / 8, and they need it")
+        if (gm in (7, 8)) != (reference_path is not None):
+            raise ValueError("ClosedLoopSim: reference_path= goes with gradient_mode 7 / 8, and they need it")
+        if reference_path is not None and float(params.dt if plant_dt is None else plant_dt) != float(params.dt):
+            raise ValueError("ClosedLoopSim: reference_path= slides one sample per step: plant_dt must equal dt")
         torch = _torch()
         self.penalty_grid, self.collision_map = penalty_grid, collision_map
         self.safety_margin, self.collision_threshold = float(safety_margin), float(collision_threshold)
@@ -79,6 +92,11 @@ class ClosedLoopSim:
             self._spheres_dev = torch.as_tensor(rows).to(self.device) if len(rows) else None
             self.spheres = _cabi.Spheres(len(rows), 0, None if self._spheres_dev is None
                                          else self._spheres_dev.data_ptr(), float(sphere_margin))
+        self._ref_rows = None
+        if reference_path is not None:
+            from .planner import reference_rows
+            P, V = reference_path
+            self._ref_rows = reference_rows(P, V, self.B, self.ld, self.device)
         f8 = dict(dtype=torch.float64, device=self.device)
         self.state = torch.zeros((9, self.ld), **f8)            # rows p xyz | v xyz | goal xyz
         self.x = torch.zeros((9 * self.N, self.ld), **f8)       # current solution, reference order
@@ -95,11 +113,16 @@ class ClosedLoopSim:
 
     def _untilted_mode(self) -> bool:
         """Modes whose cold-started lateral thrust stays exactly zero (all but the dynamics-consistent
-        modes 3, 4 and 6)."""
+        modes 3, 4, 6, 7 and 8)."""
         return int(self.params.gradient_mode) in (0, 1, 2, 5)
 
-    def reset(self, p0, v0, goals):
+    def reset(self, p0, v0, goals=None):
+        """Initial states; ``goals`` (B, 3), which the tracking modes 7 / 8 do not read (None: zeros)."""
         torch = _torch()
+        if goals is None:
+            if self._ref_rows is None:
+                raise ValueError("ClosedLoopSim.reset: goals are needed without reference_path=")
+            goals = np.zeros((self.B, 3))
         for i, a in enumerate((p0, v0, goals)):
             t = torch.as_tensor(np.asarray(a, np.float64) if not torch.is_tensor(a) else a,
                                 dtype=torch.float64).to(self.device)
@@ -125,7 +148,13 @@ class ClosedLoopSim:
             record = (C.byref(cg) if cg is not None else None, self.safety_margin, self.collision_threshold,
                       self.steps_done, self._first_collision.data_ptr() + 4 * lo if cg is not None else None,
                       stream.cuda_stream)
-            if self.spheres is not None:
+            if self._ref_rows is not None:
+                name = "dart_se3mpc_closed_loop_step_track"
+                ref = _cabi.TrackRef(self._ref_rows.shape[0] // 6, self.steps_done, self._ref_rows.data_ptr() + 8 * lo)
+                rc = self._lib.dart_se3mpc_closed_loop_step_track(
+                    *args[:5], *args[6:], C.byref(ref), None if self.spheres is None else C.byref(self.spheres),
+                    *record)
+            elif self.spheres is not None:
                 name = "dart_se3mpc_closed_loop_step_spheres"
                 rc = self._lib.dart_se3mpc_closed_loop_step_spheres(*args, C.byref(self.spheres), *record)
             elif self.penalty_grid is None and self.collision_map is None:

@@ -86,6 +86,11 @@ struct SolveArgs {
     const double *spheres;
     int n_spheres;
     double sphere_margin;
+    /* the per-timestep reference of gradient_mode 7 / 8 (dart_track_ref): [6 track_len][ld] doubles of
+     * device memory; timestep k of a solve reads sample min(track_start + k, track_len - 1).  Last,
+     * as the sphere fields; null / 0 in every launch of the other modes */
+    const double *track_rows;
+    int track_len, track_start;
 };
 constexpr int PRIO_CAP = 16384;
 
@@ -204,8 +209,9 @@ se3mpc_solve_kernel(const __grid_constant__ dart_se3mpc_params P, const __grid_c
         for (int c = 0; c < 3; ++c) {
             p0[c] = __ldg(A.p0 + c * A.ld + b);
             v0[c] = __ldg(A.v0 + c * A.ld + b);
-            if (phase != 2) sv.goal[c] = __ldg(A.goal + c * A.ld + b);
+            if (phase != 2) sv.goal[c] = SolverT::TRACK ? 0.0 : __ldg(A.goal + c * A.ld + b); /* not read in TRACK */
         }
+        if constexpr (SolverT::TRACK) sv.set_reference(A.track_rows + b, A.ld, A.track_len, A.track_start);
         if (phase != 2) sv.has_goal = A.has_goal ? (A.has_goal[b] != 0) : true;
         if (skip_near) {
             /* a member of the priority list met in a regular round: solved (or about to be) in a
@@ -620,11 +626,12 @@ se3mpc_extract_kernel(const __grid_constant__ dart_se3mpc_params P, const __grid
     }
 }
 
-/* the eleven instantiations of one lane configuration: [gradient_mode][tilt].  The dynamics-consistent
- * modes 3 / 4 / 6 move the lateral thrust, so they exist only with tilt (fn[3][0] = fn[4][0] =
- * fn[6][0] = null). */
+/* the instantiations of one lane configuration: [gradient_mode][tilt].  The dynamics-consistent
+ * modes 3 / 4 / 6 / 7 / 8 move the lateral thrust, so they exist only with tilt (fn[3][0] = fn[4][0] =
+ * fn[6][0] = fn[7][0] = fn[8][0] = null).  The tracking modes 7 / 8 exist only in the builds that
+ * serve horizons <= 16, the library's limit for them: null in the 32-lane builds. */
 struct KernelSet {
-    const void *fn[7][2];
+    const void *fn[9][2];
     const void *extract_fn[2]; /* [tilt] */
     int lanes, tpl, block, minb;
     int gpb;      /* problems per block */
@@ -646,9 +653,18 @@ KernelSet make_kernel_set()
     k.fn[5][1] = (const void *)se3mpc_solve_kernel<LANES, TPL, BLK, MINB, 5, true>;
     k.fn[5][0] = (const void *)se3mpc_solve_kernel<LANES, TPL, BLK, MINB, 5, false>;
     k.fn[6][1] = (const void *)se3mpc_solve_kernel<LANES, TPL, BLK, MINB, 6, true>;
+    if constexpr (LANES * TPL <= 16) {
+        k.fn[7][1] = (const void *)se3mpc_solve_kernel<LANES, TPL, BLK, MINB, 7, true>;
+        k.fn[8][1] = (const void *)se3mpc_solve_kernel<LANES, TPL, BLK, MINB, 8, true>;
+    } else {
+        k.fn[7][1] = nullptr;
+        k.fn[8][1] = nullptr;
+    }
     k.fn[3][0] = nullptr;
     k.fn[4][0] = nullptr;
     k.fn[6][0] = nullptr;
+    k.fn[7][0] = nullptr;
+    k.fn[8][0] = nullptr;
     k.extract_fn[1] = (const void *)se3mpc_extract_kernel<LANES, TPL, BLK, true>;
     k.extract_fn[0] = (const void *)se3mpc_extract_kernel<LANES, TPL, BLK, false>;
     k.lanes = LANES;

@@ -162,8 +162,10 @@ int prepare(KernelChoice *k)
     const int smem = smem_bytes(*k);
     const void *fns[] = {k->set.fn[0][0], k->set.fn[0][1], k->set.fn[1][0], k->set.fn[1][1],
                          k->set.fn[2][0], k->set.fn[2][1], k->set.fn[3][1], k->set.fn[4][1],
-                         k->set.fn[5][0], k->set.fn[5][1], k->set.fn[6][1]};
+                         k->set.fn[5][0], k->set.fn[5][1], k->set.fn[6][1], k->set.fn[7][1],
+                         k->set.fn[8][1]};
     for (const void *fn : fns) {
+        if (!fn) continue; /* modes 7 / 8 in the 32-lane builds */
         e = cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
         if (e != cudaSuccess) return set_err(e, "cudaFuncSetAttribute(smem)");
     }
@@ -172,6 +174,7 @@ int prepare(KernelChoice *k)
     int carve = (int)((long long)k->set.resident * (smem + 1024) * 100 / (228 * 1024)) + 1;
     if (carve > 100) carve = 100;
     for (const void *fn : fns) {
+        if (!fn) continue;
         e = cudaFuncSetAttribute(fn, cudaFuncAttributePreferredSharedMemoryCarveout, carve);
         if (e != cudaSuccess) return set_err(e, "cudaFuncSetAttribute(carveout)");
     }
@@ -187,18 +190,20 @@ int prepare(KernelChoice *k)
 }
 
 /* the dynamics-consistent modes: thrusts are the only variables, P / V their rollout */
-bool rollout_mode(int gm) { return gm == 3 || gm == 4 || gm == 6; }
+bool rollout_mode(int gm) { return gm == 3 || gm == 4 || gm == 6 || gm == 7 || gm == 8; }
 
-/* spheres: the caller is one of the _spheres entries, which serve modes 5 and 6 only; every other
- * entry serves modes 0..4 */
-int check_params(const dart_se3mpc_params *p, bool spheres = false)
+/* spheres: the caller is one of the _spheres entries, which serve modes 5 and 6 only; track: one of
+ * the _track entries, which serve modes 7 and 8 only; every other entry serves modes 0..4 */
+int check_params(const dart_se3mpc_params *p, bool spheres = false, bool track = false)
 {
     if (!p || p->struct_size != (int)sizeof(dart_se3mpc_params)) return DART_E_BADARG;
     if (p->horizon < 1 || p->horizon > 64) return DART_E_UNSUPPORTED;
     if (p->max_corrections < 1 || p->max_corrections > MMAX) return DART_E_UNSUPPORTED;
     /* maxls >= 1, as SciPy requires; with 0 every solve would end ABNORMAL after one evaluation */
     if (p->max_iterations < 0 || p->max_linesearch < 1) return DART_E_BADARG;
-    if (spheres) {
+    if (track) {
+        if (p->gradient_mode != 7 && p->gradient_mode != 8) return DART_E_BADARG;
+    } else if (spheres) {
         if (p->gradient_mode != 5 && p->gradient_mode != 6) return DART_E_BADARG;
     } else if (p->gradient_mode < 0 || p->gradient_mode > 4)
         return DART_E_UNSUPPORTED;
@@ -223,6 +228,22 @@ void set_spheres(SolveArgs &a, const dart_spheres *s)
     a.spheres = s->cxyzr;
     a.n_spheres = s->n;
     a.sphere_margin = s->margin;
+}
+
+/* the reference and sphere list of a _track entry (mode 7 takes no spheres, mode 8 needs them) */
+int check_track(const dart_se3mpc_params *p, const dart_track_ref *ref, const dart_spheres *s)
+{
+    if (!ref || !ref->rows || ref->len < 1 || ref->start < 0) return DART_E_BADARG;
+    if ((p->gradient_mode == 8) != (s != nullptr)) return DART_E_BADARG;
+    return s ? check_spheres(s) : DART_OK;
+}
+
+void set_track(SolveArgs &a, const dart_track_ref *ref)
+{
+    if (!ref) return;
+    a.track_rows = ref->rows;
+    a.track_len = ref->len;
+    a.track_start = ref->start;
 }
 
 long long grid_for(const KernelChoice &k, long long B)
@@ -327,9 +348,11 @@ static int launch_solve(const dart_se3mpc_params *params, const SolveArgs &a, vo
          * place, and a member of the list met again in a regular round is recognised by the
          * predicate on the state it loads -- after its priority-round solve has moved it, the drone
          * could leave the radius and be stepped twice (tests/test_gpu_closed_loop.py,
-         * test_run_in_sub_populations_changes_no_result). */
+         * test_run_in_sub_populations_changes_no_result).  Not in the tracking modes 7 / 8: the
+         * predicate reads the goal, which they do not have. */
         if (k->minb >= 3 && DART_THROUGHPUT_SCHED == 2 && a.B >= PRIO_MIN_B && a.B < (1ll << 31) &&
-            a.x_warm == nullptr && a.p_next == nullptr && params->w_pos > 0.0 && !getenv("DART_SE3MPC_NO_PRIO")) {
+            a.x_warm == nullptr && a.p_next == nullptr && params->w_pos > 0.0 && a.track_rows == nullptr &&
+            !getenv("DART_SE3MPC_NO_PRIO")) {
             StashBuf &pb = g_prio[dev][g_prio_next[dev]++ % PRIO_RING];
             const size_t need = 16 + (size_t)PRIO_CAP * sizeof(int); /* fixed: allocated once per slot */
             if (pb.done) {
@@ -397,8 +420,9 @@ static int launch_solve(const dart_se3mpc_params *params, const SolveArgs &a, vo
      * bit for bit, which a separate kernel cannot promise -- ptxas contracts the plain products and
      * sums of the shared solver code kernel by kernel (DESIGN.md 5e) */
     int gm = params->gradient_mode;
-    if ((gm == 5 || gm == 6) && a.n_spheres == 0) gm = (gm == 5) ? 0 : 3;
+    if ((gm == 5 || gm == 6 || gm == 8) && a.n_spheres == 0) gm = (gm == 5) ? 0 : (gm == 6 ? 3 : 7);
     const void *fn = k->set.fn[gm][cold];
+    if (!fn) return DART_E_UNSUPPORTED; /* modes 7 / 8 forced onto a 32-lane build (DART_SE3MPC_VARIANT) */
     cudaError_t e;
     if (prio_event) {
         /* programmatic dependent launch: the solve may begin while the scan in front of it runs */
@@ -432,12 +456,13 @@ static int solve_batch_impl(const dart_se3mpc_params *params, int64_t B, int64_t
                             int32_t *nit, int32_t *nfev, int32_t *status, int32_t *task, double *acc,
                             double *att, double *rates, double *thrust, const dart_grid *grid, double margin,
                             double threshold, int32_t *first_hit, const dart_spheres *spheres,
-                            void *cuda_stream)
+                            void *cuda_stream, const dart_track_ref *ref = nullptr, bool track = false)
 {
-    int rc = check_params(params, spheres != nullptr);
+    int rc = check_params(params, spheres != nullptr, track);
     if (rc) return rc;
-    if (spheres && (rc = check_spheres(spheres))) return rc;
-    if (B < 0 || ld < B || !p0 || !v0 || !goal) return DART_E_BADARG;
+    if (track && (rc = check_track(params, ref, spheres))) return rc;
+    if (!track && spheres && (rc = check_spheres(spheres))) return rc;
+    if (B < 0 || ld < B || !p0 || !v0 || (!goal && !track)) return DART_E_BADARG;
     const bool need_grid = first_hit != nullptr || params->gradient_mode == 2 || params->gradient_mode == 4;
     if (need_grid && (!grid || !grid->occ || grid->nx <= 0 || grid->ny <= 0 || grid->nz <= 0 ||
                       !(grid->resolution > 0.0)))
@@ -458,6 +483,7 @@ static int solve_batch_impl(const dart_se3mpc_params *params, int64_t B, int64_t
         a.check_map = 1;
     }
     set_spheres(a, spheres);
+    set_track(a, ref);
     return launch_solve(params, a, cuda_stream);
 }
 
@@ -527,12 +553,16 @@ static int closed_loop_step_impl(const dart_se3mpc_params *params, int64_t B, in
                                  double *cost, int32_t *nit, int32_t *nfev, int32_t *status, double plant_dt,
                                  const dart_grid *penalty_grid, const dart_spheres *spheres,
                                  const dart_grid *check_grid, double margin, double threshold, int32_t step,
-                                 int32_t *first_collision, void *cuda_stream)
+                                 int32_t *first_collision, void *cuda_stream, const dart_track_ref *ref = nullptr,
+                                 bool track = false)
 {
-    int rc = check_params(params, spheres != nullptr);
+    int rc = check_params(params, spheres != nullptr, track);
     if (rc) return rc;
-    if (spheres && (rc = check_spheres(spheres))) return rc;
-    if (B < 0 || ld < B || !p || !v || !goal || !x || !(plant_dt > 0.0)) return DART_E_BADARG;
+    if (track && (rc = check_track(params, ref, spheres))) return rc;
+    if (!track && spheres && (rc = check_spheres(spheres))) return rc;
+    if (B < 0 || ld < B || !p || !v || (!goal && !track) || !x || !(plant_dt > 0.0)) return DART_E_BADARG;
+    /* the reference window slides one sample per replan: one plant step must be one sample */
+    if (track && plant_dt != params->dt) return DART_E_BADARG;
     const bool penalty = params->gradient_mode == 2 || params->gradient_mode == 4;
     if (penalty && !grid_ok(penalty_grid)) return DART_E_BADARG;
     if ((check_grid != nullptr) != (first_collision != nullptr)) return DART_E_BADARG;
@@ -557,6 +587,7 @@ static int closed_loop_step_impl(const dart_se3mpc_params *params, int64_t B, in
         a.step = step;
     }
     set_spheres(a, spheres);
+    set_track(a, ref);
     return launch_solve(params, a, cuda_stream);
 }
 
@@ -583,6 +614,31 @@ int dart_se3mpc_closed_loop_step_spheres(const dart_se3mpc_params *params, int64
     return closed_loop_step_impl(params, B, ld, p, v, goal, has_goal, x, warm, cost, nit, nfev, status, plant_dt,
                                  nullptr, spheres, check_grid, margin, threshold, step, first_collision,
                                  cuda_stream);
+}
+
+int dart_se3mpc_solve_batch_track(const dart_se3mpc_params *params, int64_t B, int64_t ld,
+                                  const double *p0, const double *v0, const uint8_t *has_goal,
+                                  const double *x_warm, const uint8_t *warm_mask, double *x_out, double *cost,
+                                  int32_t *nit, int32_t *nfev, int32_t *status, int32_t *task, double *acc,
+                                  double *att, double *rates, double *thrust, const dart_track_ref *ref,
+                                  const dart_spheres *spheres, const dart_grid *grid, double margin,
+                                  double threshold, int32_t *first_hit, void *cuda_stream)
+{
+    return solve_batch_impl(params, B, ld, p0, v0, nullptr, has_goal, x_warm, warm_mask, x_out, cost, nit, nfev,
+                            status, task, acc, att, rates, thrust, grid, margin, threshold, first_hit, spheres,
+                            cuda_stream, ref, true);
+}
+
+int dart_se3mpc_closed_loop_step_track(const dart_se3mpc_params *params, int64_t B, int64_t ld, double *p,
+                                       double *v, const uint8_t *has_goal, double *x, int32_t warm, double *cost,
+                                       int32_t *nit, int32_t *nfev, int32_t *status, double plant_dt,
+                                       const dart_track_ref *ref, const dart_spheres *spheres,
+                                       const dart_grid *check_grid, double margin, double threshold,
+                                       int32_t step, int32_t *first_collision, void *cuda_stream)
+{
+    return closed_loop_step_impl(params, B, ld, p, v, nullptr, has_goal, x, warm, cost, nit, nfev, status, plant_dt,
+                                 nullptr, spheres, check_grid, margin, threshold, step, first_collision,
+                                 cuda_stream, ref, true);
 }
 
 int dart_se3mpc_solve_batch(const dart_se3mpc_params *params, int64_t B, int64_t ld,

@@ -130,3 +130,42 @@ class BatchedMissionGoals:
 
     def phase_names(self) -> List[str]:
         return [PHASE_NAMES[p] for p in self.phase]
+
+
+def reference_path(waypoints, speed: float, dt: float, T: int):
+    """Waypoints -> the per-timestep reference of the tracking modes (gradient_mode 7 / 8:
+    ``plan_batch(reference=)``, ``ClosedLoopSim(reference_path=)``).
+
+    waypoints : (W, 3), or (B, W, 3) one polyline per drone
+    Sample j = 0 .. T-1 is the point at arc length s_j = min((speed * j) * dt, L) along the polyline
+    of length L: on segment i with cum_i <= s_j < cum_{i+1} (zero-length segments are never current),
+    P_j = w_i + ((s_j - cum_i) / len_i) (w_{i+1} - w_i), and its velocity is speed along that
+    segment, V_j = (speed / len_i) (w_{i+1} - w_i).  Once (speed * j) * dt >= L the end is reached:
+    P_j = the last waypoint, V_j = +0.
+    Returns (P, V), both (B, T, 3) float64 (B = 1 for a single polyline)."""
+    w = np.asarray(waypoints, np.float64)
+    if w.ndim == 2:
+        w = w[None]
+    if w.ndim != 3 or w.shape[2] != 3 or w.shape[1] < 1:
+        raise ValueError(f"waypoints must be (W, 3) or (B, W, 3), got {np.shape(waypoints)}")
+    if not (speed > 0.0) or not (dt > 0.0) or int(T) < 1:
+        raise ValueError("reference_path needs speed > 0, dt > 0 and T >= 1")
+    B, W, T = w.shape[0], w.shape[1], int(T)
+    d = w[:, 1:] - w[:, :-1]                                   # (B, W-1, 3)
+    seg = np.sqrt((d * d).sum(axis=2))                         # (B, W-1)
+    cum = np.concatenate([np.zeros((B, 1)), np.cumsum(seg, axis=1)], axis=1)
+    s_raw = (float(speed) * np.arange(T)) * float(dt)          # (T,)
+    P = np.empty((B, T, 3))
+    V = np.zeros((B, T, 3))
+    for b in range(B):
+        L = cum[b, -1]
+        done = s_raw >= L
+        P[b, done] = w[b, -1]
+        j = np.nonzero(~done)[0]
+        if len(j):
+            s = s_raw[j]
+            i = np.minimum(np.searchsorted(cum[b], s, side="right") - 1, W - 2)
+            frac = (s - cum[b, i]) / seg[b, i]
+            P[b, j] = w[b, i] + frac[:, None] * d[b, i]
+            V[b, j] = (float(speed) / seg[b, i])[:, None] * d[b, i]
+    return P, V

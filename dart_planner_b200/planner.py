@@ -273,11 +273,31 @@ def sphere_rows(spheres) -> np.ndarray:
     return np.ascontiguousarray(np.concatenate([c, r[:, None]], axis=1))
 
 
+def reference_rows(P, V, B: int, ld: int, device):
+    """(P (B, T, 3), V (B, T, 3) or None) from NumPy or torch -> the (6T, ld) float64 device block of
+    ``dart_track_ref`` (rows 3j+c position, 3T+3j+c velocity of sample j; V None = zero velocities)."""
+    torch = _torch()
+    as_t = lambda a: (a if torch.is_tensor(a) else torch.as_tensor(np.asarray(a, np.float64))).to(  # noqa: E731
+        device, torch.float64)
+    Pt = as_t(P)
+    if Pt.dim() != 3 or Pt.shape[0] != B or Pt.shape[2] != 3 or Pt.shape[1] < 1:
+        raise ValueError(f"reference positions must be (B={B}, T, 3), got {tuple(Pt.shape)}")
+    T = Pt.shape[1]
+    Vt = torch.zeros_like(Pt) if V is None else as_t(V)
+    if tuple(Vt.shape) != tuple(Pt.shape):
+        raise ValueError(f"reference velocities must be (B, T, 3) like the positions, got {tuple(Vt.shape)}")
+    rows = torch.zeros((6 * T, ld), dtype=torch.float64, device=device)
+    rows[: 3 * T, :B] = Pt.reshape(B, 3 * T).t()
+    rows[3 * T:, :B] = Vt.reshape(B, 3 * T).t()
+    return rows
+
+
 def solve_batch_tensors(params: _cabi.Params, inp, B: int, *, has_goal=None, x_warm=None,
                         warm_mask=None, out=None, meta=None, stream=None,
                         outputs: str = "all", grid=None, safety_margin: float = 1.0,
                         collision_threshold: float = 0.6, hit=None, penalty_grid=None,
-                        spheres: Optional[_cabi.Spheres] = None) -> BatchSolution:
+                        spheres: Optional[_cabi.Spheres] = None,
+                        reference: Optional[_cabi.TrackRef] = None) -> BatchSolution:
     """Lowest Python level: device tensors in, device tensors out, one kernel launch.
 
     inp      : (9, ld) float64 CUDA tensor, rows [p0 xyz | v0 xyz | goal xyz]
@@ -293,6 +313,8 @@ def solve_batch_tensors(params: _cabi.Params, inp, B: int, *, has_goal=None, x_w
                the solved positions
     spheres  : _cabi.Spheres over a device list, or None; the sphere penalty of gradient_mode 5 / 6
                (``grid`` then serves only the fused safety check)
+    reference : _cabi.TrackRef over a (6T, ld) device block, or None; the per-timestep reference of
+               gradient_mode 7 / 8 (``inp``'s goal rows are not read)
     """
     torch = _torch()
     L = _cabi.lib()
@@ -337,11 +359,17 @@ def solve_batch_tensors(params: _cabi.Params, inp, B: int, *, has_goal=None, x_w
     check = (C.byref(g) if g is not None else None, float(safety_margin), float(collision_threshold),
              hit.data_ptr() if fused else None, stream.cuda_stream)
     with torch.cuda.device(inp.device):
-        if spheres is None:
+        if reference is not None:
+            name = "dart_se3mpc_solve_batch_track"
+            rc = L.dart_se3mpc_solve_batch_track(*args[:5], *args[6:], C.byref(reference),
+                                                 None if spheres is None else C.byref(spheres), *check)
+        elif spheres is None:
+            name = "dart_se3mpc_solve_batch_map"
             rc = L.dart_se3mpc_solve_batch_map(*args, *check)
         else:
+            name = "dart_se3mpc_solve_batch_spheres"
             rc = L.dart_se3mpc_solve_batch_spheres(*args, C.byref(spheres), *check)
-    _cabi.check(rc, "dart_se3mpc_solve_batch_map" if spheres is None else "dart_se3mpc_solve_batch_spheres")
+    _cabi.check(rc, name)
     if grid is not None and not fused:
         grid.trajectories_safe_soa(out[: 3 * N], B, N, safety_margin, collision_threshold, out=hit, stream=stream)
     return BatchSolution(N=N, B=B, out=out, meta=meta, hit=hit if grid is not None else None)
@@ -372,6 +400,7 @@ class BatchWorkspace:
         self.grid, self.safety_margin, self.collision_threshold, self.hit = None, 1.0, 0.6, None
         self.penalty_grid = None
         self.spheres = self.spheres_dev = None
+        self.reference = self.reference_dev = None
         self.h_inp = self.h_out = self.h_meta = self.h_rows = None
         # DART_ROWS_FULL / DART_ROWS_CONTROLS / DART_ROWS_SOLUTION
         if outputs not in ("all", "controls", "solution"):
@@ -451,13 +480,26 @@ class BatchWorkspace:
         self.spheres_dev = torch.as_tensor(rows).to(self.device) if len(rows) else None
         self.spheres = _cabi.Spheres(len(rows), 0, _ptr(self.spheres_dev), float(margin))
 
+    def set_reference(self, P, V=None, start: int = 0):
+        """The per-timestep reference of gradient_mode 7 / 8: positions P (B, T, 3) and velocities V
+        (B, T, 3) or None (zero), NumPy or torch; timestep k of every solve tracks sample
+        min(start + k, T - 1).  Uploaded once, used by every SoA solve.  P None removes it."""
+        if P is None:
+            self.reference = self.reference_dev = None
+            return
+        if int(start) < 0:
+            raise ValueError("reference start must be >= 0")
+        self.reference_dev = reference_rows(P, V, self.B, self.ld, self.device)
+        self.reference = _cabi.TrackRef(self.reference_dev.shape[0] // 6, int(start), self.reference_dev.data_ptr())
+
     def solve_device(self, stream=None) -> BatchSolution:
         return solve_batch_tensors(self.params, self.inp, self.B, has_goal=self.has_goal,
                                    x_warm=self.x_warm, warm_mask=self.warm_mask, out=self.out,
                                    meta=self.meta, stream=stream, outputs=self.outputs,
                                    grid=self.grid, safety_margin=self.safety_margin,
                                    collision_threshold=self.collision_threshold, hit=self.hit,
-                                   penalty_grid=self.penalty_grid, spheres=self.spheres)
+                                   penalty_grid=self.penalty_grid, spheres=self.spheres,
+                                   reference=self.reference)
 
     def stage_host_inputs(self, p0, v0, goal):
         """Write (B,3) host arrays into the pinned SoA staging block (host-side transpose)."""
@@ -470,7 +512,7 @@ class BatchWorkspace:
         """pinned H2D -> solve -> pinned D2H, all on one stream; returns after synchronising."""
         torch = _torch()
         if (self.B >= 65536 and self.B == self.ld and self.has_goal is None and self.x_warm is None
-                and self.grid is None and self.spheres is None):
+                and self.grid is None and self.spheres is None and self.reference is None):
             return self._solve_staged_pipelined()
         stream = stream or torch.cuda.current_stream(self.device)
         with torch.cuda.stream(stream):
@@ -484,8 +526,9 @@ class BatchWorkspace:
 
     @property
     def rows_supported(self) -> bool:
-        """Row output: no entry of it takes a sphere list."""
-        return self.row_stride > 0 and self.h_inp is not None and self.spheres is None
+        """Row output: no entry of it takes a sphere list or a reference."""
+        return (self.row_stride > 0 and self.h_inp is not None and self.spheres is None
+                and self.reference is None)
 
     @property
     def d2h_bytes_rows(self) -> int:
@@ -505,6 +548,8 @@ class BatchWorkspace:
             raise ValueError("row output has no separate penalty grid")
         if self.spheres is not None:
             raise ValueError("row output has no sphere penalty")
+        if self.reference is not None:
+            raise ValueError("row output has no reference tracking")
         if not self.rows_supported:
             raise RuntimeError("row output needs pinned buffers and a horizon of at most 25 steps")
         if self.h_rows is None:
@@ -537,6 +582,8 @@ class BatchWorkspace:
             raise ValueError("row output has no separate penalty grid")
         if self.spheres is not None:
             raise ValueError("row output has no sphere penalty")
+        if self.reference is not None:
+            raise ValueError("row output has no reference tracking")
         if self.row_stride <= 0:
             raise RuntimeError("row output needs a horizon of at most 25 steps (64 for controls rows)")
         if rows_ptr is None and getattr(self, "d_rows", None) is None:
@@ -639,7 +686,7 @@ def plan_batch(positions, velocities, goals, config: Optional[SE3MPCConfig] = No
                device=None, outputs: str = "all", to_host: bool = False, grid=None,
                safety_margin: float = 1.0, collision_threshold: float = 0.6,
                obstacle_penalty: bool = False, dynamics_consistent: bool = False, penalty_grid=None,
-               spheres=None, sphere_margin: Optional[float] = None):
+               spheres=None, sphere_margin: Optional[float] = None, reference=None):
     """Solve B independent SE(3)-MPC problems in one call.
 
     positions, velocities, goals : (B, 3) array-likes (NumPy or torch, host or device)
@@ -665,9 +712,20 @@ def plan_batch(positions, velocities, goals, config: Optional[SE3MPCConfig] = No
              ``config.obstacle_weight``; definition in include/dart_se3mpc.h, dart_spheres).  One list
              for the whole batch, uploaded once per call.  ``grid`` then only adds the safety check.
     sphere_margin : added to every radius; default ``config.safety_margin``.
+    reference : (P (B, N, 3), V (B, N, 3) or None = zero velocities), NumPy or torch, host or device:
+             track a per-timestep reference instead of flying to a goal (gradient_mode 7, with
+             ``spheres`` mode 8; extension; definition in include/dart_se3mpc.h, dart_track_ref).
+             Needs ``dynamics_consistent=True``; ``goals`` may then be None and is not read.
     Returns a BatchSolution (device) or HostSolution (``to_host=True``).
     """
     cfg = config or SE3MPCConfig()
+    if reference is not None:
+        if not dynamics_consistent:
+            raise ValueError("reference= tracks with the dynamics-consistent solve: pass dynamics_consistent=True")
+        if obstacle_penalty or penalty_grid is not None:
+            raise ValueError("reference= does not combine with the grid penalty (obstacle_penalty)")
+    elif goals is None:
+        raise ValueError("goals may be None only with reference=")
     if dynamics_consistent:
         if gradient_mode != 0:
             raise ValueError("dynamics_consistent selects its own gradient mode")
@@ -678,6 +736,8 @@ def plan_batch(positions, velocities, goals, config: Optional[SE3MPCConfig] = No
         if gradient_mode not in (0, 3):
             raise ValueError("spheres= needs the reference gradient mode (or dynamics_consistent=True)")
         gradient_mode = 5 if gradient_mode == 0 else 6
+    if reference is not None:
+        gradient_mode = 7 if gradient_mode == 3 else 8
     pen = penalty_grid if penalty_grid is not None else grid
     if obstacle_penalty:
         if pen is None or gradient_mode not in (0, 3):
@@ -689,13 +749,18 @@ def plan_batch(positions, velocities, goals, config: Optional[SE3MPCConfig] = No
                          obstacle_free_level=pen.prob_prior if pen is not None else 0.5)
     B = int(np.shape(positions)[0])
     ws = BatchWorkspace(params, B, device=device, pinned=False, outputs=outputs)
-    ws.set_inputs_device(positions, velocities, goals)
+    ws.set_inputs_device(positions, velocities, np.zeros((B, 3)) if goals is None else goals)
     ws.set_has_goal(has_goal)
     ws.set_warm(x_warm, warm_mask)
     if grid is not None or penalty_grid is not None:
         ws.set_map(grid, safety_margin, collision_threshold, penalty_grid=penalty_grid)
     if spheres is not None:
         ws.set_spheres(spheres, cfg.safety_margin if sphere_margin is None else sphere_margin)
+    if reference is not None:
+        P, V = reference
+        if int(np.shape(P)[1]) != int(params.horizon):
+            raise ValueError(f"reference= needs N = {int(params.horizon)} samples per problem, got {np.shape(P)[1]}")
+        ws.set_reference(P, V)
     sol = ws.solve_device()
     return sol.numpy() if to_host else sol
 

@@ -70,6 +70,9 @@ typedef struct dart_se3mpc_params {
                                /*    variables; horizons 1..64 (the _spheres entries only)      */
                                /* 6: mode 3 + the sphere penalty on the rolled-out positions;   */
                                /*    horizons 1..16, warm == 2 refused (the _spheres entries)   */
+                               /* 7: mode 3 with a per-timestep reference (dart_track_ref);     */
+                               /*    horizons 1..16 (the _track entries only)                   */
+                               /* 8: mode 6 with the reference of mode 7 (the _track entries)   */
     int32_t reserved0;
     double dt;                 /* effective planner dt (timing_alignment.py:76-78)         */
     double mass, gravity;      /* 1.5 kg, 9.81 m/s^2 (:149-150)                            */
@@ -108,6 +111,29 @@ typedef struct dart_spheres {
     const double *cxyzr;   /* [n][4]: centre x, y, z, radius (device memory; host memory in the _host entry) */
     double margin;         /* added to every radius: SE3MPCConfig.safety_margin */
 } dart_spheres;
+
+/* Per-timestep reference of gradient_mode 7 and 8 (extension: tracking a time-parametrised path).
+ * Everything not stated here is as in mode 3 / 6: variables, bounds, rollout, adjoint, stopping
+ * rule, the P/V rows of x receiving the rollout, horizons 1..16.
+ *
+ * Reference tracking (gradient_mode 7 = mode 3, 8 = mode 6, with a per-timestep reference).
+ * For timestep k = 0..N-1, r_k is the reference position and u_k the reference velocity, sample
+ * j = min(s + k, T - 1) of the reference.  Each operation is rounded on its own (no contraction):
+ *   e = P_k - r_k,  ev = V_k - u_k  (per component),
+ *   f += wpf_k (e.e) + w_vel (ev.ev) + w_acc |a_k|^2 + w_thrust |T_k - m g e3|^2,
+ *        wpf_k = w_pos, and 11 w_pos at k = N-1,
+ *   dP_k = 2 w_pos e, plus 20 w_pos e at k = N-1,   dV_k = 2 w_vel ev,
+ *   mode 8 adds the sphere penalty on P_k exactly as mode 6 does.
+ * has_goal = 0 turns the position terms off; the goal input is not read.  With r_k = goal and
+ * u_k = +0, e and ev are the doubles of mode 3 (v - (+0) = v, -0 - (+0) = -0), so the objective
+ * and gradient are mode 3's bits, and mode 8's are mode 6's.
+ *
+ * The block is batch-major like the P/V rows of x, with the batch's row pitch ld. */
+typedef struct dart_track_ref {
+    int32_t len;          /* T >= 1 samples per problem, spaced params->dt apart */
+    int32_t start;        /* s >= 0: timestep k reads sample j = min(s + k, T - 1) */
+    const double *rows;   /* [6T][ld] device memory: rows 3j+c = position, 3T+3j+c = velocity of sample j */
+} dart_track_ref;
 
 /* Self-test of the solver's in-line fp64 division (reciprocal seed + Newton + residual
  * correction, csrc/se3mpc_core.cuh) against IEEE division on n random operand pairs with
@@ -290,6 +316,34 @@ int dart_se3mpc_closed_loop_step_spheres(const dart_se3mpc_params *params, int64
                                          const dart_spheres *spheres, const dart_grid *check_grid,
                                          double margin, double threshold, int32_t step,
                                          int32_t *first_collision, void *cuda_stream);
+
+/* ---- reference tracking (gradient_mode 7 / 8, see dart_track_ref) ----------------------------
+ * Every other entry refuses gradient_mode 7 and 8.  These two return DART_E_BADARG for a
+ * gradient_mode other than 7 or 8, a NULL `ref` or ref->rows, ref->len < 1, ref->start < 0, mode 7
+ * with spheres or mode 8 without them (dart_spheres as in the _spheres entries; n == 0 gives mode 7's
+ * bits), warm == 2, and in the closed-loop step plant_dt != params->dt.  A horizon above 16 is
+ * DART_E_UNSUPPORTED.  No host-memory or row-output entry takes a reference.
+ *
+ * dart_se3mpc_solve_batch_track: dart_se3mpc_solve_batch_spheres without `goal`, with the
+ * reference; `grid` (with margin, threshold, first_hit) serves only the optional fused safety check.
+ * plan_batch passes T = N and s = 0. */
+int dart_se3mpc_solve_batch_track(const dart_se3mpc_params *params, int64_t B, int64_t ld,
+                                  const double *p0, const double *v0, const uint8_t *has_goal,
+                                  const double *x_warm, const uint8_t *warm_mask, double *x_out, double *cost,
+                                  int32_t *nit, int32_t *nfev, int32_t *status, int32_t *task, double *acc,
+                                  double *att, double *rates, double *thrust, const dart_track_ref *ref,
+                                  const dart_spheres *spheres, const dart_grid *grid, double margin,
+                                  double threshold, int32_t *first_hit, void *cuda_stream);
+/* dart_se3mpc_closed_loop_step_spheres without `goal`, with the reference: a path of T samples and
+ * s = the step index, so the window slides one sample per replan (plant_dt == params->dt); past the
+ * end of the path the last sample is held.  check_grid / first_collision as in the _map step. */
+int dart_se3mpc_closed_loop_step_track(const dart_se3mpc_params *params, int64_t B, int64_t ld,
+                                       double *p, double *v, const uint8_t *has_goal, double *x,
+                                       int32_t warm, double *cost, int32_t *nit, int32_t *nfev,
+                                       int32_t *status, double plant_dt, const dart_track_ref *ref,
+                                       const dart_spheres *spheres, const dart_grid *check_grid,
+                                       double margin, double threshold, int32_t step,
+                                       int32_t *first_collision, void *cuda_stream);
 
 /* Same call with every buffer in HOST memory (pageable or pinned).  Up to 512 problems go
  * through a mapped pinned block the kernel reads and writes directly (no copies); larger batches
