@@ -13,9 +13,10 @@ from .mapper import DenseOccupancyGrid, SensorObservation  # noqa: F401
 from .mission import BatchedMissionGoals, SemanticWaypoint  # noqa: F401
 from .wire import SignedEnvelope  # noqa: F401
 from .closed_loop import ClosedLoopSim  # noqa: F401
+from .differentiable import plan_batch_differentiable  # noqa: F401
 from .sharding import ShardedSolver, replicate_map, shard_range  # noqa: F401
 
 __all__ = ["SE3MPCConfig", "load_planner_config", "DroneState", "Trajectory", "SE3MPCPlanner",
-           "BatchSolution", "plan_batch", "extract_batch", "solve_batch_tensors", "DenseOccupancyGrid", "SensorObservation", "ClosedLoopSim",
+           "BatchSolution", "plan_batch", "plan_batch_differentiable", "extract_batch", "solve_batch_tensors", "DenseOccupancyGrid", "SensorObservation", "ClosedLoopSim",
            "BatchedMissionGoals", "SemanticWaypoint", "SignedEnvelope",
            "ShardedSolver", "replicate_map", "shard_range"]

@@ -73,7 +73,7 @@ EXPORTS = [
     "dart_map_trace_ray_batch", "dart_map_update_batch", "dart_map_add_spheres", "dart_fp64_probe", "dart_ddiv_selftest",
     "dart_map_signed_distance", "dart_map_clearance_field", "dart_se3mpc_closed_loop_step_map",
     "dart_se3mpc_solve_batch_spheres", "dart_se3mpc_solve_batch_host_spheres", "dart_se3mpc_closed_loop_step_spheres",
-    "dart_se3mpc_solve_batch_track", "dart_se3mpc_closed_loop_step_track",
+    "dart_se3mpc_solve_batch_track", "dart_se3mpc_closed_loop_step_track", "dart_se3mpc_solve_vjp_batch",
 ]
 
 _lib = None
@@ -130,6 +130,9 @@ def lib():
                                                      [vp] * 4 + [C.c_double, C.POINTER(TrackRef), C.POINTER(Spheres),
                                                                   C.POINTER(Grid), C.c_double, C.c_double, i32, vp, vp])
     L.dart_se3mpc_closed_loop_step_track.restype = C.c_int
+    L.dart_se3mpc_solve_vjp_batch.argtypes = ([C.POINTER(Params), i64, i64] + [vp] * 5 + [C.POINTER(TrackRef),
+                                              C.POINTER(Spheres)] + [vp] * 9)
+    L.dart_se3mpc_solve_vjp_batch.restype = C.c_int
     L.dart_se3mpc_extract_batch.argtypes = [C.POINTER(Params), i64, i64] + [vp] * 5 + [i32, vp]
     L.dart_se3mpc_extract_batch.restype = C.c_int
     L.dart_se3mpc_release_thread_workspace.argtypes = []

@@ -20,7 +20,7 @@ UNITS = {
     "se3mpc_inst_l4.cu": [], "se3mpc_inst_l8.cu": [], "se3mpc_inst_l16.cu": [],
     "se3mpc_inst_l32.cu": [], "se3mpc_inst_l32x2.cu": [], "se3mpc_inst_l8_occ3.cu": [],
     "se3mpc_inst_l8_b64.cu": [], "se3mpc_inst_l16_occ3.cu": [], "se3mpc_inst_l32_occ3.cu": [],
-    "se3mpc_inst_l6.cu": [], "se3mpc_inst_l6_occ5.cu": [],
+    "se3mpc_inst_l6.cu": [], "se3mpc_inst_l6_occ5.cu": [], "se3mpc_vjp.cu": [],
     "mapper_kernels.cu": ["-fmad=false"],
     "probe_kernels.cu": [],
 }

@@ -345,6 +345,55 @@ int dart_se3mpc_closed_loop_step_track(const dart_se3mpc_params *params, int64_t
                                        double margin, double threshold, int32_t step,
                                        int32_t *first_collision, void *cuda_stream);
 
+/* ---- the differentiable solve: vector-Jacobian product of a returned plan (extension) ---------
+ * Scope: gradient_mode 3, 6, 7 and 8, horizons 1..16.  T* is the thrust rows of a returned solution x
+ * (any x: the P/V rows are not read).  The bounds l <= T <= u are the solve's own boxes (+-tilt_thrust
+ * on x and y, min_thrust..max_thrust on z).  The active set A is the set of entries with T*_i == l_i
+ * or T*_i == u_i, bit for bit (L-BFGS-B projects onto the box exactly); F is every other entry.
+ * Parameters theta, per problem: p0 and v0; the goal (modes 3 / 6) or the reference r_k, u_k (modes
+ * 7 / 8); the weights w = (w_pos, w_vel, w_acc, w_thrust).  The derivative holds T*_A constant and
+ * takes dT*_F/dtheta = -H_FF^-1 dg_F/dtheta, with g = grad_T f and H = hess_T f at the returned T*:
+ * defined at whatever T* the solve returned, converged or not.  (In modes 3 / 7, H and the derivatives
+ * with respect to p0, v0, goal and reference do not depend on T*; the weight derivatives do, as dg/dw
+ * is linear in T.)  Outputs that carry a derivative: x = [P | V | T], where P and V are the rollout of
+ * T*(theta) from (p0, v0), P_0 = p0 and V_0 = v0 included; and cost = f(T*(theta), theta).
+ * Given upstream gradients xbar (9N) and cbar (one per problem), the entry:
+ *   1. pulls xbar back through the rollout with the solve's adjoint,
+ *   2. adds cbar g(T*),
+ *   3. solves H_FF lam_F = tbar_F with lam_A = 0 (matrix-free conjugate gradients on F; every Hessian
+ *      product is a zero-state rollout and one adjoint; n_F <= 3N steps in exact arithmetic),
+ *   4. forms thetabar = -(dg/dtheta)^T lam + cbar df/dtheta + the rollout's direct dependence on p0 and
+ *      v0; (dg/dtheta)^T lam comes from one forward rollout of lam from a zero state.
+ * Modes 6 and 8 add the sphere penalty's Hessian on P_k where h > 0, 8 w e e^T - 4 w h I in the
+ * notation of dart_spheres; H_FF can then be indefinite.
+ * status [ld] per problem: 0 ok; 1 non-positive curvature met; 2 the linear solve did not reach its
+ * residual tolerance (|r| <= 1e-13 |tbar_F| within 2 n_F + 8 products).  Status 1 is a property of the
+ * system solved for this problem's upstream gradients, not of H_FF alone: conjugate gradients meet the
+ * curvature of H_FF only along the directions tbar_F reaches.  Where tbar_F is exactly zero no step runs,
+ * lam = 0 and the status is 0 even if H_FF is indefinite (the returned gradients are then exact).  Where
+ * the status is not 0, every gradient output of that problem is NaN.
+ *
+ * inputs   params, p0, v0, goal, has_goal : as in the solve that returned x (goal: modes 3 / 6 only,
+ *          not read in 7 / 8 or where has_goal is 0); ref (modes 7 / 8) with len = N and start = 0, as
+ *          plan_batch passes it; spheres (modes 6 / 8) as in the solve
+ *          x  : [9N][ld] the solve's solution
+ *          gx : [9N][ld] xbar, gcost : [ld] cbar; either may be NULL (zero)
+ * outputs  gp0, gv0 : [3][ld];  ggoal : [3][ld] (modes 3 / 6; not written in 7 / 8);
+ *          gref : [6N][ld] in the layout of the reference block (rows 3k+c rbar_k, 3N+3k+c ubar_k;
+ *          modes 7 / 8; not written in 3 / 6);  gw : [4][ld] wbar per problem;  any may be NULL
+ *          status : [ld] int32, required
+ * Refused with DART_E_BADARG: a gradient_mode outside {3, 6, 7, 8}; spheres in modes 3 / 7 or none in
+ * 6 / 8 (n < 0, or n > 0 with a NULL list); a reference in modes 3 / 6 or none in 7 / 8; ref->len != N,
+ * ref->start != 0 or a NULL ref->rows; NULL x, status, p0, v0, or goal in modes 3 / 6; B < 0 or
+ * ld < B.  A horizon above 16 is DART_E_UNSUPPORTED.  No gradient flows to warm starts, sphere
+ * centres or radii, obstacle_weight, or the derived arrays (attitudes, rates). */
+int dart_se3mpc_solve_vjp_batch(const dart_se3mpc_params *params, int64_t B, int64_t ld,
+                                const double *p0, const double *v0, const double *goal,
+                                const uint8_t *has_goal, const double *x, const dart_track_ref *ref,
+                                const dart_spheres *spheres, const double *gx, const double *gcost,
+                                double *gp0, double *gv0, double *ggoal, double *gref, double *gw,
+                                int32_t *status, void *cuda_stream);
+
 /* Same call with every buffer in HOST memory (pageable or pinned).  Up to 512 problems go
  * through a mapped pinned block the kernel reads and writes directly (no copies); larger batches
  * stage through an internal per-thread device workspace (chunked on two streams from 65536
