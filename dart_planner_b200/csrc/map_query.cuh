@@ -1,6 +1,6 @@
 /*
  * map_query.cuh -- occupancy-grid lookups shared by the mapper kernels and the solve kernel's
- * fused safety check.  world_to_voxel = floor(p / res) (explicit_geometric_mapper.py:91-94);
+ * fused safety check, and the grid check of every entry that takes a grid.  world_to_voxel = floor(p / res) (explicit_geometric_mapper.py:91-94);
  * keys outside the dense grid read the prior, like the reference's dict miss (:154-169).
  */
 #pragma once
@@ -10,6 +10,15 @@
 #include "../../include/dart_se3mpc.h"
 
 namespace dartb200 {
+
+/* a grid every entry may read: a dense box, a positive voxel size, float32 or float64 cells */
+inline int check_grid(const dart_grid *g)
+{
+    if (!g || !g->occ || g->nx <= 0 || g->ny <= 0 || g->nz <= 0 || !(g->resolution > 0.0))
+        return DART_E_BADARG;
+    if (g->cell_bytes != 0 && g->cell_bytes != 4 && g->cell_bytes != 8) return DART_E_BADARG;
+    return DART_OK;
+}
 
 __device__ __forceinline__ int vox(double p, double res) { return (int)floor(p / res); }
 

@@ -391,14 +391,6 @@ int grid_blocks(long long B)
     return (int)(nb < cap ? (nb < 1 ? 1 : nb) : cap);
 }
 
-int check_grid(const dart_grid *g)
-{
-    if (!g || !g->occ || g->nx <= 0 || g->ny <= 0 || g->nz <= 0 || !(g->resolution > 0.0))
-        return DART_E_BADARG;
-    if (g->cell_bytes != 0 && g->cell_bytes != 4 && g->cell_bytes != 8) return DART_E_BADARG;
-    return DART_OK;
-}
-
 } /* namespace */
 
 extern "C" {

@@ -8,6 +8,8 @@
 #pragma once
 #include <cuda_runtime.h>
 
+#include <utility>
+
 #include "map_query.cuh"
 #include "se3mpc_core.cuh"
 
@@ -626,45 +628,34 @@ se3mpc_extract_kernel(const __grid_constant__ dart_se3mpc_params P, const __grid
     }
 }
 
-/* the instantiations of one lane configuration: [gradient_mode][tilt].  The dynamics-consistent
- * modes 3 / 4 / 6 / 7 / 8 move the lateral thrust, so they exist only with tilt (fn[3][0] = fn[4][0] =
- * fn[6][0] = fn[7][0] = fn[8][0] = null).  The tracking modes 7 / 8 exist only in the builds that
- * serve horizons <= 16, the library's limit for them: null in the 32-lane builds. */
+/* the instantiations of one lane configuration: [gradient_mode][tilt], null where MODES says the
+ * kernel does not exist -- tilt = 0 in the modes without a 7-slot instantiation, and the tracking
+ * modes in the builds wider than their horizon limit (the 32-lane builds) */
 struct KernelSet {
-    const void *fn[9][2];
+    const void *fn[N_MODES][2];
     const void *extract_fn[2]; /* [tilt] */
     int lanes, tpl, block, minb;
     int gpb;      /* problems per block */
     int resident; /* blocks per SM the shared-memory carve-out is sized for (default: minb) */
 };
 
-template <int LANES, int TPL, int MINB, int BLK>
-KernelSet make_kernel_set()
+template <int LANES, int TPL, int BLK, int MINB, int GM, bool TILT>
+const void *solve_fn()
+{
+    if constexpr ((TILT || MODES[GM].seven_slot) && (!MODES[GM].track || LANES * TPL <= MODES[GM].max_horizon))
+        return (const void *)se3mpc_solve_kernel<LANES, TPL, BLK, MINB, GM, TILT>;
+    else
+        return nullptr;
+}
+
+template <int LANES, int TPL, int MINB, int BLK, int... GM>
+KernelSet make_kernel_set(std::integer_sequence<int, GM...>)
 {
     KernelSet k;
-    k.fn[0][1] = (const void *)se3mpc_solve_kernel<LANES, TPL, BLK, MINB, 0, true>;
-    k.fn[1][1] = (const void *)se3mpc_solve_kernel<LANES, TPL, BLK, MINB, 1, true>;
-    k.fn[2][1] = (const void *)se3mpc_solve_kernel<LANES, TPL, BLK, MINB, 2, true>;
-    k.fn[0][0] = (const void *)se3mpc_solve_kernel<LANES, TPL, BLK, MINB, 0, false>;
-    k.fn[1][0] = (const void *)se3mpc_solve_kernel<LANES, TPL, BLK, MINB, 1, false>;
-    k.fn[2][0] = (const void *)se3mpc_solve_kernel<LANES, TPL, BLK, MINB, 2, false>;
-    k.fn[3][1] = (const void *)se3mpc_solve_kernel<LANES, TPL, BLK, MINB, 3, true>;
-    k.fn[4][1] = (const void *)se3mpc_solve_kernel<LANES, TPL, BLK, MINB, 4, true>;
-    k.fn[5][1] = (const void *)se3mpc_solve_kernel<LANES, TPL, BLK, MINB, 5, true>;
-    k.fn[5][0] = (const void *)se3mpc_solve_kernel<LANES, TPL, BLK, MINB, 5, false>;
-    k.fn[6][1] = (const void *)se3mpc_solve_kernel<LANES, TPL, BLK, MINB, 6, true>;
-    if constexpr (LANES * TPL <= 16) {
-        k.fn[7][1] = (const void *)se3mpc_solve_kernel<LANES, TPL, BLK, MINB, 7, true>;
-        k.fn[8][1] = (const void *)se3mpc_solve_kernel<LANES, TPL, BLK, MINB, 8, true>;
-    } else {
-        k.fn[7][1] = nullptr;
-        k.fn[8][1] = nullptr;
-    }
-    k.fn[3][0] = nullptr;
-    k.fn[4][0] = nullptr;
-    k.fn[6][0] = nullptr;
-    k.fn[7][0] = nullptr;
-    k.fn[8][0] = nullptr;
+    /* tilted kernels first: in the throughput builds ptxas schedules a mode's tilted kernel
+     * differently when its 7-slot twin is instantiated before it */
+    ((k.fn[GM][1] = solve_fn<LANES, TPL, BLK, MINB, GM, true>()), ...);
+    ((k.fn[GM][0] = solve_fn<LANES, TPL, BLK, MINB, GM, false>()), ...);
     k.extract_fn[1] = (const void *)se3mpc_extract_kernel<LANES, TPL, BLK, true>;
     k.extract_fn[0] = (const void *)se3mpc_extract_kernel<LANES, TPL, BLK, false>;
     k.lanes = LANES;
@@ -674,6 +665,12 @@ KernelSet make_kernel_set()
     k.gpb = GroupMap<LANES, BLK>::GPB;
     k.resident = MINB;
     return k;
+}
+
+template <int LANES, int TPL, int MINB, int BLK>
+KernelSet make_kernel_set()
+{
+    return make_kernel_set<LANES, TPL, MINB, BLK>(std::make_integer_sequence<int, N_MODES>());
 }
 
 /* defined one per instantiation unit */

@@ -160,24 +160,18 @@ int prepare(KernelChoice *k)
         if (e != cudaSuccess) return set_err(e, "cudaDeviceGetAttribute");
     }
     const int smem = smem_bytes(*k);
-    const void *fns[] = {k->set.fn[0][0], k->set.fn[0][1], k->set.fn[1][0], k->set.fn[1][1],
-                         k->set.fn[2][0], k->set.fn[2][1], k->set.fn[3][1], k->set.fn[4][1],
-                         k->set.fn[5][0], k->set.fn[5][1], k->set.fn[6][1], k->set.fn[7][1],
-                         k->set.fn[8][1]};
-    for (const void *fn : fns) {
-        if (!fn) continue; /* modes 7 / 8 in the 32-lane builds */
-        e = cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
-        if (e != cudaSuccess) return set_err(e, "cudaFuncSetAttribute(smem)");
-    }
     /* shared-memory share of the 256 KB L1: what `minb` resident blocks need (+1 KB each that
      * the driver reserves); the rest stays L1 for the per-lane S/Y pairs in local memory */
     int carve = (int)((long long)k->set.resident * (smem + 1024) * 100 / (228 * 1024)) + 1;
     if (carve > 100) carve = 100;
-    for (const void *fn : fns) {
-        if (!fn) continue;
-        e = cudaFuncSetAttribute(fn, cudaFuncAttributePreferredSharedMemoryCarveout, carve);
-        if (e != cudaSuccess) return set_err(e, "cudaFuncSetAttribute(carveout)");
-    }
+    for (const auto &by_tilt : k->set.fn)
+        for (const void *fn : by_tilt) {
+            if (!fn) continue; /* no such instantiation (KernelSet) */
+            e = cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
+            if (e != cudaSuccess) return set_err(e, "cudaFuncSetAttribute(smem)");
+            e = cudaFuncSetAttribute(fn, cudaFuncAttributePreferredSharedMemoryCarveout, carve);
+            if (e != cudaSuccess) return set_err(e, "cudaFuncSetAttribute(carveout)");
+        }
     cudaFuncAttributes fa;
     e = cudaFuncGetAttributes(&fa, k->set.fn[0][1]);
     if (e != cudaSuccess) return set_err(e, "cudaFuncGetAttributes");
@@ -189,32 +183,47 @@ int prepare(KernelChoice *k)
     return DART_OK;
 }
 
-/* the dynamics-consistent modes: thrusts are the only variables, P / V their rollout */
-bool rollout_mode(int gm) { return gm == 3 || gm == 4 || gm == 6 || gm == 7 || gm == 8; }
-
-/* spheres: the caller is one of the _spheres entries, which serve modes 5 and 6 only; track: one of
- * the _track entries, which serve modes 7 and 8 only; every other entry serves modes 0..4 */
-int check_params(const dart_se3mpc_params *p, bool spheres = false, bool track = false)
+/* family: the entries the caller belongs to; each family serves its own modes (ModeInfo::family) */
+int check_params(const dart_se3mpc_params *p, ModeFamily family = FAM_PLAIN)
 {
     if (!p || p->struct_size != (int)sizeof(dart_se3mpc_params)) return DART_E_BADARG;
     if (p->horizon < 1 || p->horizon > 64) return DART_E_UNSUPPORTED;
     if (p->max_corrections < 1 || p->max_corrections > MMAX) return DART_E_UNSUPPORTED;
     /* maxls >= 1, as SciPy requires; with 0 every solve would end ABNORMAL after one evaluation */
     if (p->max_iterations < 0 || p->max_linesearch < 1) return DART_E_BADARG;
-    if (track) {
-        if (p->gradient_mode != 7 && p->gradient_mode != 8) return DART_E_BADARG;
-    } else if (spheres) {
-        if (p->gradient_mode != 5 && p->gradient_mode != 6) return DART_E_BADARG;
-    } else if (p->gradient_mode < 0 || p->gradient_mode > 4)
-        return DART_E_UNSUPPORTED;
-    /* dynamics-consistent modes: verified against the oracle up to the 16-lane builds; on 32-lane
-     * groups (horizons 17..64) the scan's rounding makes 5-7 % of the solves take other iteration
-     * counts than the sequential oracle at tolerance 1e-3 (DESIGN.md 5c) */
-    if (rollout_mode(p->gradient_mode) && p->horizon > 16) return DART_E_UNSUPPORTED;
+    const ModeInfo *m = mode_info(p->gradient_mode);
+    if (!m || m->family != family) return family == FAM_PLAIN ? DART_E_UNSUPPORTED : DART_E_BADARG;
+    if (p->horizon > m->max_horizon) return DART_E_UNSUPPORTED;
     if (!(p->dt > 0.0) || !(p->mass > 0.0)) return DART_E_BADARG;
     if (!(p->gtol >= 0.0)) return DART_E_BADARG; /* the Cauchy step relies on it (se3mpc_core.cuh) */
     return DART_OK;
 }
+
+/* What a solve entry was called with: the modes it serves, the kind of entry, and its arguments --
+ * the caller's arrays and scalars already in the launch's SolveArgs, the structs as passed.
+ * check_request checks it, in the order the header documents the refusals, and completes `a`. */
+enum EntryKind {
+    BATCH,       /* the batch solves: optional map check into first_hit */
+    ROWS,        /* dart_se3mpc_solve_batch_rows: the result and the map check in one row */
+    STEP,        /* the closed-loop steps with a map or a list: optional collision record */
+    STEP_NO_MAP, /* dart_se3mpc_closed_loop_step: no grid argument */
+    HOST,        /* the host entries: the device solve of each chunk checks the grid */
+};
+struct SolveRequest {
+    ModeFamily family;
+    EntryKind kind;
+    const dart_se3mpc_params *params;
+    SolveArgs a;
+    const dart_spheres *spheres = nullptr;
+    const dart_track_ref *ref = nullptr;
+    const dart_grid *grid = nullptr;      /* the penalty's grid; in BATCH and ROWS the map check's too */
+    const dart_grid *step_grid = nullptr; /* STEP: the collision record's grid */
+    int warm = 0;                         /* STEP: 0 cold, 1 warm, 2 warm with zero lateral thrust */
+    SolveRequest(ModeFamily f, EntryKind k, const dart_se3mpc_params *p) : family(f), kind(k), params(p)
+    {
+        memset(&a, 0, sizeof(a));
+    }
+};
 
 int check_spheres(const dart_spheres *s)
 {
@@ -222,28 +231,60 @@ int check_spheres(const dart_spheres *s)
     return DART_OK;
 }
 
-void set_spheres(SolveArgs &a, const dart_spheres *s)
+int check_request(SolveRequest &r)
 {
-    if (!s) return;
-    a.spheres = s->cxyzr;
-    a.n_spheres = s->n;
-    a.sphere_margin = s->margin;
-}
-
-/* the reference and sphere list of a _track entry (mode 7 takes no spheres, mode 8 needs them) */
-int check_track(const dart_se3mpc_params *p, const dart_track_ref *ref, const dart_spheres *s)
-{
-    if (!ref || !ref->rows || ref->len < 1 || ref->start < 0) return DART_E_BADARG;
-    if ((p->gradient_mode == 8) != (s != nullptr)) return DART_E_BADARG;
-    return s ? check_spheres(s) : DART_OK;
-}
-
-void set_track(SolveArgs &a, const dart_track_ref *ref)
-{
-    if (!ref) return;
-    a.track_rows = ref->rows;
-    a.track_len = ref->len;
-    a.track_start = ref->start;
+    const dart_se3mpc_params *p = r.params;
+    SolveArgs &a = r.a;
+    if (r.family == FAM_SPHERES && !r.spheres) return DART_E_BADARG;
+    int rc = check_params(p, r.family);
+    if (rc) return rc;
+    const ModeInfo &m = MODES[p->gradient_mode];
+    if (r.family == FAM_TRACK) {
+        const dart_track_ref *ref = r.ref;
+        if (!ref || !ref->rows || ref->len < 1 || ref->start < 0) return DART_E_BADARG;
+        if (m.spheres != (r.spheres != nullptr)) return DART_E_BADARG; /* mode 8 needs a list, mode 7 takes none */
+        a.track_rows = ref->rows;
+        a.track_len = ref->len;
+        a.track_start = ref->start;
+    }
+    if (r.spheres) {
+        if ((rc = check_spheres(r.spheres))) return rc;
+        a.spheres = r.spheres->cxyzr;
+        a.n_spheres = r.spheres->n;
+        a.sphere_margin = r.spheres->margin;
+    }
+    if (a.B < 0 || a.ld < a.B || !a.p0 || !a.v0 || (!a.goal && r.family != FAM_TRACK)) return DART_E_BADARG;
+    if (r.kind == HOST) return DART_OK;
+    if (r.kind == ROWS) {
+        if (!a.rows || a.rows_kind < 0 || a.rows_kind > 2) return DART_E_BADARG;
+        if (a.rows_kind == 1 && a.check_map) return DART_E_UNSUPPORTED; /* controls rows carry no map check */
+        const int need = row_stride_doubles(p->horizon, a.rows_kind);
+        if (need == 0) return DART_E_UNSUPPORTED; /* the row does not fit its staging block */
+        if (a.row_stride < need || (a.row_stride & 15) != 0 || a.row_stride > SM_DOUBLES ||
+            ((uintptr_t)a.rows & 127) != 0)
+            return DART_E_BADARG;
+    }
+    if (r.kind == BATCH || r.kind == ROWS) {
+        if (r.kind == BATCH) a.check_map = a.first_hit != nullptr;
+        if (!a.check_map && !m.grid_pen) return DART_OK;
+        if (check_grid(r.grid)) return DART_E_BADARG;
+        a.grid = a.check_grid = *r.grid;
+        return DART_OK;
+    }
+    if (!a.x_out || !(a.plant_dt > 0.0)) return DART_E_BADARG;
+    /* the reference window slides one sample per replan: one plant step must be one sample */
+    if (r.family == FAM_TRACK && a.plant_dt != p->dt) return DART_E_BADARG;
+    if (m.grid_pen && r.kind == STEP_NO_MAP) return DART_E_UNSUPPORTED;
+    if (m.grid_pen && check_grid(r.grid)) return DART_E_BADARG;
+    if ((r.step_grid != nullptr) != (a.first_collision != nullptr)) return DART_E_BADARG;
+    if (r.step_grid && check_grid(r.step_grid)) return DART_E_BADARG;
+    /* the promise of warm == 2 (zero lateral thrust) does not hold where the lateral thrust moves */
+    if (m.rollout && r.warm == 2) return DART_E_BADARG;
+    if (m.grid_pen) a.grid = *r.grid;
+    if (r.step_grid) a.check_grid = *r.step_grid;
+    a.x_warm = r.warm ? a.x_out : nullptr;
+    a.no_tilt_promise = r.warm == 2;
+    return DART_OK;
 }
 
 long long grid_for(const KernelChoice &k, long long B)
@@ -413,14 +454,13 @@ static int launch_solve(const dart_se3mpc_params *params, const SolveArgs &a, vo
             stash_event = sb.done;
         }
     }
-    /* never the 7-slot instantiation in the dynamics-consistent modes: their lateral thrust moves */
-    const int cold = ((a.x_warm == nullptr || a.no_tilt_promise) && !rollout_mode(params->gradient_mode) &&
-                      !getenv("DART_SE3MPC_NO_COLD")) ? 0 : 1;
-    /* an empty sphere list runs the plain mode's own kernel (mode 5 -> 0, 6 -> 3): the same results
-     * bit for bit, which a separate kernel cannot promise -- ptxas contracts the plain products and
-     * sums of the shared solver code kernel by kernel (DESIGN.md 5e) */
     int gm = params->gradient_mode;
-    if ((gm == 5 || gm == 6 || gm == 8) && a.n_spheres == 0) gm = (gm == 5) ? 0 : (gm == 6 ? 3 : 7);
+    const int cold = ((a.x_warm == nullptr || a.no_tilt_promise) && MODES[gm].seven_slot &&
+                      !getenv("DART_SE3MPC_NO_COLD")) ? 0 : 1;
+    /* an empty sphere list runs the plain mode's own kernel (mode 5 -> 0, 6 -> 3, 8 -> 7): the same
+     * results bit for bit, which a separate kernel cannot promise -- ptxas contracts the plain
+     * products and sums of the shared solver code kernel by kernel (DESIGN.md 5e) */
+    if (MODES[gm].spheres && a.n_spheres == 0) gm = MODES[gm].empty_spheres;
     const void *fn = k->set.fn[gm][cold];
     if (!fn) return DART_E_UNSUPPORTED; /* modes 7 / 8 forced onto a 32-lane build (DART_SE3MPC_VARIANT) */
     cudaError_t e;
@@ -448,43 +488,46 @@ static int launch_solve(const dart_se3mpc_params *params, const SolveArgs &a, vo
     return DART_OK;
 }
 
-/* the device solve of dart_se3mpc_solve_batch_map (spheres == NULL) and
- * dart_se3mpc_solve_batch_spheres */
-static int solve_batch_impl(const dart_se3mpc_params *params, int64_t B, int64_t ld, const double *p0,
-                            const double *v0, const double *goal, const uint8_t *has_goal,
-                            const double *x_warm, const uint8_t *warm_mask, double *x_out, double *cost,
-                            int32_t *nit, int32_t *nfev, int32_t *status, int32_t *task, double *acc,
-                            double *att, double *rates, double *thrust, const dart_grid *grid, double margin,
-                            double threshold, int32_t *first_hit, const dart_spheres *spheres,
-                            void *cuda_stream, const dart_track_ref *ref = nullptr, bool track = false)
+/* a checked request runs on the device; B == 0 ends after the checks */
+static int solve(SolveRequest &r, void *cuda_stream)
 {
-    int rc = check_params(params, spheres != nullptr, track);
-    if (rc) return rc;
-    if (track && (rc = check_track(params, ref, spheres))) return rc;
-    if (!track && spheres && (rc = check_spheres(spheres))) return rc;
-    if (B < 0 || ld < B || !p0 || !v0 || (!goal && !track)) return DART_E_BADARG;
-    const bool need_grid = first_hit != nullptr || params->gradient_mode == 2 || params->gradient_mode == 4;
-    if (need_grid && (!grid || !grid->occ || grid->nx <= 0 || grid->ny <= 0 || grid->nz <= 0 ||
-                      !(grid->resolution > 0.0)))
-        return DART_E_BADARG;
-    if (B == 0) return DART_OK;
-    SolveArgs a;
-    memset(&a, 0, sizeof(a));
+    const int rc = check_request(r);
+    if (rc || r.a.B == 0) return rc;
+    return launch_solve(r.params, r.a, cuda_stream);
+}
+
+/* the arguments every batch solve shares */
+static SolveArgs &batch_args(SolveRequest &r, int64_t B, int64_t ld, const double *p0, const double *v0,
+                             const double *goal, const uint8_t *has_goal, const double *x_warm,
+                             const uint8_t *warm_mask)
+{
+    SolveArgs &a = r.a;
     a.B = B; a.ld = ld;
     a.p0 = p0; a.v0 = v0; a.goal = goal; a.has_goal = has_goal;
     a.x_warm = x_warm; a.warm_mask = warm_mask;
+    return a;
+}
+
+static void set_outputs(SolveArgs &a, double *x_out, double *cost, int32_t *nit, int32_t *nfev, int32_t *status,
+                        int32_t *task, double *acc, double *att, double *rates, double *thrust)
+{
     a.x_out = x_out; a.cost = cost; a.nit = nit; a.nfev = nfev; a.status = status; a.task = task;
     a.acc = acc; a.att = att; a.rates = rates; a.thrust = thrust;
-    if (need_grid) a.grid = a.check_grid = *grid;
-    if (first_hit) {
-        a.margin = margin;
-        a.threshold = threshold;
-        a.first_hit = first_hit;
-        a.check_map = 1;
-    }
-    set_spheres(a, spheres);
-    set_track(a, ref);
-    return launch_solve(params, a, cuda_stream);
+}
+
+/* the arguments every closed-loop step shares: the state p / v is stepped in place, x is the warm
+ * start (warm != 0) and the new plan */
+static SolveArgs &step_args(SolveRequest &r, int64_t B, int64_t ld, double *p, double *v, const double *goal,
+                            const uint8_t *has_goal, double *x, int32_t warm, double *cost, int32_t *nit,
+                            int32_t *nfev, int32_t *status, double plant_dt)
+{
+    SolveArgs &a = r.a;
+    a.B = B; a.ld = ld;
+    a.p0 = a.p_next = p; a.v0 = a.v_next = v; a.goal = goal; a.has_goal = has_goal;
+    a.x_out = x; a.cost = cost; a.nit = nit; a.nfev = nfev; a.status = status;
+    a.plant_dt = plant_dt;
+    r.warm = warm;
+    return a;
 }
 
 int dart_se3mpc_solve_batch_map(const dart_se3mpc_params *params, int64_t B, int64_t ld,
@@ -496,9 +539,11 @@ int dart_se3mpc_solve_batch_map(const dart_se3mpc_params *params, int64_t B, int
                                 double margin, double threshold, int32_t *first_hit,
                                 void *cuda_stream)
 {
-    return solve_batch_impl(params, B, ld, p0, v0, goal, has_goal, x_warm, warm_mask, x_out, cost, nit, nfev,
-                            status, task, acc, att, rates, thrust, grid, margin, threshold, first_hit, nullptr,
-                            cuda_stream);
+    SolveRequest r(FAM_PLAIN, BATCH, params);
+    SolveArgs &a = batch_args(r, B, ld, p0, v0, goal, has_goal, x_warm, warm_mask);
+    set_outputs(a, x_out, cost, nit, nfev, status, task, acc, att, rates, thrust);
+    r.grid = grid; a.margin = margin; a.threshold = threshold; a.first_hit = first_hit;
+    return solve(r, cuda_stream);
 }
 
 int dart_se3mpc_solve_batch_spheres(const dart_se3mpc_params *params, int64_t B, int64_t ld,
@@ -510,110 +555,12 @@ int dart_se3mpc_solve_batch_spheres(const dart_se3mpc_params *params, int64_t B,
                                     const dart_grid *grid, double margin, double threshold,
                                     int32_t *first_hit, void *cuda_stream)
 {
-    if (!spheres) return DART_E_BADARG;
-    return solve_batch_impl(params, B, ld, p0, v0, goal, has_goal, x_warm, warm_mask, x_out, cost, nit, nfev,
-                            status, task, acc, att, rates, thrust, grid, margin, threshold, first_hit, spheres,
-                            cuda_stream);
-}
-
-int dart_se3mpc_closed_loop_step(const dart_se3mpc_params *params, int64_t B, int64_t ld, double *p,
-                                 double *v, const double *goal, const uint8_t *has_goal, double *x,
-                                 int32_t warm, double *cost, int32_t *nit, int32_t *nfev,
-                                 int32_t *status, double plant_dt, void *cuda_stream)
-{
-    int rc = check_params(params);
-    if (rc) return rc;
-    if (B < 0 || ld < B || !p || !v || !goal || !x || !(plant_dt > 0.0)) return DART_E_BADARG;
-    /* no map argument here: no obstacle penalty */
-    if (params->gradient_mode == 2 || params->gradient_mode == 4) return DART_E_UNSUPPORTED;
-    /* the promise of warm == 2 (zero lateral thrust) does not hold in the dynamics-consistent mode */
-    if (params->gradient_mode == 3 && warm == 2) return DART_E_BADARG;
-    if (B == 0) return DART_OK;
-    SolveArgs a;
-    memset(&a, 0, sizeof(a));
-    a.B = B; a.ld = ld;
-    a.p0 = p; a.v0 = v; a.goal = goal; a.has_goal = has_goal;
-    a.x_warm = warm ? x : nullptr;
-    a.no_tilt_promise = (warm == 2) ? 1 : 0;
-    a.x_out = x; a.cost = cost; a.nit = nit; a.nfev = nfev; a.status = status;
-    a.p_next = p; a.v_next = v; a.plant_dt = plant_dt;
-    return launch_solve(params, a, cuda_stream);
-}
-
-static bool grid_ok(const dart_grid *g)
-{
-    return g && g->occ && g->nx > 0 && g->ny > 0 && g->nz > 0 && g->resolution > 0.0 &&
-           (g->cell_bytes == 0 || g->cell_bytes == 4 || g->cell_bytes == 8);
-}
-
-/* the step of dart_se3mpc_closed_loop_step_map (spheres == NULL) and
- * dart_se3mpc_closed_loop_step_spheres */
-static int closed_loop_step_impl(const dart_se3mpc_params *params, int64_t B, int64_t ld, double *p, double *v,
-                                 const double *goal, const uint8_t *has_goal, double *x, int32_t warm,
-                                 double *cost, int32_t *nit, int32_t *nfev, int32_t *status, double plant_dt,
-                                 const dart_grid *penalty_grid, const dart_spheres *spheres,
-                                 const dart_grid *check_grid, double margin, double threshold, int32_t step,
-                                 int32_t *first_collision, void *cuda_stream, const dart_track_ref *ref = nullptr,
-                                 bool track = false)
-{
-    int rc = check_params(params, spheres != nullptr, track);
-    if (rc) return rc;
-    if (track && (rc = check_track(params, ref, spheres))) return rc;
-    if (!track && spheres && (rc = check_spheres(spheres))) return rc;
-    if (B < 0 || ld < B || !p || !v || (!goal && !track) || !x || !(plant_dt > 0.0)) return DART_E_BADARG;
-    /* the reference window slides one sample per replan: one plant step must be one sample */
-    if (track && plant_dt != params->dt) return DART_E_BADARG;
-    const bool penalty = params->gradient_mode == 2 || params->gradient_mode == 4;
-    if (penalty && !grid_ok(penalty_grid)) return DART_E_BADARG;
-    if ((check_grid != nullptr) != (first_collision != nullptr)) return DART_E_BADARG;
-    if (check_grid && !grid_ok(check_grid)) return DART_E_BADARG;
-    /* the promise of warm == 2 (zero lateral thrust) does not hold in the dynamics-consistent modes */
-    if (rollout_mode(params->gradient_mode) && warm == 2) return DART_E_BADARG;
-    if (B == 0) return DART_OK;
-    SolveArgs a;
-    memset(&a, 0, sizeof(a));
-    a.B = B; a.ld = ld;
-    a.p0 = p; a.v0 = v; a.goal = goal; a.has_goal = has_goal;
-    a.x_warm = warm ? x : nullptr;
-    a.no_tilt_promise = (warm == 2) ? 1 : 0;
-    a.x_out = x; a.cost = cost; a.nit = nit; a.nfev = nfev; a.status = status;
-    a.p_next = p; a.v_next = v; a.plant_dt = plant_dt;
-    if (penalty) a.grid = *penalty_grid;
-    if (check_grid) {
-        a.check_grid = *check_grid;
-        a.margin = margin;
-        a.threshold = threshold;
-        a.first_collision = first_collision;
-        a.step = step;
-    }
-    set_spheres(a, spheres);
-    set_track(a, ref);
-    return launch_solve(params, a, cuda_stream);
-}
-
-int dart_se3mpc_closed_loop_step_map(const dart_se3mpc_params *params, int64_t B, int64_t ld, double *p,
-                                     double *v, const double *goal, const uint8_t *has_goal, double *x,
-                                     int32_t warm, double *cost, int32_t *nit, int32_t *nfev,
-                                     int32_t *status, double plant_dt, const dart_grid *penalty_grid,
-                                     const dart_grid *check_grid, double margin, double threshold,
-                                     int32_t step, int32_t *first_collision, void *cuda_stream)
-{
-    return closed_loop_step_impl(params, B, ld, p, v, goal, has_goal, x, warm, cost, nit, nfev, status, plant_dt,
-                                 penalty_grid, nullptr, check_grid, margin, threshold, step, first_collision,
-                                 cuda_stream);
-}
-
-int dart_se3mpc_closed_loop_step_spheres(const dart_se3mpc_params *params, int64_t B, int64_t ld, double *p,
-                                         double *v, const double *goal, const uint8_t *has_goal, double *x,
-                                         int32_t warm, double *cost, int32_t *nit, int32_t *nfev,
-                                         int32_t *status, double plant_dt, const dart_spheres *spheres,
-                                         const dart_grid *check_grid, double margin, double threshold,
-                                         int32_t step, int32_t *first_collision, void *cuda_stream)
-{
-    if (!spheres) return DART_E_BADARG;
-    return closed_loop_step_impl(params, B, ld, p, v, goal, has_goal, x, warm, cost, nit, nfev, status, plant_dt,
-                                 nullptr, spheres, check_grid, margin, threshold, step, first_collision,
-                                 cuda_stream);
+    SolveRequest r(FAM_SPHERES, BATCH, params);
+    SolveArgs &a = batch_args(r, B, ld, p0, v0, goal, has_goal, x_warm, warm_mask);
+    set_outputs(a, x_out, cost, nit, nfev, status, task, acc, att, rates, thrust);
+    r.spheres = spheres;
+    r.grid = grid; a.margin = margin; a.threshold = threshold; a.first_hit = first_hit;
+    return solve(r, cuda_stream);
 }
 
 int dart_se3mpc_solve_batch_track(const dart_se3mpc_params *params, int64_t B, int64_t ld,
@@ -624,21 +571,13 @@ int dart_se3mpc_solve_batch_track(const dart_se3mpc_params *params, int64_t B, i
                                   const dart_spheres *spheres, const dart_grid *grid, double margin,
                                   double threshold, int32_t *first_hit, void *cuda_stream)
 {
-    return solve_batch_impl(params, B, ld, p0, v0, nullptr, has_goal, x_warm, warm_mask, x_out, cost, nit, nfev,
-                            status, task, acc, att, rates, thrust, grid, margin, threshold, first_hit, spheres,
-                            cuda_stream, ref, true);
-}
-
-int dart_se3mpc_closed_loop_step_track(const dart_se3mpc_params *params, int64_t B, int64_t ld, double *p,
-                                       double *v, const uint8_t *has_goal, double *x, int32_t warm, double *cost,
-                                       int32_t *nit, int32_t *nfev, int32_t *status, double plant_dt,
-                                       const dart_track_ref *ref, const dart_spheres *spheres,
-                                       const dart_grid *check_grid, double margin, double threshold,
-                                       int32_t step, int32_t *first_collision, void *cuda_stream)
-{
-    return closed_loop_step_impl(params, B, ld, p, v, nullptr, has_goal, x, warm, cost, nit, nfev, status, plant_dt,
-                                 nullptr, spheres, check_grid, margin, threshold, step, first_collision,
-                                 cuda_stream, ref, true);
+    SolveRequest r(FAM_TRACK, BATCH, params);
+    SolveArgs &a = batch_args(r, B, ld, p0, v0, nullptr, has_goal, x_warm, warm_mask);
+    set_outputs(a, x_out, cost, nit, nfev, status, task, acc, att, rates, thrust);
+    r.ref = ref;
+    r.spheres = spheres;
+    r.grid = grid; a.margin = margin; a.threshold = threshold; a.first_hit = first_hit;
+    return solve(r, cuda_stream);
 }
 
 int dart_se3mpc_solve_batch(const dart_se3mpc_params *params, int64_t B, int64_t ld,
@@ -651,6 +590,76 @@ int dart_se3mpc_solve_batch(const dart_se3mpc_params *params, int64_t B, int64_t
     return dart_se3mpc_solve_batch_map(params, B, ld, p0, v0, goal, has_goal, x_warm, warm_mask, x_out,
                                        cost, nit, nfev, status, task, acc, att, rates, thrust, nullptr,
                                        0.0, 0.0, nullptr, cuda_stream);
+}
+
+int dart_se3mpc_solve_batch_rows(const dart_se3mpc_params *params, int64_t B, int64_t ld,
+                                 const double *p0, const double *v0, const double *goal,
+                                 const uint8_t *has_goal, const double *x_warm,
+                                 const uint8_t *warm_mask, double *rows, int64_t row_stride,
+                                 int32_t row_kind, const dart_grid *grid, double margin,
+                                 double threshold, int32_t check_map, void *cuda_stream)
+{
+    SolveRequest r(FAM_PLAIN, ROWS, params);
+    SolveArgs &a = batch_args(r, B, ld, p0, v0, goal, has_goal, x_warm, warm_mask);
+    a.rows = rows; a.row_stride = row_stride; a.rows_kind = row_kind;
+    r.grid = grid; a.margin = margin; a.threshold = threshold; a.check_map = check_map != 0;
+    return solve(r, cuda_stream);
+}
+
+int dart_se3mpc_closed_loop_step(const dart_se3mpc_params *params, int64_t B, int64_t ld, double *p,
+                                 double *v, const double *goal, const uint8_t *has_goal, double *x,
+                                 int32_t warm, double *cost, int32_t *nit, int32_t *nfev,
+                                 int32_t *status, double plant_dt, void *cuda_stream)
+{
+    SolveRequest r(FAM_PLAIN, STEP_NO_MAP, params);
+    step_args(r, B, ld, p, v, goal, has_goal, x, warm, cost, nit, nfev, status, plant_dt);
+    return solve(r, cuda_stream);
+}
+
+int dart_se3mpc_closed_loop_step_map(const dart_se3mpc_params *params, int64_t B, int64_t ld, double *p,
+                                     double *v, const double *goal, const uint8_t *has_goal, double *x,
+                                     int32_t warm, double *cost, int32_t *nit, int32_t *nfev,
+                                     int32_t *status, double plant_dt, const dart_grid *penalty_grid,
+                                     const dart_grid *check_grid, double margin, double threshold,
+                                     int32_t step, int32_t *first_collision, void *cuda_stream)
+{
+    SolveRequest r(FAM_PLAIN, STEP, params);
+    SolveArgs &a = step_args(r, B, ld, p, v, goal, has_goal, x, warm, cost, nit, nfev, status, plant_dt);
+    r.grid = penalty_grid;
+    r.step_grid = check_grid; a.margin = margin; a.threshold = threshold; a.step = step;
+    a.first_collision = first_collision;
+    return solve(r, cuda_stream);
+}
+
+int dart_se3mpc_closed_loop_step_spheres(const dart_se3mpc_params *params, int64_t B, int64_t ld, double *p,
+                                         double *v, const double *goal, const uint8_t *has_goal, double *x,
+                                         int32_t warm, double *cost, int32_t *nit, int32_t *nfev,
+                                         int32_t *status, double plant_dt, const dart_spheres *spheres,
+                                         const dart_grid *check_grid, double margin, double threshold,
+                                         int32_t step, int32_t *first_collision, void *cuda_stream)
+{
+    SolveRequest r(FAM_SPHERES, STEP, params);
+    SolveArgs &a = step_args(r, B, ld, p, v, goal, has_goal, x, warm, cost, nit, nfev, status, plant_dt);
+    r.spheres = spheres;
+    r.step_grid = check_grid; a.margin = margin; a.threshold = threshold; a.step = step;
+    a.first_collision = first_collision;
+    return solve(r, cuda_stream);
+}
+
+int dart_se3mpc_closed_loop_step_track(const dart_se3mpc_params *params, int64_t B, int64_t ld, double *p,
+                                       double *v, const uint8_t *has_goal, double *x, int32_t warm, double *cost,
+                                       int32_t *nit, int32_t *nfev, int32_t *status, double plant_dt,
+                                       const dart_track_ref *ref, const dart_spheres *spheres,
+                                       const dart_grid *check_grid, double margin, double threshold,
+                                       int32_t step, int32_t *first_collision, void *cuda_stream)
+{
+    SolveRequest r(FAM_TRACK, STEP, params);
+    SolveArgs &a = step_args(r, B, ld, p, v, nullptr, has_goal, x, warm, cost, nit, nfev, status, plant_dt);
+    r.ref = ref;
+    r.spheres = spheres;
+    r.step_grid = check_grid; a.margin = margin; a.threshold = threshold; a.step = step;
+    a.first_collision = first_collision;
+    return solve(r, cuda_stream);
 }
 
 int dart_se3mpc_extract_batch(const dart_se3mpc_params *params, int64_t B, int64_t ld,
@@ -686,43 +695,6 @@ int64_t dart_se3mpc_row_stride(const dart_se3mpc_params *params, int32_t row_kin
     return (int64_t)row_stride_doubles(params->horizon, row_kind);
 }
 
-int dart_se3mpc_solve_batch_rows(const dart_se3mpc_params *params, int64_t B, int64_t ld,
-                                 const double *p0, const double *v0, const double *goal,
-                                 const uint8_t *has_goal, const double *x_warm,
-                                 const uint8_t *warm_mask, double *rows, int64_t row_stride,
-                                 int32_t row_kind, const dart_grid *grid, double margin,
-                                 double threshold, int32_t check_map, void *cuda_stream)
-{
-    int rc = check_params(params);
-    if (rc) return rc;
-    if (B < 0 || ld < B || !p0 || !v0 || !goal || !rows) return DART_E_BADARG;
-    if (row_kind < 0 || row_kind > 2) return DART_E_BADARG;
-    if (row_kind == 1 && check_map) return DART_E_UNSUPPORTED; /* controls rows carry no map check */
-    const int need = row_stride_doubles(params->horizon, row_kind);
-    if (need == 0) return DART_E_UNSUPPORTED; /* the row does not fit its staging block */
-    if (row_stride < need || (row_stride & 15) != 0 || row_stride > SM_DOUBLES ||
-        ((uintptr_t)rows & 127) != 0)
-        return DART_E_BADARG;
-    const bool need_grid = check_map != 0 || params->gradient_mode == 2 || params->gradient_mode == 4;
-    if (need_grid && (!grid || !grid->occ || grid->nx <= 0 || grid->ny <= 0 || grid->nz <= 0 ||
-                      !(grid->resolution > 0.0)))
-        return DART_E_BADARG;
-    if (B == 0) return DART_OK;
-    SolveArgs a;
-    memset(&a, 0, sizeof(a));
-    a.B = B; a.ld = ld;
-    a.p0 = p0; a.v0 = v0; a.goal = goal; a.has_goal = has_goal;
-    a.x_warm = x_warm; a.warm_mask = warm_mask;
-    a.rows = rows; a.row_stride = row_stride; a.rows_kind = row_kind;
-    if (need_grid) a.grid = a.check_grid = *grid;
-    if (check_map) {
-        a.margin = margin;
-        a.threshold = threshold;
-        a.check_map = 1; /* the result goes into the row */
-    }
-    return launch_solve(params, a, cuda_stream);
-}
-
 /* ---- host-buffer entry: staged through a cached per-thread device workspace --------------- */
 namespace {
 struct HostWs {
@@ -737,32 +709,17 @@ struct HostWs {
 };
 thread_local HostWs g_ws;
 
-/* workspace layout for row pitch Bp (elements): fp64 rows [p0 3 | v0 3 | goal 3 | x_warm 9N |
- * x 9N | cost 1 | acc 3N | att 3N | rates 3N | thrust N], int32 rows [nit nfev status task],
- * u8 row [has_goal].  Inputs are one contiguous range, outputs another. */
-struct WsLayout {
-    size_t Bp, in_rows, out_off_rows, out_rows, int_off, hg_off, bytes;
-    WsLayout(int N, size_t Bp_) : Bp(Bp_)
-    {
-        in_rows = 9 + 9 * (size_t)N;
-        out_off_rows = in_rows;
-        out_rows = 9 * (size_t)N + 1 + 9 * (size_t)N + (size_t)N;
-        int_off = (in_rows + out_rows) * Bp * 8;
-        hg_off = int_off + 4 * Bp * 4;
-        bytes = hg_off + ((Bp + 7) / 8) * 8;
-    }
+/* one block of rows of the workspace: the caller's array of `rows` rows of B elements of esz bytes
+ * (NULL: not passed, not copied) and its place in the workspace, rows of Bp elements from byte `off` */
+struct WsRows {
+    const void *user;
+    size_t off, rows, esz;
 };
 
-void rows_in(void *dst, size_t pitch, const void *src, size_t B, size_t rows, size_t esz)
+/* the host's cudaMemcpy2D: `rows` rows of `width` bytes */
+void copy_rows(void *dst, size_t dpitch, const void *src, size_t spitch, size_t width, size_t rows)
 {
-    for (size_t r = 0; r < rows; ++r)
-        memcpy((char *)dst + r * pitch * esz, (const char *)src + r * B * esz, B * esz);
-}
-void rows_out(void *dst, const void *src, size_t pitch, size_t B, size_t rows, size_t esz)
-{
-    if (!dst) return;
-    for (size_t r = 0; r < rows; ++r)
-        memcpy((char *)dst + r * B * esz, (const char *)src + r * pitch * esz, B * esz);
+    for (size_t r = 0; r < rows; ++r) memcpy((char *)dst + r * dpitch, (const char *)src + r * spitch, width);
 }
 }
 
@@ -784,29 +741,37 @@ void dart_se3mpc_release_thread_workspace(void)
     g_ws = HostWs();
 }
 
-/* the host entry of dart_se3mpc_solve_batch_host (spheres == NULL) and
- * dart_se3mpc_solve_batch_host_spheres (the list in host memory: staged behind the workspace) */
-static int solve_batch_host_impl(const dart_se3mpc_params *params, int64_t B, const double *p0, const double *v0,
-                                 const double *goal, const uint8_t *has_goal, const double *x_warm,
-                                 double *x_out, double *cost, int32_t *nit, int32_t *nfev, int32_t *status,
-                                 double *acc, double *att, double *rates, double *thrust,
-                                 const dart_spheres *spheres)
+/* the host entries: r holds the caller's host arrays; the sphere list, if any, is staged behind the
+ * workspace */
+static int solve_host(SolveRequest &r)
 {
-    int rc = check_params(params, spheres != nullptr);
+    int rc = check_request(r);
     if (rc) return rc;
-    if (spheres && (rc = check_spheres(spheres))) return rc;
-    if (B < 0 || !p0 || !v0 || !goal) return DART_E_BADARG;
+    const SolveArgs &u = r.a;
+    const int64_t B = u.B;
     if (B == 0) return DART_OK;
-    const size_t N = (size_t)params->horizon;
+    const size_t N = (size_t)r.params->horizon;
+    const dart_spheres *spheres = r.spheres;
     /* small batches (the drop-in planner's single solve): no copies at all -- the kernel reads its
      * inputs from and writes its results to a mapped pinned block over PCIe (zero-copy: one
      * launch and one synchronise; 62 us instead of 85 us at 512 problems); large batches copy
      * rows straight from / to the caller's buffers */
     const bool staged = B <= 512;
     const size_t Bp = staged ? (size_t)((B + 3) / 4 * 4) : (size_t)((B + 31) / 32 * 32);
-    const WsLayout L((int)N, Bp);
+    /* workspace layout for row pitch Bp (elements): fp64 rows [p0 3 | v0 3 | goal 3 | x_warm 9N |
+     * x 9N | cost 1 | acc 3N | att 3N | rates 3N | thrust N], int32 rows [nit nfev status task],
+     * u8 row [has_goal] */
+    const size_t d8 = Bp * 8, x_off = (9 + 9 * N) * d8, acc_off = x_off + (9 * N + 1) * d8;
+    const size_t int_off = acc_off + 10 * N * d8, hg_off = int_off + 4 * Bp * 4;
+    const WsRows in[] = {{u.p0, 0, 3, 8}, {u.v0, 3 * d8, 3, 8}, {u.goal, 6 * d8, 3, 8},
+                         {u.has_goal, hg_off, 1, 1}, {u.x_warm, 9 * d8, 9 * N, 8}};
+    const WsRows out[] = {{u.x_out, x_off, 9 * N, 8},           {u.cost, x_off + 9 * N * d8, 1, 8},
+                          {u.nit, int_off, 1, 4},               {u.nfev, int_off + 4 * Bp, 1, 4},
+                          {u.status, int_off + 8 * Bp, 1, 4},   {u.acc, acc_off, 3 * N, 8},
+                          {u.att, acc_off + 3 * N * d8, 3 * N, 8}, {u.rates, acc_off + 6 * N * d8, 3 * N, 8},
+                          {u.thrust, acc_off + 9 * N * d8, N, 8}};
     /* the sphere list, if any, follows the workspace: [n][4] doubles at a 16-byte offset */
-    const size_t sph_off = (L.bytes + 15) / 16 * 16;
+    const size_t sph_off = (hg_off + (Bp + 7) / 8 * 8 + 15) / 16 * 16;
     const size_t sph_bytes = spheres ? (size_t)spheres->n * 4 * sizeof(double) : 0;
     const size_t ws_bytes = sph_off + sph_bytes;
     cudaError_t e;
@@ -861,14 +826,6 @@ static int solve_batch_host_impl(const dart_se3mpc_params *params, int64_t B, co
         if (e != cudaSuccess) return set_err(e, "cudaHostGetDevicePointer");
         base = (char *)mapped;
     }
-    double *d = (double *)base;
-    double *d_p0 = d, *d_v0 = d_p0 + 3 * Bp, *d_goal = d_v0 + 3 * Bp, *d_xw = d_goal + 3 * Bp;
-    double *d_x = d_xw + 9 * N * Bp, *d_cost = d_x + 9 * N * Bp;
-    double *d_acc = d_cost + Bp, *d_att = d_acc + 3 * N * Bp, *d_rates = d_att + 3 * N * Bp;
-    double *d_thr = d_rates + 3 * N * Bp;
-    int32_t *d_nit = (int32_t *)(base + L.int_off), *d_nfev = d_nit + Bp, *d_status = d_nfev + Bp,
-            *d_task = d_status + Bp;
-    uint8_t *d_hg = (uint8_t *)(base + L.hg_off);
     /* the device copy of the list the solves read (uploaded once per call) */
     dart_spheres dsph;
     if (spheres) {
@@ -881,12 +838,42 @@ static int solve_batch_host_impl(const dart_se3mpc_params *params, int64_t B, co
             if (e != cudaSuccess) return set_err(e, "cudaMemcpyAsync H2D (spheres)");
         }
     }
-    const dart_spheres *dsp = spheres ? &dsph : nullptr;
-    if (!staged && B >= 65536) {
-        /* Large batch: chunks of 32768 problems alternate between two streams, each doing its own
-         * pitched H2D rows -> solve -> pitched D2H rows, so the read-back of chunk i (the
-         * dominant cost: 1.3 KB per solve over PCIe) overlaps the solve of chunk i+1 and the
-         * upload of chunk i+2.  Fully asynchronous when the caller's buffers are pinned. */
+    /* the device solve of problems [c0, c0 + cb) on the workspace's rows; only the outputs the
+     * caller asked for are computed and written */
+    auto run = [&](int64_t c0, int64_t cb, cudaStream_t cs) {
+        auto at = [&](const WsRows &w) { return w.user ? base + w.off + c0 * w.esz : nullptr; };
+        SolveRequest d(r.family, BATCH, r.params);
+        d.spheres = spheres ? &dsph : nullptr;
+        SolveArgs &a = batch_args(d, cb, (int64_t)Bp, (const double *)at(in[0]), (const double *)at(in[1]),
+                                  (const double *)at(in[2]), (const uint8_t *)at(in[3]), (const double *)at(in[4]),
+                                  nullptr);
+        set_outputs(a, (double *)at(out[0]), (double *)at(out[1]), (int32_t *)at(out[2]), (int32_t *)at(out[3]),
+                    (int32_t *)at(out[4]), nullptr, (double *)at(out[5]), (double *)at(out[6]),
+                    (double *)at(out[7]), (double *)at(out[8]));
+        return solve(d, (void *)cs);
+    };
+    if (staged) {
+        char *h = (char *)g_ws.pin;
+        for (const WsRows &w : in)
+            if (w.user) copy_rows(h + w.off, Bp * w.esz, w.user, (size_t)B * w.esz, (size_t)B * w.esz, w.rows);
+        rc = run(0, B, s);
+        if (rc) return rc;
+        e = cudaStreamSynchronize(s);
+        if (e != cudaSuccess) return set_err(e, "cudaStreamSynchronize");
+        for (const WsRows &w : out)
+            if (w.user)
+                copy_rows(const_cast<void *>(w.user), (size_t)B * w.esz, h + w.off, Bp * w.esz, (size_t)B * w.esz,
+                          w.rows);
+        return DART_OK;
+    }
+    /* Large batch: chunks of 32768 problems alternate between two streams, each doing its own
+     * pitched H2D rows -> solve -> pitched D2H rows, so the read-back of chunk i (the dominant
+     * cost: 1.3 KB per solve over PCIe) overlaps the solve of chunk i+1 and the upload of chunk
+     * i+2.  Fully asynchronous when the caller's buffers are pinned.  Below 65536 problems: one
+     * chunk on one stream. */
+    const bool pipelined = B >= 65536;
+    const int64_t chunk = pipelined ? 32768 : B;
+    if (pipelined) {
         if (!g_ws.stream2) {
             e = cudaStreamCreateWithFlags(&g_ws.stream2, cudaStreamNonBlocking);
             if (e != cudaSuccess) return set_err(e, "cudaStreamCreate");
@@ -900,133 +887,40 @@ static int solve_batch_host_impl(const dart_se3mpc_params *params, int64_t B, co
             if (e == cudaSuccess) e = cudaStreamWaitEvent(g_ws.stream2, g_ws.spheres_up, 0);
             if (e != cudaSuccess) return set_err(e, "cudaStreamWaitEvent(spheres)");
         }
-        const int64_t chunk = 32768;
-        int ci = 0;
-        /* on a failure mid-loop the copies already queued still write into the caller's buffers:
-         * wait for them before handing the buffers back */
-        auto drain = [&]() {
-            cudaStreamSynchronize(g_ws.stream);
-            cudaStreamSynchronize(g_ws.stream2);
-        };
-        struct HintScope { /* every chunk runs the build chosen for the whole batch */
-            explicit HintScope(long long b) { g_batch_hint = b; }
-            ~HintScope() { g_batch_hint = 0; }
-        } hint_scope(B);
-        for (int64_t c0 = 0; c0 < B; c0 += chunk, ++ci) {
-            const int64_t cb = (B - c0 < chunk) ? (B - c0) : chunk;
-            cudaStream_t cs = (ci & 1) ? g_ws.stream2 : g_ws.stream;
-#define ROWS_H2D(dst, src, rows, esz)                                                                        \
-    do {                                                                                                     \
-        e = cudaMemcpy2DAsync((char *)(dst) + c0 * (esz), Bp * (esz), (const char *)(src) + c0 * (esz),        \
-                              (size_t)B * (esz), (size_t)cb * (esz), rows, cudaMemcpyHostToDevice, cs);       \
-        if (e != cudaSuccess) return drain(), set_err(e, "cudaMemcpy2DAsync H2D");                           \
-    } while (0)
-#define ROWS_D2H(dst, src, rows, esz)                                                                        \
-    do {                                                                                                     \
-        if (dst) {                                                                                           \
-            e = cudaMemcpy2DAsync((char *)(dst) + c0 * (esz), (size_t)B * (esz), (const char *)(src) + c0 * (esz), \
-                                  Bp * (esz), (size_t)cb * (esz), rows, cudaMemcpyDeviceToHost, cs);          \
-            if (e != cudaSuccess) return drain(), set_err(e, "cudaMemcpy2DAsync D2H");                       \
-        }                                                                                                    \
-    } while (0)
-            ROWS_H2D(d_p0, p0, 3, 8);
-            ROWS_H2D(d_v0, v0, 3, 8);
-            ROWS_H2D(d_goal, goal, 3, 8);
-            if (has_goal) ROWS_H2D(d_hg, has_goal, 1, 1);
-            if (x_warm) ROWS_H2D(d_xw, x_warm, 9 * N, 8);
-            rc = solve_batch_impl(params, cb, (int64_t)Bp, d_p0 + c0, d_v0 + c0, d_goal + c0,
-                                  has_goal ? d_hg + c0 : nullptr, x_warm ? d_xw + c0 : nullptr, nullptr,
-                                  x_out ? d_x + c0 : nullptr, cost ? d_cost + c0 : nullptr,
-                                  nit ? d_nit + c0 : nullptr, nfev ? d_nfev + c0 : nullptr,
-                                  status ? d_status + c0 : nullptr, nullptr, acc ? d_acc + c0 : nullptr,
-                                  att ? d_att + c0 : nullptr, rates ? d_rates + c0 : nullptr,
-                                  thrust ? d_thr + c0 : nullptr, nullptr, 0.0, 0.0, nullptr, dsp, (void *)cs);
-            if (rc) return drain(), rc;
-            ROWS_D2H(x_out, d_x, 9 * N, 8);
-            ROWS_D2H(cost, d_cost, 1, 8);
-            ROWS_D2H(nit, d_nit, 1, 4);
-            ROWS_D2H(nfev, d_nfev, 1, 4);
-            ROWS_D2H(status, d_status, 1, 4);
-            ROWS_D2H(acc, d_acc, 3 * N, 8);
-            ROWS_D2H(att, d_att, 3 * N, 8);
-            ROWS_D2H(rates, d_rates, 3 * N, 8);
-            ROWS_D2H(thrust, d_thr, N, 8);
-#undef ROWS_H2D
-#undef ROWS_D2H
+    }
+    /* on a failure mid-loop the copies already queued still write into the caller's buffers:
+     * wait for them before handing the buffers back */
+    auto drain = [&]() {
+        if (!pipelined) return;
+        cudaStreamSynchronize(g_ws.stream);
+        cudaStreamSynchronize(g_ws.stream2);
+    };
+    struct HintScope { /* every chunk runs the build chosen for the whole batch */
+        explicit HintScope(long long b) { g_batch_hint = b; }
+        ~HintScope() { g_batch_hint = 0; }
+    } hint_scope(B);
+    int ci = 0;
+    for (int64_t c0 = 0; c0 < B; c0 += chunk, ++ci) {
+        const int64_t cb = (B - c0 < chunk) ? (B - c0) : chunk;
+        cudaStream_t cs = (ci & 1) ? g_ws.stream2 : g_ws.stream;
+        for (const WsRows &w : in) {
+            if (!w.user) continue;
+            e = cudaMemcpy2DAsync(base + w.off + c0 * w.esz, Bp * w.esz, (const char *)w.user + c0 * w.esz,
+                                  (size_t)B * w.esz, (size_t)cb * w.esz, w.rows, cudaMemcpyHostToDevice, cs);
+            if (e != cudaSuccess) return drain(), set_err(e, "cudaMemcpy2DAsync H2D");
         }
-        e = cudaStreamSynchronize(g_ws.stream);
-        if (e == cudaSuccess) e = cudaStreamSynchronize(g_ws.stream2);
-        if (e != cudaSuccess) return set_err(e, "cudaStreamSynchronize");
-        return DART_OK;
+        rc = run(c0, cb, cs);
+        if (rc) return drain(), rc;
+        for (const WsRows &w : out) {
+            if (!w.user) continue;
+            e = cudaMemcpy2DAsync((char *)const_cast<void *>(w.user) + c0 * w.esz, (size_t)B * w.esz,
+                                  base + w.off + c0 * w.esz, Bp * w.esz, (size_t)cb * w.esz, w.rows,
+                                  cudaMemcpyDeviceToHost, cs);
+            if (e != cudaSuccess) return drain(), set_err(e, "cudaMemcpy2DAsync D2H");
+        }
     }
-    if (staged) {
-        char *h = (char *)g_ws.pin;
-        rows_in(h, Bp, p0, (size_t)B, 3, 8);
-        rows_in(h + 3 * Bp * 8, Bp, v0, (size_t)B, 3, 8);
-        rows_in(h + 6 * Bp * 8, Bp, goal, (size_t)B, 3, 8);
-        if (x_warm) rows_in(h + 9 * Bp * 8, Bp, x_warm, (size_t)B, 9 * N, 8);
-        if (has_goal) memcpy(h + L.hg_off, has_goal, (size_t)B);
-    } else {
-#define H2D(dst, src, rows, esz)                                                              \
-    do {                                                                                      \
-        e = cudaMemcpy2DAsync(dst, Bp * (esz), src, (size_t)B * (esz), (size_t)B * (esz), rows, \
-                              cudaMemcpyHostToDevice, s);                                     \
-        if (e != cudaSuccess) return set_err(e, "cudaMemcpy2DAsync H2D");                     \
-    } while (0)
-        H2D(d_p0, p0, 3, 8);
-        H2D(d_v0, v0, 3, 8);
-        H2D(d_goal, goal, 3, 8);
-        if (has_goal) H2D(d_hg, has_goal, 1, 1);
-        if (x_warm) H2D(d_xw, x_warm, 9 * N, 8);
-#undef H2D
-    }
-    const bool all = false; /* only the rows the caller asked for are computed and written */
-    rc = solve_batch_impl(params, B, (int64_t)Bp, d_p0, d_v0, d_goal, has_goal ? d_hg : nullptr,
-                          x_warm ? d_xw : nullptr, nullptr, (all || x_out) ? d_x : nullptr,
-                          (all || cost) ? d_cost : nullptr, (all || nit) ? d_nit : nullptr,
-                          (all || nfev) ? d_nfev : nullptr, (all || status) ? d_status : nullptr,
-                          nullptr, (all || acc) ? d_acc : nullptr, (all || att) ? d_att : nullptr,
-                          (all || rates) ? d_rates : nullptr, (all || thrust) ? d_thr : nullptr,
-                          nullptr, 0.0, 0.0, nullptr, dsp, (void *)s);
-    if (rc) return rc;
-    if (staged) {
-        char *h = (char *)g_ws.pin;
-        e = cudaStreamSynchronize(s);
-        if (e != cudaSuccess) return set_err(e, "cudaStreamSynchronize");
-        const double *hd = (const double *)h;
-        const double *h_x = hd + L.in_rows * Bp, *h_cost = h_x + 9 * N * Bp, *h_acc = h_cost + Bp,
-                     *h_att = h_acc + 3 * N * Bp, *h_rates = h_att + 3 * N * Bp, *h_thr = h_rates + 3 * N * Bp;
-        const int32_t *h_nit = (const int32_t *)(h + L.int_off);
-        rows_out(x_out, h_x, Bp, (size_t)B, 9 * N, 8);
-        rows_out(cost, h_cost, Bp, (size_t)B, 1, 8);
-        rows_out(acc, h_acc, Bp, (size_t)B, 3 * N, 8);
-        rows_out(att, h_att, Bp, (size_t)B, 3 * N, 8);
-        rows_out(rates, h_rates, Bp, (size_t)B, 3 * N, 8);
-        rows_out(thrust, h_thr, Bp, (size_t)B, N, 8);
-        rows_out(nit, h_nit, Bp, (size_t)B, 1, 4);
-        rows_out(nfev, h_nit + Bp, Bp, (size_t)B, 1, 4);
-        rows_out(status, h_nit + 2 * Bp, Bp, (size_t)B, 1, 4);
-        return DART_OK;
-    }
-#define D2H(dst, src, rows, esz)                                                              \
-    do {                                                                                      \
-        if (dst) {                                                                            \
-            e = cudaMemcpy2DAsync(dst, (size_t)B * (esz), src, Bp * (esz), (size_t)B * (esz), rows, \
-                                  cudaMemcpyDeviceToHost, s);                                 \
-            if (e != cudaSuccess) return set_err(e, "cudaMemcpy2DAsync D2H");                 \
-        }                                                                                     \
-    } while (0)
-    D2H(x_out, d_x, 9 * N, 8);
-    D2H(cost, d_cost, 1, 8);
-    D2H(nit, d_nit, 1, 4);
-    D2H(nfev, d_nfev, 1, 4);
-    D2H(status, d_status, 1, 4);
-    D2H(acc, d_acc, 3 * N, 8);
-    D2H(att, d_att, 3 * N, 8);
-    D2H(rates, d_rates, 3 * N, 8);
-    D2H(thrust, d_thr, N, 8);
-#undef D2H
-    e = cudaStreamSynchronize(s);
+    e = cudaStreamSynchronize(g_ws.stream);
+    if (e == cudaSuccess && pipelined) e = cudaStreamSynchronize(g_ws.stream2);
     if (e != cudaSuccess) return set_err(e, "cudaStreamSynchronize");
     return DART_OK;
 }
@@ -1037,8 +931,10 @@ int dart_se3mpc_solve_batch_host(const dart_se3mpc_params *params, int64_t B,
                                  double *cost, int32_t *nit, int32_t *nfev, int32_t *status,
                                  double *acc, double *att, double *rates, double *thrust)
 {
-    return solve_batch_host_impl(params, B, p0, v0, goal, has_goal, x_warm, x_out, cost, nit, nfev, status, acc,
-                                 att, rates, thrust, nullptr);
+    SolveRequest r(FAM_PLAIN, HOST, params);
+    SolveArgs &a = batch_args(r, B, B, p0, v0, goal, has_goal, x_warm, nullptr);
+    set_outputs(a, x_out, cost, nit, nfev, status, nullptr, acc, att, rates, thrust);
+    return solve_host(r);
 }
 
 int dart_se3mpc_solve_batch_host_spheres(const dart_se3mpc_params *params, int64_t B,
@@ -1048,9 +944,11 @@ int dart_se3mpc_solve_batch_host_spheres(const dart_se3mpc_params *params, int64
                                          double *acc, double *att, double *rates, double *thrust,
                                          const dart_spheres *spheres)
 {
-    if (!spheres) return DART_E_BADARG;
-    return solve_batch_host_impl(params, B, p0, v0, goal, has_goal, x_warm, x_out, cost, nit, nfev, status, acc,
-                                 att, rates, thrust, spheres);
+    SolveRequest r(FAM_SPHERES, HOST, params);
+    SolveArgs &a = batch_args(r, B, B, p0, v0, goal, has_goal, x_warm, nullptr);
+    set_outputs(a, x_out, cost, nit, nfev, status, nullptr, acc, att, rates, thrust);
+    r.spheres = spheres;
+    return solve_host(r);
 }
 
 } /* extern "C" */

@@ -42,15 +42,17 @@ extern "C" int dart_se3mpc_solve_vjp_batch(const dart_se3mpc_params *params, int
                                            int32_t *status, void *cuda_stream)
 {
     if (!params || params->struct_size != (int)sizeof(dart_se3mpc_params)) return DART_E_BADARG;
-    const int gm = params->gradient_mode, N = params->horizon;
-    if (gm != 3 && gm != 6 && gm != 7 && gm != 8) return DART_E_BADARG;
-    const bool track = gm == 7 || gm == 8, sph = gm == 6 || gm == 8;
+    const int N = params->horizon;
+    /* the dynamics-consistent modes without the grid penalty: 3, 6, 7 and 8 */
+    const ModeInfo *m = mode_info(params->gradient_mode);
+    if (!m || !m->rollout || m->grid_pen) return DART_E_BADARG;
+    const bool track = m->track, sph = m->spheres;
     if (sph != (spheres != nullptr) || track != (ref != nullptr)) return DART_E_BADARG;
     if (spheres && (spheres->n < 0 || (spheres->n > 0 && !spheres->cxyzr))) return DART_E_BADARG;
     if (ref && (!ref->rows || ref->len != N || ref->start != 0)) return DART_E_BADARG;
     if (!x || !status || !p0 || !v0 || (!track && !goal) || B < 0 || ld < B) return DART_E_BADARG;
     if (N < 1) return DART_E_BADARG;
-    if (N > 16) return DART_E_UNSUPPORTED;
+    if (N > m->max_horizon) return DART_E_UNSUPPORTED;
     if (!(params->dt > 0.0) || !(params->mass > 0.0)) return DART_E_BADARG;
     if (B == 0) return DART_OK;
     VjpArgs a;

@@ -146,7 +146,8 @@ int dart_ddiv_selftest(int64_t n, uint64_t seed, int32_t emax, uint64_t *mismatc
  * occ: [nz][ny][nx] (x fastest) of float32 (cell_bytes 4 or 0: half the bytes, probabilities to
  * 1e-7) or float64 (cell_bytes 8: the reference's own precision -- its voxels hold Python floats);
  * voxel key (kx,ky,kz) = floor(p/res) lives at index (kx-ox, ky-oy, kz-oz); keys outside the grid
- * read `prior` (the reference's dict miss, :168). */
+ * read `prior` (the reference's dict miss, :168).  Every entry that reads a grid refuses one with
+ * nx, ny or nz < 1, resolution <= 0, a NULL occ or cell_bytes outside {0, 4, 8} (DART_E_BADARG). */
 typedef struct dart_grid {
     int32_t nx, ny, nz;
     int32_t ox, oy, oz;
